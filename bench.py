@@ -4,6 +4,7 @@
     python bench.py --gpus N --steps K --warmup W          (N > 1: launched by torchrun, one rank per GPU)
     python bench.py --config C1|C2|C3|C4|C5 ...            one BASELINE.json config as the headline line (default C2)
     python bench.py --impl reference ...                   CPU arm: the oracle port on all host cores
+    python bench.py --dump-outputs DIR ...                 also write the headline's last-step outputs as DIR/<name>.npy
 
 Headline (default): config C2 = BASELINE.json configs[1] (Pilz 6-DOF + armature 1e-2, N = 100 nodes x B = 65,536 scenarios per
 GPU, fp64, dense Jacobians; weak scaling).  One "step" = one pass of the hot path over the rank's whole batch: the Jacobian
@@ -32,6 +33,7 @@ METRIC = "rollout_steps_per_s_with_jacobians"
 UNIT = "rollout-steps/s"
 ARMATURE = 1e-2
 JAC_CHUNK_BYTES = 24 << 30  # Jacobian buffer reused over the scenario chunks of a config (C2's own Jacobian is 23.6 GB)
+DUMP_BYTES = 48 << 20  # --dump-outputs: all arrays together stay under 64 MB
 
 # name -> (model, nodes N, scenarios, dt, scaling)   scenarios: per GPU for "weak", total for "strong"
 CONFIGS = {
@@ -401,14 +403,44 @@ class ConfigRunner:
     def launches_per_step(self) -> int:
         return -1
 
+    def outputs(self, gathered) -> dict:
+        """What a caller of step() holds after it: q+, qd+, f+ of every chunk, the Jacobian of the last chunk (one buffer is
+        reused by all chunks) and the per-scenario cost / residual rows (of every rank after the all-gather)."""
+        return {"q_next": [o[0] for o in self.out], "qd_next": [o[1] for o in self.out], "f_next": [o[2] for o in self.out],
+                "jacobian": [self.jac], "cost_residual": list(gathered.reshape(-1, 4, self.Bc))}
+
+
+def dump_outputs(path: str, arrays: dict) -> None:
+    """Write every array as <path>/<name>.npy in float64.  `arrays` maps a name to a list of equally wide chunks whose last
+    axes together make the unit axis.  An array larger than its share of DUMP_BYTES keeps a fixed, seeded sample of its unit
+    columns (in ascending order), so runs with the same arguments write the same elements and two builds compare one to one."""
+    import numpy as np
+    import torch
+    os.makedirs(path, exist_ok=True)
+    share = DUMP_BYTES // len(arrays)
+    for name, chunks in arrays.items():
+        width = chunks[0].shape[-1]
+        total, rows = width * len(chunks), chunks[0].numel() // width
+        keep = min(total, max(1, share // (8 * rows)))
+        idx = np.sort(np.random.default_rng(0).choice(total, keep, replace=False)) if keep < total else np.arange(total)
+        cols = [torch.from_numpy(idx[idx // width == i] % width).to(c.device) for i, c in enumerate(chunks)]
+        out = torch.cat([c.index_select(c.dim() - 1, k) for c, k in zip(chunks, cols)], -1)
+        np.save(os.path.join(path, name + ".npy"), out.to(torch.float64).cpu().numpy())
+
+
+def warmup_steps(steps: int, warmup: int) -> int:
+    """Warm-up steps actually run before K timed steps: W, but at least one (module load, first-touch allocations) and at
+    least three when more than one step is timed."""
+    return max(warmup, 3) if steps > 1 else max(warmup, 1)
+
 
 def time_config(runner: ConfigRunner, steps: int, warmup: int, fence, sampler=None):
-    """W warm-up steps, then exactly K timed steps bracketed by fence(); device time by CUDA events; per-kernel times of the
-    pipeline through the library's event hooks (compile-time families) or the events around the whole Jacobian call."""
+    """warmup_steps(K, W) warm-up steps, then exactly K timed steps bracketed by fence(); device time by CUDA events; per-kernel
+    times of the pipeline through the library's event hooks (compile-time families) or the events around the whole Jacobian call."""
     import ctypes as C
     import torch
     from mpc_fatigue_b200 import _capi
-    for _ in range(max(warmup, 3) if steps > 1 else max(warmup, 1)):
+    for _ in range(warmup_steps(steps, warmup)):
         runner.step()
     fence()
     launches0 = _capi.lib.mpcf_launch_count()
@@ -486,11 +518,12 @@ def config_result(name: str, runner: ConfigRunner, t: dict, steps: int, world: i
             "checksum_cost": float(t["gathered"].reshape(-1, 4, runner.Bc)[:, 0].sum().item())}
 
 
-def run_c1(dev) -> dict:
+def run_c1(dev, steps: int = 10, warmup: int = 3, outputs: dict | None = None) -> dict:
     """C1: Pilz 3-DOF fatigue OCP (python/Pilz_3_DOF/inverse_dynamics_pilz_3DOF.py:78-89,124-146: N=20, T=4; per node
     tau = RNEA(q, qd, 0), F0 bound tau0=50, alpha=2, floor=10, Euler).  "CPU CasADi reference run" stand-in: the oracle's
     reference-mode node evaluation of ONE OCP (20 nodes, one thread), timed; beside it the GPU evaluating 65,536 such OCPs
-    per launch, and the agreement of the two on the first OCP."""
+    per launch (`steps` timed launches after warmup_steps(steps, warmup)), and the agreement of the two on the first OCP.
+    `outputs` receives the GPU results of the last timed launch."""
     import numpy as np
     import torch
     from mpc_fatigue_b200.evaluator import BatchEvaluator
@@ -520,19 +553,23 @@ def run_c1(dev) -> dict:
         tau_c, qn_c, Tn_c, viol_c = cpu_once()
     cpu_s = (time.perf_counter() - t0) / reps
     # GPU: all B OCPs
-    for _ in range(3):
+    warm = warmup_steps(steps, warmup)
+    for _ in range(warm):
         tau_g, qn_g, Tn_g = ev.node_eval_ref([], -1.0, q, qd, None, f, h)
     torch.cuda.synchronize()
     e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
     e0.record()
-    for _ in range(10):
+    for _ in range(steps):
         tau_g, qn_g, Tn_g = ev.node_eval_ref([], -1.0, q, qd, None, f, h)
     e1.record()
     torch.cuda.synchronize()
-    gpu_ms = e0.elapsed_time(e1) / 10
+    gpu_ms = e0.elapsed_time(e1) / steps
+    if outputs is not None:
+        outputs.update(tau=[tau_g], q_next=[qn_g], T_next=[Tn_g])
     err = max(float(np.abs(a[:, idx].cpu().numpy() - b).max() / max(1.0, np.abs(b).max())) for a, b in ((tau_g, tau_c), (qn_g, qn_c), (Tn_g, Tn_c)))
     return {"config": {"workload": "C1: Pilz 3-DOF fatigue OCP, reference-mode node evaluation (RNEA(q,qd,0), Euler, thermal ZOH, F0 bound), "
                                    "N=20 nodes, T=4", "robot": "pilz3", "nodes": N},
+            "steps": steps, "warmup": warm,
             "cpu_reference_run": {"seconds_per_ocp_evaluation": cpu_s, "node_evaluations_per_s": N / cpu_s, "cores": 1, "kind": "port",
                                   "what": "oracle reference-mode node evaluation of one OCP (20 nodes), the stand-in for the per-node CasADi "
                                           "calls of inverse_dynamics_pilz_3DOF.py:124-146 (casadi is not installable here)",
@@ -578,8 +615,11 @@ def run_gpu(args) -> None:
 
     # ---- headline config ----
     if head == "C1":
-        line = run_c1(dev) if rank == 0 else None
+        outputs = {}
+        line = run_c1(dev, args.steps, args.warmup, outputs) if rank == 0 else None
         if rank == 0:
+            if args.dump_outputs:
+                dump_outputs(args.dump_outputs, outputs)
             print(json.dumps(dict(line, metric="reference_mode_node_evaluations_per_s", value=line["gpu"]["node_evaluations_per_s"],
                                   unit="node-evaluations/s", n_gpus=world, higher_is_better=True, dtype="f64", data="synthetic")))
         if world > 1:
@@ -587,6 +627,8 @@ def run_gpu(args) -> None:
         return
     runner = ConfigRunner(head, dev, rank, world)
     t = time_config(runner, args.steps, args.warmup, fence, sampler)
+    if args.dump_outputs and rank == 0:  # before the legs below overwrite the first chunk's states and free the Jacobian
+        dump_outputs(args.dump_outputs, runner.outputs(t["gathered"]))
     t["el_ms"] = max_over_ranks(t["el_ms"])
     clocks = sampler.stop(*t["marks"]) if rank == 0 else None
     peak_tf = fp64_probe(dev)
@@ -684,7 +726,7 @@ def run_gpu(args) -> None:
         fmv = frozen_flop_model(n)
         cpu = cpu_baseline() if world == 1 and not args.no_cpu else None
         line = {
-            "metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": max(args.warmup, 3),
+            "metric": METRIC, "value": res["value"], "unit": UNIT, "n_gpus": world, "steps": args.steps, "warmup": warmup_steps(args.steps, args.warmup),
             "ms_per_step": res["ms_per_step"], "higher_is_better": True, "scaling": CONFIGS[head]["scaling"], "vs_baseline": None,
             "dtype": "f64", "data": "synthetic", "config": res["config"], "clocks": clocks, "gpu_launches": res["gpu_launches"],
             "e2e": e2e, "e2e_reduced_rows": e2e_reduced, "roofline": res["roofline"],
@@ -710,7 +752,13 @@ def main():
     ap.add_argument("--config", default="C2", choices=["C1", "C2", "C3", "C4", "C5"])
     ap.add_argument("--only-headline", action="store_true", help="skip the side configs (C1, C3, C4, C5) of the default run")
     ap.add_argument("--no-cpu", action="store_true", help="skip the cpu_baseline leg")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write the headline config's outputs of the last "
+                    "step as DIR/<name>.npy (float64, under 64 MB in all: larger outputs keep a fixed, seeded sample of their units)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the outputs of the GPU path (--impl ours)")
     if args.impl == "reference":
         run_reference(args)
     else:

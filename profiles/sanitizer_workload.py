@@ -1,5 +1,5 @@
 import sys, os
-sys.path.insert(0, '/root/repo')
+sys.path.insert(0, os.path.dirname(os.path.dirname(os.path.abspath(__file__))))
 import torch
 from mpc_fatigue_b200.evaluator import BatchEvaluator
 from mpc_fatigue_b200.model import Model, data_urdf
