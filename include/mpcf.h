@@ -213,11 +213,20 @@ int mpcf_cost_residual_table_batch(const mpcf_model *model, long B, int N, const
                                    double f_max, double *out, long ld_out, void *stream);
 
 /* Fused reference-mode OCP node rows: every constraint row and the running cost the reference's scripts build per shooting
-   node, one launch for B scenarios x N nodes (node-major units u = k*B + b).  Compile-time families only.
-   One arm (chain3/6/7; python/Pilz_6_DOF/force_optimization_pilz_6DOF.py:130-177), 3 + 3n rows:
+   node, one launch for B scenarios x N nodes (node-major units u = k*B + b).  Every kernel family:
+     compile-time families: chain3/6/7 have one arm, forest12x6 / forest14x7 two (opts->ee_frame[1] is ignored on the
+       one-arm chains); ee_frame[c] must be carried by arm c (MPCF_EFRAME otherwise, world-fixed frames included).
+     run-time trees (generic16 / generic64: branched trees, prismatic and continuous joints, up to 64 DOF): one arm when
+       opts->ee_frame[1] < 0, two otherwise; the frames may sit anywhere in the tree.  On a tree both end-effectors may share
+       ancestors (e.g. a torso joint): tau = ID(q,qd,0) + wsign (J_L^T [F_L;0] + J_R^T [F_R;0]) sums both terms there, and
+       dtau_dF is non-zero in both arm blocks on those joints (on the forests the cross-arm blocks are structural zeros).  A
+       prismatic joint contributes z_j to J_lin and nothing to the rotation.  A frame whose parent is the world (fparent -1)
+       has a constant pose and a zero Jacobian.
+   A frame index out of range is MPCF_EFRAME.  mpcf_ocp_rows_count_arms gives the row count for either arm count.
+   One arm (python/Pilz_6_DOF/force_optimization_pilz_6DOF.py:130-177), 3 + 3n rows:
      [0,3) ee_pos - p_ref | n: tau = ID(q,qd,0) + wsign J^T [F;0] | n: q + h qd - q_next | n: T+ - T_next (thermal ZOH)
      cost = w_F F.F + w_qd qd.qd                                                   (w_F = -1: the script's -F^T F)
-   Two arms (forest12x6 / forest14x7; Box_Pilz_6DOF2.py:244-293,454-475, mpc_principal.py:229-327,
+   Two arms (Box_Pilz_6DOF2.py:244-293,454-475, mpc_principal.py:229-327,
    RepeatedMPCwithThermal_confriction.py:251-273), 26 + 3n rows:
      [0,3) F_L + F_R - fdes | [3,6) (pL-pR) x F_L + (pR-pL) x F_R | [6] |pL-pR|^2 - dist2_ref |
      [7,10) R_L^T (pR-pL) - (the same at the previous node | rel_pos0 at node 0) | [10,13) e(R_L R_R^T) - rel_ori0 |
@@ -225,7 +234,8 @@ int mpcf_cost_residual_table_batch(const mpcf_model *model, long B, int N, const
      cost = w_box |p_box - p_ref|^2 + w_qd qd.qd + w_F (F_L.F_L + F_R.F_R)
    Arrays: q, qd [n][U]; F [3 arms][U]; T [n][U] or NULL (thermal rows = 0); q_last / T_last [n][B]: the trailing state the
    last node's defects compare with (NULL: zero defect there); rel_pos0 / rel_ori0 [3][B] (two arms; NULL = 0);
-   rows [rows][U], cost [U].  Optional derivative outputs (NULL to skip): dtau_dF [n][3 arms][U] = wsign J_lin^T,
+   rows [rows][U], cost [U].  Optional derivative outputs (NULL to skip): dtau_dF [n][3 arms][U] = wsign J_c,lin^T (arm c's
+   block; J_c,lin = linear rows of the frame Jacobian of arm c's end-effector),
    dT_dtau [n][U] = d T+ / d tau (chain it with mpcf_node_eval_ref_jvp_batch for the thermal rows), kin_jac
    [26 | 3][n + 3 arms][U] = d (kinematic rows) / d (q, F) of the node's own variables (the relative-position row's block
    with respect to the previous node's q is minus the same block evaluated there). */
@@ -235,7 +245,11 @@ typedef struct {
     double fdes[3];    /* e.g. (0, 0, m g) */
     double dist2_ref, mu, p_ref[3], w_box, w_qd, w_F, h;
 } mpcf_rows_opts;
+/* rows of mpcf_ocp_rows_batch for a compile-time family (26 + 3n with two arms, 3 + 3n with one); MPCF_EINVAL on run-time trees */
 int mpcf_ocp_rows_count(const mpcf_model *model);
+/* (narm == 2 ? 26 : 3) + 3n for any family; MPCF_EINVAL when narm is not 1 or 2, or differs from a compile-time family's
+   arm count.  Host only. */
+int mpcf_ocp_rows_count_arms(const mpcf_model *model, int narm);
 int mpcf_ocp_rows_batch(const mpcf_model *model, const mpcf_rows_opts *opts, long B, int N, const double *q,
                         const double *qd, const double *F, const double *T, const double *q_last, const double *T_last,
                         const double *rel_pos0, const double *rel_ori0, double *rows, double *cost, double *dtau_dF,

@@ -78,6 +78,7 @@ _sig = {
     "mpcf_cost_residual_table_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 7 + [C.c_double] * 2 + [_dp, C.c_double, _dp, C.c_long,
                                                                                                          C.c_void_p]),
     "mpcf_ocp_rows_count": (C.c_int, [C.c_void_p]),
+    "mpcf_ocp_rows_count_arms": (C.c_int, [C.c_void_p, C.c_int]),
     "mpcf_ocp_rows_batch": (C.c_int, [C.c_void_p, C.POINTER(RowsOpts), C.c_long, C.c_int] + [_dp] * 13 + [C.c_void_p]),
     "mpcf_probe_fp64": (C.c_int, [C.c_long, C.c_int, _dp, C.c_void_p]),
     "mpcf_memcpy2d_async": (C.c_int, [C.c_void_p, C.c_size_t, C.c_void_p, C.c_size_t, C.c_size_t, C.c_size_t, C.c_int, C.c_void_p]),

@@ -674,6 +674,16 @@ extern "C" int mpcf_ocp_rows_count(const mpcf_model *model)
     return (arms == 2 ? 26 : 3) + 3 * model->h.n;
 }
 
+extern "C" int mpcf_ocp_rows_count_arms(const mpcf_model *model, int narm)
+{
+    if (!model) return fail(MPCF_EINVAL, "null model");
+    if (narm != 1 && narm != 2) return fail(MPCF_EINVAL, "ocp rows: narm must be 1 or 2");
+    const int arms = family_chains(model->fam);
+    if (arms != 0 && narm != arms)
+        return fail(MPCF_EINVAL, "ocp rows: this compile-time family has " + std::to_string(arms) + " arm(s), not " + std::to_string(narm));
+    return (narm == 2 ? 26 : 3) + 3 * model->h.n;
+}
+
 extern "C" int mpcf_ocp_rows_batch(const mpcf_model *model, const mpcf_rows_opts *o, long B, int N, const double *q, const double *qd,
                                    const double *F, const double *T, const double *q_last, const double *T_last, const double *rel_pos0,
                                    const double *rel_ori0, double *rows, double *cost, double *dtau_dF, double *dT_dtau, double *kin_jac,
@@ -683,15 +693,22 @@ extern "C" int mpcf_ocp_rows_batch(const mpcf_model *model, const mpcf_rows_opts
     PROLOGUE(q && qd && F && rows && cost)
     if (!o || B < 0 || N <= 0) return fail(MPCF_EINVAL, "bad options / B / N");
     const int arms = family_chains(model->fam), L = family_chain_len(model->fam);
-    if (arms == 0) return fail(MPCF_EINVAL, "the fused OCP rows need a compile-time family (chain3/6/7: one arm, forest12x6/14x7: two arms)");
+    // run-time trees: one arm when ee_frame[1] < 0, two otherwise; the frames may sit anywhere in the tree (shared ancestors,
+    // world-fixed).  Compile-time families: the arm count and the arm carrying each frame are fixed by the family.
+    const bool tree = arms == 0;
     RowsHost h;
-    h.narm = arms; h.N = N; h.B = B;
-    for (int a = 0; a < arms; ++a) {
+    h.narm = tree ? (o->ee_frame[1] < 0 ? 1 : 2) : arms;
+    h.N = N; h.B = B;
+    for (int a = 0; a < h.narm; ++a) {
         const int fr = o->ee_frame[a];
         if (fr < 0 || fr >= (int)model->h.fparent.size()) return fail(MPCF_EFRAME, "ocp rows: end-effector frame index out of range");
         const int j = model->h.fparent[fr];
-        if (j < a * L || j >= (a + 1) * L) return fail(MPCF_EFRAME, "ocp rows: ee_frame[" + std::to_string(a) + "] is not carried by arm " + std::to_string(a));
-        h.ee_joint[a] = j - a * L;
+        if (tree) {
+            h.ee_joint[a] = j;  // -1: world-fixed frame
+        } else {
+            if (j < a * L || j >= (a + 1) * L) return fail(MPCF_EFRAME, "ocp rows: ee_frame[" + std::to_string(a) + "] is not carried by arm " + std::to_string(a));
+            h.ee_joint[a] = j - a * L;
+        }
         std::memcpy(h.ee_p[a], &model->h.fp[3 * fr], 3 * sizeof(double));
         std::memcpy(h.ee_R[a], &model->h.fR[9 * fr], 9 * sizeof(double));
     }

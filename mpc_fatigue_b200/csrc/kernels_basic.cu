@@ -1,5 +1,5 @@
 // kernels_basic.cu — RNEA, frame FK, frame Jacobian, reference-mode node evaluation, cost/residual reduction.
-#include "launch.cuh"
+#include "frames.cuh"
 
 namespace mpcf {
 
@@ -43,21 +43,6 @@ struct FkBody {
     }
 };
 
-// column i of the LOCAL_WORLD_ALIGNED frame Jacobian: [z_i x (p_f - o_i); z_i] (revolute), [z_i; 0] (prismatic)
-template <class MP>
-MPCF_DI void jac_column(const MP &m, int i, double (*oR)[9], double (*op)[3], const double *pf, double *col)
-{
-    const double z[3] = {oR[i][2], oR[i][5], oR[i][8]};
-    if (!m.prismatic(i)) {
-        const double d[3] = {pf[0] - op[i][0], pf[1] - op[i][1], pf[2] - op[i][2]};
-        cross3(z, d, col);
-        col[3] = z[0]; col[4] = z[1]; col[5] = z[2];
-    } else {
-        col[0] = z[0]; col[1] = z[1]; col[2] = z[2];
-        col[3] = 0.0; col[4] = 0.0; col[5] = 0.0;
-    }
-}
-
 struct JacBody {
     template <class MP>
     static MPCF_DI void run(const MP &m, long u, long U, FrameArg f, const double *q, double *J)
@@ -87,70 +72,7 @@ struct JacBody {
 //   tau = RNEA(q, qd, qdd) + wsign * sum_e J_e^T W_e ; qnext = q + h qd ; Tnext = ZOH(T; tau, qd, h)
 // (python/2_pilz_6_DOF/Box_Pilz_6DOF2.py:290-293,463 ; python/Centauro_script/mpc_principal.py:267-301)
 // jtw_only: skip RNEA and the integrators and write only J^T W (mpcf_frame_jac_t_wrench_batch).
-// Contact wrenches as external link forces for run-time trees (cf. WrenchExt below for the static chains): the world
-// orientation of every link advances inside the RNEA's forward sweep — carried in registers along chain segments, parked in
-// a local array only for links that others branch off (m.keep) — and the wrench of end-effector e, given in world axes
-// at its frame point, enters link je[e] as [R^T F ; R^T n + p x R^T F].
-template <class MP>
-struct WrenchExtTree {
-    double R[9];
-    double Rk[MP::MAXN][9];
-    int nee;
-    int je[MPCF_MAX_EE];
-    double Wl[MPCF_MAX_EE][6], pl[MPCF_MAX_EE][3];
-    double wsign;
-    MPCF_DI void link(const MP &m, int i, const JointVar<double> &jv, double *f)
-    {
-        if (nee == 0) return;
-        const int par = m.parent(i);
-        double Rp_[9], Rl[9], Rn[9];
-        if (par >= 0 && par != i - 1) {
-#pragma unroll
-            for (int k = 0; k < 9; ++k) Rp_[k] = Rk[par][k];
-        } else {
-#pragma unroll
-            for (int k = 0; k < 9; ++k) Rp_[k] = R[k];
-        }
-        if (!m.prismatic(i)) {
-#pragma unroll
-            for (int r = 0; r < 3; ++r) {
-                Rl[3 * r + 0] = m.Rp(i, 3 * r) * jv.c + m.Rp(i, 3 * r + 1) * jv.s;
-                Rl[3 * r + 1] = m.Rp(i, 3 * r + 1) * jv.c - m.Rp(i, 3 * r) * jv.s;
-                Rl[3 * r + 2] = m.Rp(i, 3 * r + 2);
-            }
-        } else {
-#pragma unroll
-            for (int k = 0; k < 9; ++k) Rl[k] = m.Rp(i, k);
-        }
-#pragma unroll
-        for (int r = 0; r < 3; ++r)
-#pragma unroll
-            for (int c = 0; c < 3; ++c)
-                Rn[3 * r + c] = (par < 0) ? Rl[3 * r + c] : Rp_[3 * r] * Rl[c] + Rp_[3 * r + 1] * Rl[3 + c] + Rp_[3 * r + 2] * Rl[6 + c];
-#pragma unroll
-        for (int k = 0; k < 9; ++k) R[k] = Rn[k];
-        if (m.keep(i)) {
-#pragma unroll
-            for (int k = 0; k < 9; ++k) Rk[i][k] = Rn[k];
-        }
-        for (int e = 0; e < nee; ++e)
-            if (je[e] == i) {
-                double Fl[3], nl[3], t[3];
-#pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    Fl[c] = Rn[c] * Wl[e][0] + Rn[3 + c] * Wl[e][1] + Rn[6 + c] * Wl[e][2];
-                    nl[c] = Rn[c] * Wl[e][3] + Rn[3 + c] * Wl[e][4] + Rn[6 + c] * Wl[e][5];
-                }
-                cross3(pl[e], Fl, t);
-#pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    f[c] += wsign * Fl[c];
-                    f[3 + c] += wsign * (nl[c] + t[c]);
-                }
-            }
-    }
-};
-
+// Run-time trees carry the wrenches through the RNEA sweep (frames.cuh: WrenchExtTree).
 struct NodeEvalBody {
     template <class MP>
     static MPCF_DI void run(const MP &m, long u, long U, EeArgs ee, double wsign, const double *q, const double *qd,

@@ -23,15 +23,28 @@
 // The kinematic rows are written once, generic over the scalar (double | Dual); k_rows_kin_jac evaluates them with one
 // dual-number seed per launch row (blockIdx.y = direction in (q, F)) and gives d rows / d (q, F).  The torque rows'
 // derivatives come from mpcf_node_eval_ref_jvp_batch (analytic) and d tau / d F, d T+ / d tau are emitted here in closed form.
-// Static families only (chain3/6/7: one arm; forest12x6 / forest14x7: two arms).  Oracle twin: oracle/core.inc.h: ocp_rows.
-#include "launch.cuh"
+//
+// Two paths, one row function:
+//   compile-time families (chain3/6/7: one arm; forest12x6 / forest14x7: two arms): k_ocp_rows + k_rows_kin_jac, arm by arm.
+//   run-time trees (generic16 / generic64: branched trees, prismatic and continuous joints, shared ancestors such as a torso
+//   joint under both arms; one or two end-effector frames): RowsTreeBody and RowsTreeJacBody, thread per unit through
+//   dispatch_generic.  RowsTreeBody runs ONE RNEA sweep with the forces injected as external link forces (frames.cuh:
+//   WrenchExtTree, which also captures both frame poses on the way), so tau = ID + wsign (J_L^T [F_L;0] + J_R^T [F_R;0]) sums
+//   both terms on shared ancestors without an explicit Jacobian; the previous node's relative position walks the two frames'
+//   ancestor paths only.  RowsTreeJacBody computes the poses of the frames' ancestors once, takes their Jacobian columns
+//   (d tau / d F = wsign J_c,lin^T, non-zero in both arm blocks on shared ancestors) and evaluates box_kin_rows<Dual> once per
+//   direction seeded with the pose tangent (q_j: dp_c = J_c,lin[:, j], dR_c = [J_c,ang[:, j]]x R_c, zero when j is not an
+//   ancestor of frame c; F: the force entry itself) — no frame kinematics per direction.  A world-fixed frame (no parent
+//   joint) has a constant pose and a zero Jacobian.
+// Oracle twin: oracle/core.inc.h: ocp_rows.
+#include "frames.cuh"
 
 namespace mpcf {
 
 struct RowsArgs {
     int narm, n, N;
     long B;
-    int ee_joint[2];     // end-effector joint, local to its arm
+    int ee_joint[2];     // end-effector joint: local to its arm (compile-time families), global index or -1 = world (trees)
     double ee_p[2][3], ee_R[2][9];
     double wsign, fdes[3], dist2_ref, mu, p_ref[3], w_box, w_qd, w_F, h;
 };
@@ -278,6 +291,191 @@ __global__ void __launch_bounds__(kThreads) k_rows_kin_jac(const __grid_constant
     for (int r = 0; r < KIN; ++r) out[((long)r * ND + d) * U + u] = g[r].d;
 }
 
+// ---- run-time trees (header comment).  Arm c's frame: a.ee_joint[c] (global joint, -1 = world-fixed), a.ee_p / a.ee_R[c].
+
+// rows, cost and (optional) d T+ / d tau: one RNEA sweep with the forces as external link forces
+struct RowsTreeBody {
+    template <class MP>
+    static MPCF_DI void run(const MP &m, long u, long U, RowsArgs a, const double *q, const double *qd, const double *F, const double *T,
+                            const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
+                            double *cost, double *dT_dtau)
+    {
+        const int n = m.n(), narm = a.narm, KIN = narm == 2 ? 26 : 3;
+        const long b = u % a.B;
+        const int k = (int)(u / a.B);
+        double qa[MP::MAXN], qda[MP::MAXN], zero[MP::MAXN], tau[MP::MAXN];
+        double cqd = 0.0, cF = 0.0, ckin = 0.0;
+#pragma unroll 1
+        for (int i = 0; i < n; ++i) {
+            qa[i] = q[(long)i * U + u];
+            qda[i] = qd[(long)i * U + u];
+            zero[i] = 0.0;
+            cqd += qda[i] * qda[i];
+        }
+        double Fv[6];
+#pragma unroll
+        for (int i = 0; i < 6; ++i) {
+            Fv[i] = i < 3 * narm ? F[(long)i * U + u] : 0.0;
+            cF += Fv[i] * Fv[i];
+        }
+        WrenchExtTree<MP, true> ext;
+        ext.nee = narm;
+        ext.wsign = a.wsign;
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+            if (c >= narm) break;
+            ext.je[c] = a.ee_joint[c];  // -1 (world-fixed frame) never matches a link: no torque, the constant pose stays
+#pragma unroll
+            for (int r = 0; r < 3; ++r) {
+                ext.Wl[c][r] = Fv[3 * c + r];
+                ext.Wl[c][3 + r] = 0.0;
+                ext.pl[c][r] = a.ee_p[c][r];
+                ext.Pw[c][r] = a.ee_p[c][r];
+            }
+#pragma unroll
+            for (int r = 0; r < 9; ++r) { ext.Rf[c][r] = a.ee_R[c][r]; ext.Rw[c][r] = a.ee_R[c][r]; }
+        }
+        JointVar<double> jv[MP::MAXN];
+        Dyn<double, MP>::template rnea_impl<false>(m, qa, jv, qda, zero, tau, ext);
+#pragma unroll 1
+        for (int i = 0; i < n; ++i) {
+            const double t = tau[i];
+            rows[(long)(KIN + i) * U + u] = t;
+            // Euler defect against the next node's q (last node: the trailing q_N)
+            const double qn = qa[i] + a.h * qda[i];
+            const double qnext = k + 1 < a.N ? q[(long)i * U + u + a.B] : (q_last ? q_last[(long)i * a.B + b] : qn);
+            rows[(long)(KIN + n + i) * U + u] = qn - qnext;
+            double Tdef = 0.0, dTdt = 0.0;
+            if (T) {
+                const double lam = m.fat(i, 0), kap = m.fat(i, 1);
+                const double Pl = m.fat(i, 2) * t * t + m.fat(i, 3) * qda[i] * qda[i];
+                const double Ti = T[(long)i * U + u];
+                const double za = exp(-lam * a.h);
+                const double gain = lam == 0.0 ? a.h * kap : (1.0 - za) * (kap / lam);
+                const double Tn = za * Ti + gain * Pl;
+                const double Tnext = k + 1 < a.N ? T[(long)i * U + u + a.B] : (T_last ? T_last[(long)i * a.B + b] : Tn);
+                Tdef = Tn - Tnext;
+                dTdt = gain * 2.0 * m.fat(i, 2) * t;
+            }
+            rows[(long)(KIN + 2 * n + i) * U + u] = Tdef;
+            if (dT_dtau) dT_dtau[(long)i * U + u] = dTdt;
+        }
+        if (narm == 2) {
+            double relprev[3], ori0[3], g[26];
+            if (k == 0) {
+#pragma unroll
+                for (int r = 0; r < 3; ++r) relprev[r] = rel_pos0 ? rel_pos0[(long)r * a.B + b] : 0.0;
+            } else {  // the same quantity at the previous node (unit u - B): the two frames' ancestor paths only
+                double pL[3], RL[9], pR[3], RR[9];
+                frame_pose_walk(m, a.ee_joint[0], a.ee_R[0], a.ee_p[0], q, U, u - a.B, pL, RL);
+                frame_pose_walk(m, a.ee_joint[1], a.ee_R[1], a.ee_p[1], q, U, u - a.B, pR, RR);
+#pragma unroll
+                for (int r = 0; r < 3; ++r) relprev[r] = RL[r] * (pR[0] - pL[0]) + RL[3 + r] * (pR[1] - pL[1]) + RL[6 + r] * (pR[2] - pL[2]);
+            }
+#pragma unroll
+            for (int r = 0; r < 3; ++r) ori0[r] = rel_ori0 ? rel_ori0[(long)r * a.B + b] : 0.0;
+            box_kin_rows<double>(a, ext.Pw[0], ext.Rw[0], ext.Pw[1], ext.Rw[1], Fv, Fv + 3, relprev, ori0, g);
+#pragma unroll
+            for (int r = 0; r < 26; ++r) rows[(long)r * U + u] = g[r];
+            ckin = g[23] * g[23] + g[24] * g[24] + g[25] * g[25];
+        } else {
+#pragma unroll
+            for (int r = 0; r < 3; ++r) rows[(long)r * U + u] = ext.Pw[0][r] - a.p_ref[r];
+        }
+        cost[u] = a.w_box * ckin + a.w_qd * cqd + a.w_F * cF;
+    }
+};
+
+// dtau_dF [n][3 narm][U] and kin_jac [KIN][n + 3 narm][U] (either may be NULL): frame kinematics of the two frames' ancestors
+// once, then one box_kin_rows<Dual> per direction seeded with the pose tangent
+struct RowsTreeJacBody {
+    template <class MP>
+    static MPCF_DI void run(const MP &m, long u, long U, RowsArgs a, const double *q, const double *F, double *dtau_dF, double *kin_jac)
+    {
+        const int n = m.n(), narm = a.narm, KIN = narm == 2 ? 26 : 3, ND = n + 3 * narm;
+        unsigned long long anc[2] = {0ull, 0ull};  // ancestor sets of the frames (bit j: joint j moves frame c)
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+            if (c >= narm) break;
+            for (int j = a.ee_joint[c]; j >= 0; j = m.parent(j)) anc[c] |= 1ull << j;
+        }
+        const unsigned long long both = anc[0] | anc[1];
+        double oR[MP::MAXN][9], op[MP::MAXN][3];
+        fk_subset(m, both, q, U, u, oR, op);
+        double pe[2][3], Re[2][9], Fv[6];
+#pragma unroll
+        for (int c = 0; c < 2; ++c) {
+            const int cc = c < narm ? c : 0;
+            Dyn<double, MP>::frame_pose(a.ee_joint[cc], a.ee_R[cc], a.ee_p[cc], oR, op, pe[c], Re[c]);
+        }
+#pragma unroll
+        for (int i = 0; i < 6; ++i) Fv[i] = i < 3 * narm ? F[(long)i * U + u] : 0.0;
+        if (dtau_dF) {
+#pragma unroll 1
+            for (int j = 0; j < n; ++j) {
+#pragma unroll
+                for (int c = 0; c < 2; ++c) {
+                    if (c >= narm) break;
+                    double col[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+                    if ((anc[c] >> j) & 1ull) jac_column(m, j, oR, op, pe[c], col);
+#pragma unroll
+                    for (int r = 0; r < 3; ++r) dtau_dF[((long)j * 3 * narm + 3 * c + r) * U + u] = a.wsign * col[r];
+                }
+            }
+        }
+        if (!kin_jac) return;
+        const long ld = (long)ND * U;  // stride between the rows of one direction
+        const Dual relprev[3] = {Dual(0.0), Dual(0.0), Dual(0.0)};
+        const double ori0[3] = {0.0, 0.0, 0.0};
+#pragma unroll 1
+        for (int d = 0; d < ND; ++d) {
+            double *out = kin_jac + (long)d * U + u;
+            if (d < n && !((both >> d) & 1ull)) {  // joint d moves neither frame
+                for (int r = 0; r < KIN; ++r) out[r * ld] = 0.0;
+                continue;
+            }
+            if (narm == 1) {  // rows p - p_ref: J_lin, nothing in F
+                double col[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+                if (d < n) jac_column(m, d, oR, op, pe[0], col);
+#pragma unroll
+                for (int r = 0; r < 3; ++r) out[r * ld] = col[r];
+                continue;
+            }
+            Dual pd[2][3], Rd[2][9], Fd[6], g[26];
+#pragma unroll
+            for (int c = 0; c < 2; ++c) {
+                double col[6] = {0.0, 0.0, 0.0, 0.0, 0.0, 0.0};
+                if (d < n && ((anc[c] >> d) & 1ull)) jac_column(m, d, oR, op, pe[c], col);
+#pragma unroll
+                for (int r = 0; r < 3; ++r) pd[c][r] = Dual(pe[c][r], col[r]);
+#pragma unroll
+                for (int cc = 0; cc < 3; ++cc) {  // d R = [w]x R, column by column
+                    const double rc[3] = {Re[c][cc], Re[c][3 + cc], Re[c][6 + cc]};
+                    double dr[3];
+                    cross3(col + 3, rc, dr);
+#pragma unroll
+                    for (int r = 0; r < 3; ++r) Rd[c][3 * r + cc] = Dual(Re[c][3 * r + cc], dr[r]);
+                }
+            }
+#pragma unroll
+            for (int i = 0; i < 6; ++i) Fd[i] = Dual(Fv[i], d == n + i ? 1.0 : 0.0);
+            box_kin_rows<Dual>(a, pd[0], Rd[0], pd[1], Rd[1], Fd, Fd + 3, relprev, ori0, g);
+#pragma unroll
+            for (int r = 0; r < 26; ++r) out[r * ld] = g[r].d;
+        }
+    }
+};
+
+static cudaError_t rows_tree_launch(const LaunchModel &m, const RowsArgs &a, const double *q, const double *qd, const double *F, const double *T,
+                                    const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
+                                    double *cost, double *dtau_dF, double *dT_dtau, double *kin_jac, cudaStream_t s)
+{
+    const long U = a.B * a.N;
+    cudaError_t e = dispatch_generic<RowsTreeBody>(m, U, 1, s, a, q, qd, F, T, q_last, T_last, rel_pos0, rel_ori0, rows, cost, dT_dtau);
+    if (e != cudaSuccess || !(dtau_dF || kin_jac)) return e;
+    return dispatch_generic<RowsTreeJacBody>(m, U, 1, s, a, q, F, dtau_dF, kin_jac);
+}
+
 template <int L, int NARM>
 static cudaError_t rows_launch(const StaticParams<L> *cp, const RowsArgs &a, const double *q, const double *qd, const double *F, const double *T,
                                const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
@@ -316,6 +514,8 @@ cudaError_t launch_ocp_rows(const LaunchModel &m, const RowsHost &h, const doubl
     case FAM_CHAIN7: return rows_launch<7, 1>(static_cast<const StaticParams<7> *>(m.static_params), ROWS_ARGS);
     case FAM_FOREST12x6: return rows_launch<6, 2>(static_cast<const StaticParams<6> *>(m.chain_params), ROWS_ARGS);
     case FAM_FOREST14x7: return rows_launch<7, 2>(static_cast<const StaticParams<7> *>(m.chain_params), ROWS_ARGS);
+    case FAM_GENERIC16:
+    case FAM_GENERIC64: return rows_tree_launch(m, ROWS_ARGS);
     default: return cudaErrorInvalidValue;
     }
 #undef ROWS_ARGS

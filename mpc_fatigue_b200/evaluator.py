@@ -282,14 +282,26 @@ class BatchEvaluator:
                  fdes=(0.0, 0.0, 0.0), dist2_ref=0.0, mu=0.0, p_ref=(0.0, 0.0, 0.0), w_box=0.0, w_qd=0.0, w_F=0.0, h=0.0, derivatives=False):
         """Fused reference-mode OCP node rows (include/mpcf.h: mpcf_ocp_rows_batch): every constraint row + the running cost of
         the reference's per-node loops in one launch.  Returns (rows [nrows, U], cost [U]) and, with derivatives=True, also
-        (dtau_dF [n, 3 arms, U], dT_dtau [n, U], kin_jac [26 | 3, n + 3 arms, U])."""
+        (dtau_dF [n, 3 arms, U], dT_dtau [n, U], kin_jac [26 | 3, n + 3 arms, U]).
+        Compile-time families fix the arm count (chain3/6/7: one frame, forest12x6/14x7: two); on run-time trees (branched
+        trees, prismatic joints) the arm count is len(ee_frames), one or two, and the frames may share ancestors."""
         n, U = self.n, B * N
-        nrows = int(_capi.lib.mpcf_ocp_rows_count(self.model.handle))
+        if self.model.kernel_family.startswith("generic"):
+            narm = len(ee_frames)
+            if narm not in (1, 2):
+                raise ValueError("the OCP rows need one or two end-effector frames, got %d" % narm)
+        else:
+            nrows = int(_capi.lib.mpcf_ocp_rows_count(self.model.handle))
+            _capi.check(nrows)
+            narm = 2 if nrows == 26 + 3 * n else 1
+            if len(ee_frames) != narm:
+                raise ValueError("this model needs %d end-effector frame(s)" % narm)
+        nrows = int(_capi.lib.mpcf_ocp_rows_count_arms(self.model.handle, narm))
         _capi.check(nrows)
-        narm = 2 if nrows == 26 + 3 * n else 1
-        if len(ee_frames) != narm:
-            raise ValueError("this model needs %d end-effector frame(s)" % narm)
-        fr = [self.model.frame_id(f) if isinstance(f, str) else int(f) for f in ee_frames] + [0] * (2 - narm)
+        fr = [self.model.frame_id(f) if isinstance(f, str) else int(f) for f in ee_frames]
+        if any(f < 0 for f in fr):  # a negative second frame would mean "one arm" to the library
+            raise IndexError("end-effector frame index out of range: %s" % fr)
+        fr += [-1] * (2 - narm)
         o = _capi.RowsOpts((C.c_int * 2)(*fr), float(wsign), (C.c_double * 3)(*[float(v) for v in fdes]), float(dist2_ref), float(mu),
                            (C.c_double * 3)(*[float(v) for v in p_ref]), float(w_box), float(w_qd), float(w_F), float(h))
         f64 = dict(dtype=torch.float64, device=self.device)
