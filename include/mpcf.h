@@ -213,7 +213,8 @@ int mpcf_cost_residual_table_batch(const mpcf_model *model, long B, int N, const
                                    double f_max, double *out, long ld_out, void *stream);
 
 /* Fused reference-mode OCP node rows: every constraint row and the running cost the reference's scripts build per shooting
-   node, one launch for B scenarios x N nodes (node-major units u = k*B + b).  Every kernel family:
+   node, one launch for B scenarios x N nodes (node-major units u = k*B + b).  The same kernel serves every family; the
+   families differ only in how the arm count is set and which frames they accept:
      compile-time families: chain3/6/7 have one arm, forest12x6 / forest14x7 two (opts->ee_frame[1] is ignored on the
        one-arm chains); ee_frame[c] must be carried by arm c (MPCF_EFRAME otherwise, world-fixed frames included).
      run-time trees (generic16 / generic64: branched trees, prismatic and continuous joints, up to 64 DOF): one arm when

@@ -702,13 +702,10 @@ extern "C" int mpcf_ocp_rows_batch(const mpcf_model *model, const mpcf_rows_opts
     for (int a = 0; a < h.narm; ++a) {
         const int fr = o->ee_frame[a];
         if (fr < 0 || fr >= (int)model->h.fparent.size()) return fail(MPCF_EFRAME, "ocp rows: end-effector frame index out of range");
-        const int j = model->h.fparent[fr];
-        if (tree) {
-            h.ee_joint[a] = j;  // -1: world-fixed frame
-        } else {
-            if (j < a * L || j >= (a + 1) * L) return fail(MPCF_EFRAME, "ocp rows: ee_frame[" + std::to_string(a) + "] is not carried by arm " + std::to_string(a));
-            h.ee_joint[a] = j - a * L;
-        }
+        const int j = model->h.fparent[fr];  // -1: world-fixed frame
+        if (!tree && (j < a * L || j >= (a + 1) * L))
+            return fail(MPCF_EFRAME, "ocp rows: ee_frame[" + std::to_string(a) + "] is not carried by arm " + std::to_string(a));
+        h.ee_joint[a] = j;
         std::memcpy(h.ee_p[a], &model->h.fp[3 * fr], 3 * sizeof(double));
         std::memcpy(h.ee_R[a], &model->h.fR[9 * fr], 9 * sizeof(double));
     }

@@ -1,5 +1,5 @@
-// frames.cuh — frame kinematics shared by the reference-mode node evaluation (kernels_basic.cu) and the fused OCP rows of
-// run-time trees (kernels_rows.cu): Jacobian columns, contact wrenches riding the RNEA sweep, and frame poses by ancestor walk.
+// frames.cuh — frame kinematics shared by the reference-mode node evaluation (kernels_basic.cu) and the fused OCP rows
+// (kernels_rows.cu): Jacobian columns, contact wrenches riding the RNEA sweep, and frame poses by ancestor walk.
 #pragma once
 #include "launch.cuh"
 
@@ -20,7 +20,7 @@ MPCF_DI void jac_column(const MP &m, int i, double (*oR)[9], double (*op)[3], co
     }
 }
 
-// Contact wrenches as external link forces for run-time trees (cf. WrenchExt for the static chains): the world
+// Contact wrenches as external link forces for run-time trees and the OCP rows of every family (cf. WrenchExt): the world
 // orientation of every link advances inside the RNEA's forward sweep — carried in registers along chain segments, parked in
 // a local array only for links that others branch off (m.keep) — and the wrench of end-effector e, given in world axes
 // at its frame point, enters link je[e] as [R^T F ; R^T n + p x R^T F].
@@ -96,30 +96,37 @@ struct WrenchExtTree : PoseTrack<MP::MAXN, kPose> {
 #pragma unroll
             for (int k = 0; k < 9; ++k) Rk[i][k] = Rn[k];
         }
-        for (int e = 0; e < nee; ++e)
-            if (je[e] == i) {
-                double Fl[3], nl[3], t[3];
+        auto frame = [&](int e) {
+            double Fl[3], nl[3], t[3];
 #pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    Fl[c] = Rn[c] * Wl[e][0] + Rn[3 + c] * Wl[e][1] + Rn[6 + c] * Wl[e][2];
-                    nl[c] = Rn[c] * Wl[e][3] + Rn[3 + c] * Wl[e][4] + Rn[6 + c] * Wl[e][5];
-                }
-                cross3(pl[e], Fl, t);
+            for (int c = 0; c < 3; ++c) {
+                Fl[c] = Rn[c] * Wl[e][0] + Rn[3 + c] * Wl[e][1] + Rn[6 + c] * Wl[e][2];
+                nl[c] = Rn[c] * Wl[e][3] + Rn[3 + c] * Wl[e][4] + Rn[6 + c] * Wl[e][5];
+            }
+            cross3(pl[e], Fl, t);
 #pragma unroll
-                for (int c = 0; c < 3; ++c) {
-                    f[c] += wsign * Fl[c];
-                    f[3 + c] += wsign * (nl[c] + t[c]);
-                }
-                if constexpr (kPose) {
+            for (int c = 0; c < 3; ++c) {
+                f[c] += wsign * Fl[c];
+                f[3 + c] += wsign * (nl[c] + t[c]);
+            }
+            if constexpr (kPose) {
 #pragma unroll
-                    for (int r = 0; r < 3; ++r) {
-                        this->Pw[e][r] = this->p[r] + Rn[3 * r] * pl[e][0] + Rn[3 * r + 1] * pl[e][1] + Rn[3 * r + 2] * pl[e][2];
+                for (int r = 0; r < 3; ++r) {
+                    this->Pw[e][r] = this->p[r] + Rn[3 * r] * pl[e][0] + Rn[3 * r + 1] * pl[e][1] + Rn[3 * r + 2] * pl[e][2];
 #pragma unroll
-                        for (int c = 0; c < 3; ++c)
-                            this->Rw[e][3 * r + c] = Rn[3 * r] * this->Rf[e][c] + Rn[3 * r + 1] * this->Rf[e][3 + c] + Rn[3 * r + 2] * this->Rf[e][6 + c];
-                    }
+                    for (int c = 0; c < 3; ++c)
+                        this->Rw[e][3 * r + c] = Rn[3 * r] * this->Rf[e][c] + Rn[3 * r + 1] * this->Rf[e][3 + c] + Rn[3 * r + 2] * this->Rf[e][6 + c];
                 }
             }
+        };
+        if constexpr (MP::kStatic) {  // a fixed trip count: the frame arrays index at compile time and stay in registers
+#pragma unroll
+            for (int e = 0; e < MPCF_MAX_EE; ++e)
+                if (e < nee && je[e] == i) frame(e);
+        } else {
+            for (int e = 0; e < nee; ++e)
+                if (je[e] == i) frame(e);
+        }
     }
 };
 

@@ -109,7 +109,7 @@ cudaError_t launch_fd_derivs(const LaunchModel &m, long U, const double *q, cons
 struct RowsHost {
     int narm = 1, N = 0;
     long B = 0;
-    int ee_joint[2] = {0, 0};
+    int ee_joint[2] = {0, 0};  // end-effector joint: global index, -1 = world-fixed frame
     double ee_p[2][3] = {{0, 0, 0}, {0, 0, 0}}, ee_R[2][9] = {{1, 0, 0, 0, 1, 0, 0, 0, 1}, {1, 0, 0, 0, 1, 0, 0, 0, 1}};
     double wsign = -1.0, fdes[3] = {0, 0, 0}, dist2_ref = 0.0, mu = 0.0, p_ref[3] = {0, 0, 0}, w_box = 0.0, w_qd = 0.0, w_F = 0.0, h = 0.0;
 };

@@ -20,22 +20,19 @@
 //        then tau (n), Euler defect (n), thermal defect (n) as above, with tau = ID + wsign (J_L^T [F_L;0] + J_R^T [F_R;0])
 //        cost       w_box |p_box - p_ref|^2 + w_qd qd.qd + w_F (F_L.F_L + F_R.F_R)                 (mpc_principal.py:281-284)
 //
-// The kinematic rows are written once, generic over the scalar (double | Dual); k_rows_kin_jac evaluates them with one
-// dual-number seed per launch row (blockIdx.y = direction in (q, F)) and gives d rows / d (q, F).  The torque rows'
-// derivatives come from mpcf_node_eval_ref_jvp_batch (analytic) and d tau / d F, d T+ / d tau are emitted here in closed form.
-//
-// Two paths, one row function:
-//   compile-time families (chain3/6/7: one arm; forest12x6 / forest14x7: two arms): k_ocp_rows + k_rows_kin_jac, arm by arm.
-//   run-time trees (generic16 / generic64: branched trees, prismatic and continuous joints, shared ancestors such as a torso
-//   joint under both arms; one or two end-effector frames): RowsTreeBody and RowsTreeJacBody, thread per unit through
-//   dispatch_generic.  RowsTreeBody runs ONE RNEA sweep with the forces injected as external link forces (frames.cuh:
-//   WrenchExtTree, which also captures both frame poses on the way), so tau = ID + wsign (J_L^T [F_L;0] + J_R^T [F_R;0]) sums
-//   both terms on shared ancestors without an explicit Jacobian; the previous node's relative position walks the two frames'
-//   ancestor paths only.  RowsTreeJacBody computes the poses of the frames' ancestors once, takes their Jacobian columns
-//   (d tau / d F = wsign J_c,lin^T, non-zero in both arm blocks on shared ancestors) and evaluates box_kin_rows<Dual> once per
-//   direction seeded with the pose tangent (q_j: dp_c = J_c,lin[:, j], dR_c = [J_c,ang[:, j]]x R_c, zero when j is not an
-//   ancestor of frame c; F: the force entry itself) — no frame kinematics per direction.  A world-fixed frame (no parent
-//   joint) has a constant pose and a zero Jacobian.
+// One pair of thread-per-unit bodies serves every kernel family through dispatch: the compile-time chains and forests and
+// the run-time trees (branched trees, prismatic and continuous joints, shared ancestors such as a torso joint under both
+// arms).  Arm c's frame sits on joint a.ee_joint[c] (global index, -1 = world-fixed: constant pose, zero Jacobian).
+//   RowsBody runs ONE RNEA sweep with the forces injected as external link forces (frames.cuh: WrenchExtTree, which also
+//   captures both frame poses on the way), so tau = ID + wsign (J_L^T [F_L;0] + J_R^T [F_R;0]) sums both terms on shared
+//   ancestors without an explicit Jacobian; the previous node's relative position walks the two frames' ancestor paths only.
+//   RowsJacBody (launched only when dtau_dF or kin_jac is requested) computes the poses of the frames' ancestors once, takes
+//   their Jacobian columns (d tau / d F = wsign J_c,lin^T, non-zero in both arm blocks on shared ancestors) and evaluates the
+//   kinematic rows (box_kin_rows, generic over double | Dual) once per direction in (q, F), seeded with the pose tangent
+//   (q_j: dp_c = J_c,lin[:, j], dR_c = [J_c,ang[:, j]]x R_c, zero when j is not an ancestor of frame c; F: the force entry
+//   itself) — no frame kinematics per direction.
+// The torque rows' derivatives in (q, qd) come from mpcf_node_eval_ref_jvp_batch (analytic); d tau / d F and d T+ / d tau are
+// emitted here in closed form.
 // Oracle twin: oracle/core.inc.h: ocp_rows.
 #include "frames.cuh"
 
@@ -44,58 +41,9 @@ namespace mpcf {
 struct RowsArgs {
     int narm, n, N;
     long B;
-    int ee_joint[2];     // end-effector joint: local to its arm (compile-time families), global index or -1 = world (trees)
+    int ee_joint[2];     // end-effector joint: global index, -1 = world-fixed frame
     double ee_p[2][3], ee_R[2][9];
     double wsign, fdes[3], dist2_ref, mu, p_ref[3], w_box, w_qd, w_F, h;
-};
-
-// world pose of the end-effector frame of one serial arm and, for T = double callers that ask, the joint axes / origins
-template <class T, int L>
-struct ArmFk {
-    T pos[3], rot[9];
-    T z[L][3], o[L][3];
-    MPCF_DI void run(const StaticParams<L> &P, const T *q, int ej, const double *ep, const double *eR)
-    {
-        T R[9], p[3];
-#pragma unroll
-        for (int i = 0; i < L; ++i) {
-            T s, c;
-            sincos_t(q[i], s, c);
-            T Rl[9];
-#pragma unroll
-            for (int r = 0; r < 3; ++r) {
-                Rl[3 * r + 0] = P.Rp[i][3 * r] * c + P.Rp[i][3 * r + 1] * s;
-                Rl[3 * r + 1] = P.Rp[i][3 * r + 1] * c - P.Rp[i][3 * r] * s;
-                Rl[3 * r + 2] = T(P.Rp[i][3 * r + 2]);
-            }
-            if (i == 0) {
-#pragma unroll
-                for (int k = 0; k < 9; ++k) R[k] = Rl[k];
-#pragma unroll
-                for (int k = 0; k < 3; ++k) p[k] = T(P.pp[i][k]);
-            } else {
-                T Rn[9];
-#pragma unroll
-                for (int r = 0; r < 3; ++r) {
-                    p[r] = p[r] + (R[3 * r] * P.pp[i][0] + R[3 * r + 1] * P.pp[i][1] + R[3 * r + 2] * P.pp[i][2]);
-#pragma unroll
-                    for (int cc = 0; cc < 3; ++cc) Rn[3 * r + cc] = R[3 * r] * Rl[cc] + R[3 * r + 1] * Rl[3 + cc] + R[3 * r + 2] * Rl[6 + cc];
-                }
-#pragma unroll
-                for (int k = 0; k < 9; ++k) R[k] = Rn[k];
-            }
-#pragma unroll
-            for (int k = 0; k < 3; ++k) { z[i][k] = R[3 * k + 2]; o[i][k] = p[k]; }
-            if (i == ej) {
-#pragma unroll
-                for (int r = 0; r < 3; ++r) {
-                    pos[r] = p[r] + (R[3 * r] * ep[0] + R[3 * r + 1] * ep[1] + R[3 * r + 2] * ep[2]);
-#pragma unroll
-                    for (int cc = 0; cc < 3; ++cc) rot[3 * r + cc] = R[3 * r] * eR[cc] + R[3 * r + 1] * eR[3 + cc] + R[3 * r + 2] * eR[6 + cc];
-                }
-            }
-        }
-    }
 };
 
 // the 26 kinematic rows of the two-arm node (header comment) from the two end-effector poses and the two forces
@@ -138,174 +86,28 @@ MPCF_DI void box_kin_rows(const RowsArgs &a, const T *pL, const T *RL, const T *
     for (int k = 0; k < 3; ++k) g[23 + k] = 0.5 * (pL[k] + pR[k]) - a.p_ref[k];
 }
 
-template <int L, int NARM>
-__global__ void __launch_bounds__(kThreads) k_ocp_rows(const __grid_constant__ StaticParams<L> P0, const __grid_constant__ StaticParams<L> P1,
-                                                      RowsArgs a, const double *q, const double *qd, const double *F, const double *T,
-                                                      const double *q_last, const double *T_last, const double *rel_pos0,
-                                                      const double *rel_ori0, double *rows, double *cost, double *dtau_dF, double *dT_dtau)
+// the arm count: fixed by a compile-time family (one per serial chain), so its instantiations carry no code for the other
+template <class MP>
+MPCF_DI int arms(const RowsArgs &a)
 {
-    const long U = a.B * a.N;
-    const long u = (long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (u >= U) return;
-    constexpr int n = NARM * L;
-    const long b = u % a.B;
-    const int k = (int)(u / a.B);
-    constexpr int KIN = NARM == 2 ? 26 : 3;
-    double Fv[3 * NARM];
-#pragma unroll
-    for (int i = 0; i < 3 * NARM; ++i) Fv[i] = F[(long)i * U + u];
-    double ckin = 0.0, cqd = 0.0, cF = 0.0;
-#pragma unroll
-    for (int i = 0; i < 3 * NARM; ++i) cF += Fv[i] * Fv[i];
-    double pe[NARM][3], Re[NARM][9];
-#pragma unroll
-    for (int c = 0; c < NARM; ++c) {
-        const StaticParams<L> &P = c == 0 ? P0 : P1;
-        const StaticModel<L, L> m{P};
-        double qa[L], qda[L], zero[L], tau[L];
-#pragma unroll
-        for (int i = 0; i < L; ++i) { qa[i] = q[(long)(c * L + i) * U + u]; qda[i] = qd[(long)(c * L + i) * U + u]; zero[i] = 0.0; cqd += qda[i] * qda[i]; }
-        ArmFk<double, L> K;
-        K.run(P, qa, a.ee_joint[c], a.ee_p[c], a.ee_R[c]);
-#pragma unroll
-        for (int r = 0; r < 3; ++r) pe[c][r] = K.pos[r];
-#pragma unroll
-        for (int r = 0; r < 9; ++r) Re[c][r] = K.rot[r];
-        Dyn<double, StaticModel<L, L>>::rnea(m, qa, qda, zero, tau);
-        const double *Fc = Fv + 3 * c;
-#pragma unroll
-        for (int i = 0; i < L; ++i) {
-            // column i of the frame Jacobian (linear part): z_i x (p_ee - o_i), zero past the end-effector joint
-            double col[3] = {0.0, 0.0, 0.0};
-            if (i <= a.ee_joint[c]) {
-                const double d[3] = {K.pos[0] - K.o[i][0], K.pos[1] - K.o[i][1], K.pos[2] - K.o[i][2]};
-                cross3(K.z[i], d, col);
-            }
-            const double t = tau[i] + a.wsign * (col[0] * Fc[0] + col[1] * Fc[1] + col[2] * Fc[2]);
-            const long row = KIN + c * L + i;
-            rows[row * U + u] = t;
-            if (dtau_dF) {
-#pragma unroll
-                for (int r = 0; r < 3; ++r) dtau_dF[((long)(c * L + i) * 3 * NARM + 3 * c + r) * U + u] = a.wsign * col[r];
-                if (NARM == 2) {
-#pragma unroll
-                    for (int r = 0; r < 3; ++r) dtau_dF[((long)(c * L + i) * 3 * NARM + 3 * (1 - c) + r) * U + u] = 0.0;
-                }
-            }
-            // Euler defect against the next node's q (last node: the trailing q_N)
-            const double qn = qa[i] + a.h * qda[i];
-            const double qnext = k + 1 < a.N ? q[(long)(c * L + i) * U + u + a.B] : (q_last ? q_last[(long)(c * L + i) * a.B + b] : qn);
-            rows[(row + n) * U + u] = qn - qnext;
-            double Tdef = 0.0, dTdt = 0.0;
-            if (T) {
-                const double lam = P.fat[i][0], kap = P.fat[i][1];
-                const double Pl = P.fat[i][2] * t * t + P.fat[i][3] * qda[i] * qda[i];
-                const double Ti = T[(long)(c * L + i) * U + u];
-                const double za = exp(-lam * a.h);
-                const double gain = lam == 0.0 ? a.h * kap : (1.0 - za) * (kap / lam);
-                const double Tn = za * Ti + gain * Pl;
-                const double Tnext = k + 1 < a.N ? T[(long)(c * L + i) * U + u + a.B] : (T_last ? T_last[(long)(c * L + i) * a.B + b] : Tn);
-                Tdef = Tn - Tnext;
-                dTdt = gain * 2.0 * P.fat[i][2] * t;
-            }
-            rows[(row + 2 * n) * U + u] = Tdef;
-            if (dT_dtau) dT_dtau[(long)(c * L + i) * U + u] = dTdt;
-        }
-    }
-    if (NARM == 2) {
-        double relprev[3], ori0[3], g[26];
-        if (k == 0) {
-#pragma unroll
-            for (int r = 0; r < 3; ++r) relprev[r] = rel_pos0 ? rel_pos0[(long)r * a.B + b] : 0.0;
-        } else {  // the same quantity at the previous node (its unit is u - B): frame kinematics only
-            double pp[2][3], Rl0[9];
-#pragma unroll
-            for (int c = 0; c < 2; ++c) {
-                const StaticParams<L> &P = c == 0 ? P0 : P1;
-                double qa[L];
-#pragma unroll
-                for (int i = 0; i < L; ++i) qa[i] = q[(long)(c * L + i) * U + u - a.B];
-                ArmFk<double, L> K;
-                K.run(P, qa, a.ee_joint[c], a.ee_p[c], a.ee_R[c]);
-#pragma unroll
-                for (int r = 0; r < 3; ++r) pp[c][r] = K.pos[r];
-                if (c == 0) {
-#pragma unroll
-                    for (int r = 0; r < 9; ++r) Rl0[r] = K.rot[r];
-                }
-            }
-#pragma unroll
-            for (int r = 0; r < 3; ++r) relprev[r] = Rl0[r] * (pp[1][0] - pp[0][0]) + Rl0[3 + r] * (pp[1][1] - pp[0][1]) + Rl0[6 + r] * (pp[1][2] - pp[0][2]);
-        }
-#pragma unroll
-        for (int r = 0; r < 3; ++r) ori0[r] = rel_ori0 ? rel_ori0[(long)r * a.B + b] : 0.0;
-        box_kin_rows<double>(a, pe[0], Re[0], pe[NARM - 1], Re[NARM - 1], Fv, Fv + 3 * (NARM - 1), relprev, ori0, g);
-#pragma unroll
-        for (int r = 0; r < 26; ++r) rows[(long)r * U + u] = g[r];
-        ckin = g[23] * g[23] + g[24] * g[24] + g[25] * g[25];
-    } else {
-#pragma unroll
-        for (int r = 0; r < 3; ++r) rows[(long)r * U + u] = pe[0][r] - a.p_ref[r];
-    }
-    cost[u] = a.w_box * ckin + a.w_qd * cqd + a.w_F * cF;
+    if constexpr (MP::kStatic) return MP::MAXN / MP::kChain;
+    else return a.narm;
 }
-
-// d (kinematic rows) / d (q, F): one dual-number seed per blockIdx.y (d < n: q_d, else F_{d - n}); out[row][n + 3 NARM][U].
-// The relative-position row's dependence on the PREVIOUS node's q is the negative of the same block evaluated there.
-template <int L, int NARM>
-__global__ void __launch_bounds__(kThreads) k_rows_kin_jac(const __grid_constant__ StaticParams<L> P0, const __grid_constant__ StaticParams<L> P1,
-                                                          RowsArgs a, const double *q, const double *F, double *out)
-{
-    const long U = a.B * a.N;
-    const long u = (long)blockIdx.x * blockDim.x + threadIdx.x;
-    if (u >= U) return;
-    constexpr int n = NARM * L, ND = n + 3 * NARM;
-    constexpr int KIN = NARM == 2 ? 26 : 3;
-    const int d = blockIdx.y;
-    Dual Fv[3 * NARM], pe[NARM][3], Re[NARM][9];
-#pragma unroll
-    for (int i = 0; i < 3 * NARM; ++i) Fv[i] = Dual(F[(long)i * U + u], d == n + i ? 1.0 : 0.0);
-#pragma unroll
-    for (int c = 0; c < NARM; ++c) {
-        const StaticParams<L> &P = c == 0 ? P0 : P1;
-        Dual qa[L];
-#pragma unroll
-        for (int i = 0; i < L; ++i) qa[i] = Dual(q[(long)(c * L + i) * U + u], d == c * L + i ? 1.0 : 0.0);
-        ArmFk<Dual, L> K;
-        K.run(P, qa, a.ee_joint[c], a.ee_p[c], a.ee_R[c]);
-#pragma unroll
-        for (int r = 0; r < 3; ++r) pe[c][r] = K.pos[r];
-#pragma unroll
-        for (int r = 0; r < 9; ++r) Re[c][r] = K.rot[r];
-    }
-    Dual g[KIN];
-    if (NARM == 2) {
-        const Dual relprev[3] = {Dual(0.0), Dual(0.0), Dual(0.0)};
-        const double ori0[3] = {0.0, 0.0, 0.0};
-        box_kin_rows<Dual>(a, pe[0], Re[0], pe[NARM - 1], Re[NARM - 1], Fv, Fv + 3 * (NARM - 1), relprev, ori0, g);
-    } else {
-#pragma unroll
-        for (int r = 0; r < 3; ++r) g[r] = pe[0][r];
-    }
-#pragma unroll
-    for (int r = 0; r < KIN; ++r) out[((long)r * ND + d) * U + u] = g[r].d;
-}
-
-// ---- run-time trees (header comment).  Arm c's frame: a.ee_joint[c] (global joint, -1 = world-fixed), a.ee_p / a.ee_R[c].
 
 // rows, cost and (optional) d T+ / d tau: one RNEA sweep with the forces as external link forces
-struct RowsTreeBody {
+struct RowsBody {
     template <class MP>
     static MPCF_DI void run(const MP &m, long u, long U, RowsArgs a, const double *q, const double *qd, const double *F, const double *T,
                             const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
                             double *cost, double *dT_dtau)
     {
-        const int n = m.n(), narm = a.narm, KIN = narm == 2 ? 26 : 3;
+        constexpr int UNR = MP::kStatic ? MP::MAXN : 1;
+        const int n = m.n(), narm = arms<MP>(a), KIN = narm == 2 ? 26 : 3;
         const long b = u % a.B;
         const int k = (int)(u / a.B);
         double qa[MP::MAXN], qda[MP::MAXN], zero[MP::MAXN], tau[MP::MAXN];
         double cqd = 0.0, cF = 0.0, ckin = 0.0;
-#pragma unroll 1
+#pragma unroll UNR
         for (int i = 0; i < n; ++i) {
             qa[i] = q[(long)i * U + u];
             qda[i] = qd[(long)i * U + u];
@@ -337,18 +139,20 @@ struct RowsTreeBody {
         }
         JointVar<double> jv[MP::MAXN];
         Dyn<double, MP>::template rnea_impl<false>(m, qa, jv, qda, zero, tau, ext);
-#pragma unroll 1
+#pragma unroll UNR
         for (int i = 0; i < n; ++i) {
             const double t = tau[i];
+            // static models re-read q, qd rather than hold every joint's in registers across the sweep (forests spill less)
+            const double qi = MP::kStatic ? q[(long)i * U + u] : qa[i], qdi = MP::kStatic ? qd[(long)i * U + u] : qda[i];
             rows[(long)(KIN + i) * U + u] = t;
             // Euler defect against the next node's q (last node: the trailing q_N)
-            const double qn = qa[i] + a.h * qda[i];
+            const double qn = qi + a.h * qdi;
             const double qnext = k + 1 < a.N ? q[(long)i * U + u + a.B] : (q_last ? q_last[(long)i * a.B + b] : qn);
             rows[(long)(KIN + n + i) * U + u] = qn - qnext;
             double Tdef = 0.0, dTdt = 0.0;
             if (T) {
                 const double lam = m.fat(i, 0), kap = m.fat(i, 1);
-                const double Pl = m.fat(i, 2) * t * t + m.fat(i, 3) * qda[i] * qda[i];
+                const double Pl = m.fat(i, 2) * t * t + m.fat(i, 3) * qdi * qdi;
                 const double Ti = T[(long)i * U + u];
                 const double za = exp(-lam * a.h);
                 const double gain = lam == 0.0 ? a.h * kap : (1.0 - za) * (kap / lam);
@@ -388,11 +192,12 @@ struct RowsTreeBody {
 
 // dtau_dF [n][3 narm][U] and kin_jac [KIN][n + 3 narm][U] (either may be NULL): frame kinematics of the two frames' ancestors
 // once, then one box_kin_rows<Dual> per direction seeded with the pose tangent
-struct RowsTreeJacBody {
+struct RowsJacBody {
     template <class MP>
     static MPCF_DI void run(const MP &m, long u, long U, RowsArgs a, const double *q, const double *F, double *dtau_dF, double *kin_jac)
     {
-        const int n = m.n(), narm = a.narm, KIN = narm == 2 ? 26 : 3, ND = n + 3 * narm;
+        constexpr int UNR = MP::kStatic ? MP::MAXN : 1;
+        const int n = m.n(), narm = arms<MP>(a), KIN = narm == 2 ? 26 : 3, ND = n + 3 * narm;
         unsigned long long anc[2] = {0ull, 0ull};  // ancestor sets of the frames (bit j: joint j moves frame c)
 #pragma unroll
         for (int c = 0; c < 2; ++c) {
@@ -411,7 +216,7 @@ struct RowsTreeJacBody {
 #pragma unroll
         for (int i = 0; i < 6; ++i) Fv[i] = i < 3 * narm ? F[(long)i * U + u] : 0.0;
         if (dtau_dF) {
-#pragma unroll 1
+#pragma unroll UNR
             for (int j = 0; j < n; ++j) {
 #pragma unroll
                 for (int c = 0; c < 2; ++c) {
@@ -466,33 +271,6 @@ struct RowsTreeJacBody {
     }
 };
 
-static cudaError_t rows_tree_launch(const LaunchModel &m, const RowsArgs &a, const double *q, const double *qd, const double *F, const double *T,
-                                    const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
-                                    double *cost, double *dtau_dF, double *dT_dtau, double *kin_jac, cudaStream_t s)
-{
-    const long U = a.B * a.N;
-    cudaError_t e = dispatch_generic<RowsTreeBody>(m, U, 1, s, a, q, qd, F, T, q_last, T_last, rel_pos0, rel_ori0, rows, cost, dT_dtau);
-    if (e != cudaSuccess || !(dtau_dF || kin_jac)) return e;
-    return dispatch_generic<RowsTreeJacBody>(m, U, 1, s, a, q, F, dtau_dF, kin_jac);
-}
-
-template <int L, int NARM>
-static cudaError_t rows_launch(const StaticParams<L> *cp, const RowsArgs &a, const double *q, const double *qd, const double *F, const double *T,
-                               const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
-                               double *cost, double *dtau_dF, double *dT_dtau, double *kin_jac, cudaStream_t s)
-{
-    const long U = a.B * a.N;
-    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
-    const StaticParams<L> &P1 = cp[NARM - 1];
-    k_ocp_rows<L, NARM><<<gb, kThreads, 0, s>>>(cp[0], P1, a, q, qd, F, T, q_last, T_last, rel_pos0, rel_ori0, rows, cost, dtau_dF, dT_dtau);
-    g_launches.fetch_add(1);
-    if (kin_jac) {
-        k_rows_kin_jac<L, NARM><<<dim3(gb, NARM * L + 3 * NARM), kThreads, 0, s>>>(cp[0], P1, a, q, F, kin_jac);
-        g_launches.fetch_add(1);
-    }
-    return cudaGetLastError();
-}
-
 cudaError_t launch_ocp_rows(const LaunchModel &m, const RowsHost &h, const double *q, const double *qd, const double *F, const double *T,
                             const double *q_last, const double *T_last, const double *rel_pos0, const double *rel_ori0, double *rows,
                             double *cost, double *dtau_dF, double *dT_dtau, double *kin_jac, cudaStream_t s)
@@ -507,18 +285,10 @@ cudaError_t launch_ocp_rows(const LaunchModel &m, const RowsHost &h, const doubl
     }
     a.wsign = h.wsign; a.dist2_ref = h.dist2_ref; a.mu = h.mu; a.w_box = h.w_box; a.w_qd = h.w_qd; a.w_F = h.w_F; a.h = h.h;
     for (int k = 0; k < 3; ++k) { a.fdes[k] = h.fdes[k]; a.p_ref[k] = h.p_ref[k]; }
-#define ROWS_ARGS a, q, qd, F, T, q_last, T_last, rel_pos0, rel_ori0, rows, cost, dtau_dF, dT_dtau, kin_jac, s
-    switch (m.fam) {
-    case FAM_CHAIN3: return rows_launch<3, 1>(static_cast<const StaticParams<3> *>(m.static_params), ROWS_ARGS);
-    case FAM_CHAIN6: return rows_launch<6, 1>(static_cast<const StaticParams<6> *>(m.static_params), ROWS_ARGS);
-    case FAM_CHAIN7: return rows_launch<7, 1>(static_cast<const StaticParams<7> *>(m.static_params), ROWS_ARGS);
-    case FAM_FOREST12x6: return rows_launch<6, 2>(static_cast<const StaticParams<6> *>(m.chain_params), ROWS_ARGS);
-    case FAM_FOREST14x7: return rows_launch<7, 2>(static_cast<const StaticParams<7> *>(m.chain_params), ROWS_ARGS);
-    case FAM_GENERIC16:
-    case FAM_GENERIC64: return rows_tree_launch(m, ROWS_ARGS);
-    default: return cudaErrorInvalidValue;
-    }
-#undef ROWS_ARGS
+    const long U = a.B * a.N;
+    cudaError_t e = dispatch<RowsBody>(m, U, 1, s, a, q, qd, F, T, q_last, T_last, rel_pos0, rel_ori0, rows, cost, dT_dtau);
+    if (e != cudaSuccess || !(dtau_dF || kin_jac)) return e;
+    return dispatch<RowsJacBody>(m, U, 1, s, a, q, F, dtau_dF, kin_jac);
 }
 
 }  // namespace mpcf

@@ -114,8 +114,8 @@ class PilzForceOCP:
     decision variables per node: q_k(6), qd_k(6), Fx_k(1); trailing q_N(6)
     g per node: tau_k(6) in +-b_k ; ee_pos_xy - ref (2) = 0 ; Euler defect (6) = 0 ; cost -= Fx^2
 
-    The fused row kernel takes any model: a bare revolute chain runs the compile-time kernels, any other URDF (prismatic or
-    continuous joints, a branched tree with the frame anywhere in it) the run-time-tree kernels; n is then the model's DOF.
+    The fused row kernel takes any model, one kernel for every family: a bare revolute chain, or any other URDF (prismatic or
+    continuous joints, a branched tree with the frame anywhere in it); n is then the model's DOF.
     """
 
     def __init__(self, urdf: str, frame: str = "prbt_link_5", N: int = 60, T: float = 2.0, tau0: float = 50.0, alpha: float = 2.0,
@@ -272,9 +272,9 @@ class FusedBoxOCP:
     force / moment equilibrium, end-effector distance, relative pose, friction cones, torque rows, Euler and thermal defects
     and the running cost — ONE launch for all B scenarios x N nodes, plus the derivative blocks on request.
 
-    Any model with the two end-effector frames works: the two-arm forests (forest12x6 / forest14x7) run the compile-time
-    kernels, every other tree the run-time-tree kernels — two arms on a torso joint (the Centauro upper body), a humanoid
-    holding the box with both hands, arms with prismatic joints.  On shared ancestors the torque rows carry both forces and
+    Any model with the two end-effector frames works, through the same kernel: the two-arm forests (forest12x6 / forest14x7),
+    where each frame must sit on its own arm, and every other tree — two arms on a torso joint (the Centauro upper body), a
+    humanoid holding the box with both hands, arms with prismatic joints.  On shared ancestors the torque rows carry both forces and
     dtau_dF has both arm blocks."""
 
     ROWS = {"force_eq": (0, 3), "moment_eq": (3, 6), "dist2": (6, 7), "rel_pos": (7, 10), "rel_ori": (10, 13), "friction": (13, 23),

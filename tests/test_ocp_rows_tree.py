@@ -1,10 +1,11 @@
 """Fused reference-mode OCP node rows on run-time-topology models (include/mpcf.h: mpcf_ocp_rows_batch / mpcf_ocp_rows_count_arms,
-csrc/kernels_rows.cu: RowsTreeBody / RowsTreeJacBody; oracle/core.inc.h: ocp_rows): branched trees with a torso joint shared by
+csrc/kernels_rows.cu: RowsBody / RowsJacBody; oracle/core.inc.h: ocp_rows): branched trees with a torso joint shared by
 both arms, a humanoid holding a box with both hands, prismatic and continuous joints, a world-fixed second frame.
 
 CPU: the row counts of every family.  GPU: rows, cost and every derivative output against the oracle on ragged sizes; optional
-inputs absent; the tree kernels against the compile-time kernels on the same two Pilz arms (torso held at zero); FusedBoxOCP
-against the per-function composition; canary gaps around every output; argument rejection."""
+inputs absent; the run-time-tree and compile-time instantiations on the same two Pilz arms (torso held at zero); FusedBoxOCP
+against the per-function composition; canary gaps around every output, compile-time families included; argument rejection,
+and the frame checks of the compile-time families."""
 import ctypes as C
 import os
 
@@ -33,8 +34,10 @@ def _model(name):
         return Model.synthetic("dual_arm", 10, seed=3, armature=1e-2)
     if name == "humanoid37":
         return Model.synthetic("humanoid", 37, seed=7, armature=1e-2)
-    if name == "pilz6x2":
-        return Model.from_urdf(data_urdf("pilz6x2"), armature=1e-2)
+    if name in ("pilz6", "pilz6x2"):
+        return Model.from_urdf(data_urdf(name), armature=1e-2)
+    if name == "dual_arm14":
+        return Model.synthetic("dual_arm", 14, seed=3, armature=1e-2)
     raise KeyError(name)
 
 
@@ -178,12 +181,13 @@ def test_gpu_tree_ocp_rows_optional_inputs_absent(case, name, frames):
 
 @pytest.mark.gpu
 def test_gpu_tree_kernels_agree_with_the_compile_time_kernels():
-    """pilz6x2_torso (run-time tree, torso angle / velocity / temperature held at 0) against pilz6x2 (forest12x6, the static row
-    kernels) on the same arm inputs.  At zero angle the torso rotation is exactly the identity: only the order of summation
-    differs, so every compared plane agrees to 1e-11 of its own scale (rel_err_rows).  Planes whose exact value is zero (joint 6
-    of each arm: the end-effector frame lies on its axis and the flange carries no mass, so its torque and Jacobian column
-    vanish) hold only rounding noise — about 1e-15 from the static kernels' explicit cross products, which the 1e-6 floor of
-    rel_err_rows would count as 3e-11 — and must be zero to 1e-12 of their block's scale in both paths."""
+    """pilz6x2_torso (run-time tree: the GenericModel instantiation of the row bodies, torso angle / velocity / temperature held
+    at 0) against pilz6x2 (forest12x6: their StaticModel instantiation) on the same arm inputs.  At zero angle the torso rotation
+    is exactly the identity: only the order of summation differs, so every compared plane agrees to 1e-11 of its own scale
+    (rel_err_rows).  Planes whose exact value is zero (joint 6 of each arm: the end-effector frame lies on its axis and the
+    flange carries no mass, so its torque and Jacobian column vanish) hold only rounding noise — about 1e-15, from the forces'
+    moments about joint origins a flange length apart and the Jacobian columns' cross products, which the 1e-6 floor of
+    rel_err_rows would count as 3e-11 — and must be zero to 1e-12 of their block's scale in both instantiations."""
     import torch
     from mpc_fatigue_b200.evaluator import BatchEvaluator
     mt, ms = _model("pilz6x2_torso"), _model("pilz6x2")
@@ -274,19 +278,22 @@ def _carve(pool, sizes):
 
 @pytest.mark.gpu
 @pytest.mark.parametrize("U", [1, 33, 131])
-@pytest.mark.parametrize("name,frames", [("humanoid37", ["larm_ee", "rarm_ee"]), ("pilz6x2_torso", ["end_effector", "sec_end_effector"])])
+@pytest.mark.parametrize("name,frames", [("humanoid37", ["larm_ee", "rarm_ee"]), ("pilz6x2_torso", ["end_effector", "sec_end_effector"]),
+                                         ("pilz6x2", ["end_effector", "sec_end_effector"]), ("dual_arm14", ["left_ee", "right_ee"]),
+                                         ("pilz6", ["prbt_flange"])])
 def test_gpu_tree_ocp_rows_outputs_stay_inside_their_buffers(name, frames, U):
     """rows, cost, dtau_dF, dT_dtau and kin_jac carved out of one allocation with canary gaps: no gap written, no element left
-    unwritten (structural zeros included)."""
+    unwritten (structural zeros included).  Buffer sizes follow the arm count."""
     import torch
     B, N = {1: (1, 1), 33: (11, 3), 131: (131, 1)}[U]
     m = _model(name)
-    n = m.n
-    q, qd, F, T, q_last, T_last, rp0, ro0 = (torch.from_numpy(a).cuda() for a in _inputs(oracle_model_from_export(m), B, N, 2, seed=90))
-    sizes = [(26 + 3 * n) * U, U, n * 6 * U, n * U, 26 * (n + 6) * U]
+    n, narm = m.n, len(frames)
+    kin = 26 if narm == 2 else 3
+    q, qd, F, T, q_last, T_last, rp0, ro0 = (torch.from_numpy(a).cuda() for a in _inputs(oracle_model_from_export(m), B, N, narm, seed=90))
+    sizes = [(kin + 3 * n) * U, U, n * 3 * narm * U, n * U, kin * (n + 3 * narm) * U]
     pool = torch.full((_carve(np.empty(0), sizes)[2],), CANARY, dtype=torch.float64, device="cuda")
     (rows, cost, dF, dT, kj), gaps, _ = _carve(pool, sizes)
-    o = _capi.RowsOpts((C.c_int * 2)(*[m.frame_id(f) for f in frames]), 1.0, (C.c_double * 3)(0.0, 0.0, 294.3), 0.04, 0.5,
+    o = _capi.RowsOpts((C.c_int * 2)(*([m.frame_id(f) for f in frames] + [-1] * (2 - narm))), 1.0, (C.c_double * 3)(0.0, 0.0, 294.3), 0.04, 0.5,
                        (C.c_double * 3)(0.3, 0.6, 0.4), 1000.0, 100.0, 10.0, 0.5)
     p = lambda t: C.c_void_p(t.data_ptr())
     _capi.check(_capi.lib.mpcf_ocp_rows_batch(m.handle, C.byref(o), B, N, p(q), p(qd), p(F), p(T), p(q_last), p(T_last), p(rp0), p(ro0),
@@ -325,3 +332,32 @@ def test_gpu_tree_ocp_rows_reject_bad_arguments(name, frames):
     p = lambda t: C.c_void_p(t.data_ptr())
     assert _capi.lib.mpcf_ocp_rows_batch(m.handle, C.byref(o), B, N, p(z(n)), p(z(n)), p(z(6)), None, None, None, None, None, p(rows), p(cost),
                                          None, None, None, None) == _capi.EFRAME
+
+
+@pytest.mark.gpu
+def test_gpu_compile_time_families_keep_their_frame_checks():
+    """On a forest ee_frame[c] must be carried by arm c: swapped frames, a frame on the other arm and a world-fixed frame are
+    MPCF_EFRAME.  On a one-arm chain ee_frame[1] is ignored, whatever it holds."""
+    import torch
+    m = _model("pilz6x2")
+    B, N, n = 4, 2, m.n
+    z = lambda r: torch.zeros((r, B * N), dtype=torch.float64, device="cuda")
+    p = lambda t: C.c_void_p(t.data_ptr())
+    L, R = m.frame_id("end_effector"), m.frame_id("sec_end_effector")
+    world = m.export("fparent").tolist().index(-1)
+
+    def call(model, frames, kin, narm):
+        o = _capi.RowsOpts((C.c_int * 2)(*frames), 1.0, (C.c_double * 3)(), 0.0, 0.0, (C.c_double * 3)(), 0.0, 0.0, 0.0, 0.0)
+        rows, cost = z(kin + 3 * model.n), z(1)
+        rc = _capi.lib.mpcf_ocp_rows_batch(model.handle, C.byref(o), B, N, p(z(model.n)), p(z(model.n)), p(z(3 * narm)), None, None,
+                                           None, None, None, p(rows), p(cost), None, None, None, None)
+        torch.cuda.synchronize()
+        return rc
+    assert call(m, (L, R), 26, 2) == _capi.OK
+    for frames in ((R, L), (L, L), (R, R), (world, R), (L, world)):
+        assert call(m, frames, 26, 2) == _capi.EFRAME, frames
+    one = _model("pilz6")
+    tip = one.frame_id("prbt_flange")
+    for second in (-1, tip, one.nframes + 5):
+        assert call(one, (tip, second), 3, 1) == _capi.OK, second
+    assert call(one, (one.export("fparent").tolist().index(-1), -1), 3, 1) == _capi.EFRAME
