@@ -175,6 +175,27 @@ int mpcf_step_rk4_jvp_strided_batch(const mpcf_model *model, long cnt, long ld, 
 int mpcf_step_rk4_jvp_dual_batch(const mpcf_model *model, long U, const double *q, const double *qd,
                                  const double *tau, const double *f, double dt, const double *dt_u, double *qn,
                                  double *qdn, double *fn, double *jac, void *stream);
+/* Reverse mode.  Vector-Jacobian product of one RK4 step (the step and families of mpcf_step_rk4_jvp_batch): with
+   J = d(q+, qd+, f+)/d(q, qd, tau, f, h) and the adjoint lambda = (lq, lqd, lf), [n][U] each (any may be NULL = 0):
+     gq, gqd, gtau, gf [n][U] = lambda^T J (blocks q, qd, tau, f);  gdt [U] = lambda^T dx+/dh (optional, NULL to skip).
+   qn/qdn/fn: the step itself, all or none.  workspace: as for mpcf_step_rk4_jvp_ws_batch (size from
+   mpcf_step_rk4_jvp_workspace_bytes, 128-byte aligned; NULL = stream-ordered pool).  Coupled models: MPCF_EINVAL.
+   Compile-time families run the Jacobian pipeline's stage and derivative kernels and then one reverse sweep per unit that
+   contracts the stored stage matrices with one vector (no dense Jacobian); run-time trees with n <= 40 the same with the tree
+   kernels; larger run-time models 3n + 1 dual-number sweeps contracted with lambda.  dt = 0 is allowed (nothing divides by h). */
+int mpcf_step_rk4_vjp_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,
+                            const double *f, double dt, const double *dt_u, const double *lq, const double *lqd,
+                            const double *lf, double *gq, double *gqd, double *gtau, double *gf, double *gdt,
+                            double *qn, double *qdn, double *fn, void *workspace, size_t workspace_bytes, void *stream);
+/* Adjoint of mpcf_rollout_rk4_batch.  Loss L(x_1..x_N); gqt/gqdt/gft [n][N*B] = dL/d(trajectory entry k) in the rollout's
+   node-major layout (entry k = x_{k+1}; any may be NULL = 0); qt/qdt/ft = the trajectory that mpcf_rollout_rk4_batch
+   returned for (q0, qd0, f0, tau, dt).  Outputs: gtau [n][N*B] = dL/dtau, gq0/gqd0/gf0 [n][B] = dL/dx_0.
+   Workspace: mpcf_step_rk4_jvp_workspace_bytes(model, B) or NULL.  Coupled models: MPCF_EINVAL.  One step VJP per node,
+   k = N-1 .. 0, in stream order; besides the workspace it takes 4 n B doubles of stream-ordered scratch (nothing of size N B). */
+int mpcf_rollout_rk4_vjp_batch(const mpcf_model *model, long B, int N, const double *q0, const double *qd0,
+                               const double *f0, const double *tau, double dt, const double *qt, const double *qdt,
+                               const double *ft, const double *gqt, const double *gqdt, const double *gft, double *gtau,
+                               double *gq0, double *gqd0, double *gf0, void *workspace, size_t workspace_bytes, void *stream);
 /* Forward-dynamics derivatives at (q, qd, tau): A = d qdd/d q, B = d qdd/d qd, C = M^-1 = d qdd/d tau,
    each [n*n][U] with plane index row*n + col. */
 int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,

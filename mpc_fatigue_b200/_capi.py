@@ -72,6 +72,10 @@ _sig = {
     "mpcf_step_rk4_jvp_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_long]),
     "mpcf_step_rk4_jvp_ws_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, C.c_double, _dp, _dp, _dp, _dp, _dp,
                                              C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpcf_step_rk4_vjp_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, C.c_double, _dp] + [_dp] * 11
+                                + [C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpcf_rollout_rk4_vjp_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int, _dp, _dp, _dp, _dp, C.c_double] + [_dp] * 10
+                                   + [C.c_void_p, C.c_size_t, C.c_void_p]),
     "mpcf_fd_derivs_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, _dp, _dp, C.c_void_p]),
     "mpcf_rnea_derivs_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, _dp, _dp, C.c_void_p]),
     "mpcf_cost_residual_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 7 + [C.c_double] * 7 + [_dp, C.c_void_p]),

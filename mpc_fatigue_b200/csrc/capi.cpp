@@ -622,6 +622,123 @@ extern "C" int mpcf_step_rk4_jvp_batch(const mpcf_model *model, long U, const do
     return mpcf_step_rk4_jvp_ws_batch(model, U, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, nullptr, 0, stream);
 }
 
+// ---- reverse mode ----
+// step VJP on `cnt` units whose state / torque planes have stride `ld` (the adjoint, addend and output strides travel in `a`)
+static cudaError_t run_vjp(const mpcf_model *model, const LaunchModel &lm, long cnt, long ld, const double *q, const double *qd, const double *tau,
+                           const double *f, double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, double *ws,
+                           size_t ws_bytes, cudaStream_t st)
+{
+    if (tree_jvp_supported(lm)) return launch_step_vjp_tree(lm, model->npat, ld, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, ws_bytes, st);
+    if (jvp2_supported(lm)) return launch_step_vjp_ws(lm, ld, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, ws_bytes, st);
+    return launch_step_vjp_dual(lm, ld, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, st);
+}
+
+// the reverse entries' workspace: the caller's (checked as for mpcf_step_rk4_jvp_ws_batch) or one from the stream-ordered pool
+// (*owned set: the caller frees it with cudaFreeAsync); models without a workspace path need none
+static int vjp_workspace(const mpcf_model *model, const LaunchModel &lm, long U, void *workspace, size_t workspace_bytes, cudaStream_t st,
+                         double **ws, size_t *bytes, bool *owned)
+{
+    *ws = nullptr; *bytes = 0; *owned = false;
+    const bool tree = tree_jvp_supported(lm);
+    if (!tree && !jvp2_supported(lm)) return MPCF_OK;
+    if (workspace) {
+        const size_t min_ws = tree ? tree_jvp_workspace_bytes(model->h.n, model->npat, 32)
+                                   : (size_t)32 * jvp_ws_doubles_per_unit(family_chain_len(model->fam)) * sizeof(double);
+        if (reinterpret_cast<uintptr_t>(workspace) % 128) return fail(MPCF_EINVAL, "workspace must be 128-byte aligned");
+        if (workspace_bytes < min_ws) return fail(MPCF_EINVAL, "workspace too small: see mpcf_step_rk4_jvp_workspace_bytes");
+        *ws = static_cast<double *>(workspace);
+        *bytes = workspace_bytes;
+        return MPCF_OK;
+    }
+    *bytes = mpcf_step_rk4_jvp_workspace_bytes(model, U);
+    const cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(ws), *bytes, st);
+    if (e != cudaSuccess) return cuda_fail(e, "cudaMallocAsync(vjp workspace)");
+    *owned = true;
+    return MPCF_OK;
+}
+
+extern "C" int mpcf_step_rk4_vjp_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau, const double *f,
+                                       double dt, const double *dt_u, const double *lq, const double *lqd, const double *lf, double *gq,
+                                       double *gqd, double *gtau, double *gf, double *gdt, double *qn, double *qdn, double *fn, void *workspace,
+                                       size_t workspace_bytes, void *stream)
+{
+    PROLOGUE(q && qd && tau && f && gq && gqd && gtau && gf)
+    if ((qn || qdn || fn) && !(qn && qdn && fn)) return fail(MPCF_EINVAL, "qn/qdn/fn must be all set or all NULL");
+    if (model->couple.on) return fail(MPCF_EINVAL, "the reverse-mode entries do not support coupled fatigue");
+    if (int rc = check_forward_dynamics(model)) return rc;
+    if (U == 0) return MPCF_OK;
+    VjpArgs a;
+    a.lq = lq; a.lqd = lqd; a.lf = lf; a.ldl = U;
+    a.lda = U;
+    a.gq = gq; a.gqd = gqd; a.gf = gf; a.ldg = U;
+    a.gtau = gtau; a.ldgt = U;
+    a.gdt = gdt;
+    double *ws;
+    size_t bytes;
+    bool owned;
+    if (int rc = vjp_workspace(model, lm, U, workspace, workspace_bytes, st, &ws, &bytes, &owned)) return rc;
+    const cudaError_t e = run_vjp(model, lm, U, U, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, bytes, st);
+    const cudaError_t e2 = owned ? cudaFreeAsync(ws, st) : cudaSuccess;
+    return done(e != cudaSuccess ? e : e2, "step_rk4_vjp_batch");
+}
+
+// Adjoint of the rollout: one step VJP per node, k = N-1 .. 0, on the node's B contiguous units (plane stride N B).  lambda_k =
+// g_x(lambda_{k+1}) + dL/dx_k alternates between the g*0 outputs and an O(B) scratch buffer, so that node 0 writes dL/dx_0 into
+// the outputs; the step at node 0 reads x_0 (stride B) and a stride-B copy of tau's node-0 columns.
+extern "C" int mpcf_rollout_rk4_vjp_batch(const mpcf_model *model, long B, int N, const double *q0, const double *qd0, const double *f0,
+                                          const double *tau, double dt, const double *qt, const double *qdt, const double *ft, const double *gqt,
+                                          const double *gqdt, const double *gft, double *gtau, double *gq0, double *gqd0, double *gf0,
+                                          void *workspace, size_t workspace_bytes, void *stream)
+{
+    const long U = B;
+    PROLOGUE(q0 && qd0 && f0 && tau && qt && qdt && ft && gtau && gq0 && gqd0 && gf0)
+    if (N <= 0) return fail(MPCF_EINVAL, "N must be positive");
+    if (model->couple.on) return fail(MPCF_EINVAL, "the reverse-mode entries do not support coupled fatigue");
+    if (int rc = check_forward_dynamics(model)) return rc;
+    if (B == 0) return MPCF_OK;
+    const int n = model->h.n;
+    const long NB = (long)N * B;
+    double *ws;
+    size_t bytes;
+    bool owned;
+    if (int rc = vjp_workspace(model, lm, B, workspace, workspace_bytes, st, &ws, &bytes, &owned)) return rc;
+    double *scr = nullptr;  // [3n][B] adjoint of the odd nodes | [n][B] tau of node 0
+    cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&scr), (size_t)4 * n * B * sizeof(double), st);
+    if (e != cudaSuccess) {
+        if (owned) cudaFreeAsync(ws, st);
+        return cuda_fail(e, "cudaMallocAsync(rollout adjoint scratch)");
+    }
+    double *tau0 = scr + (size_t)3 * n * B;
+    if (N > 1) e = cudaMemcpy2DAsync(tau0, B * sizeof(double), tau, NB * sizeof(double), B * sizeof(double), n, cudaMemcpyDeviceToDevice, st);
+    auto sh = [](const double *p, long off) { return p ? p + off : p; };
+    for (int k = N - 1; k >= 0 && e == cudaSuccess; --k) {
+        VjpArgs a;
+        if (k == N - 1) {  // lambda_N = dL/dx_N = trajectory entry N - 1
+            a.lq = sh(gqt, (long)k * B); a.lqd = sh(gqdt, (long)k * B); a.lf = sh(gft, (long)k * B); a.ldl = NB;
+        } else {
+            const bool even = (k + 1) % 2 == 0;
+            a.lq = even ? gq0 : scr; a.lqd = even ? gqd0 : scr + (size_t)n * B; a.lf = even ? gf0 : scr + (size_t)2 * n * B; a.ldl = B;
+        }
+        if (k > 0) { a.aq = sh(gqt, (long)(k - 1) * B); a.aqd = sh(gqdt, (long)(k - 1) * B); a.af = sh(gft, (long)(k - 1) * B); }
+        a.lda = NB;
+        const bool even = k % 2 == 0;
+        a.gq = even ? gq0 : scr; a.gqd = even ? gqd0 : scr + (size_t)n * B; a.gf = even ? gf0 : scr + (size_t)2 * n * B; a.ldg = B;
+        a.gtau = gtau + (long)k * B; a.ldgt = NB;
+        if (k == 0)
+            e = run_vjp(model, lm, B, B, q0, qd0, N > 1 ? tau0 : tau, f0, dt, nullptr, a, nullptr, nullptr, nullptr, ws, bytes, st);
+        else {
+            const long off = (long)(k - 1) * B;
+            e = run_vjp(model, lm, B, NB, qt + off, qdt + off, tau + (long)k * B, ft + off, dt, nullptr, a, nullptr, nullptr, nullptr, ws, bytes, st);
+        }
+    }
+    cudaError_t e2 = cudaFreeAsync(scr, st);
+    if (owned) {
+        const cudaError_t e3 = cudaFreeAsync(ws, st);
+        if (e2 == cudaSuccess) e2 = e3;
+    }
+    return done(e != cudaSuccess ? e : e2, "rollout_rk4_vjp_batch");
+}
+
 extern "C" int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau, double *A,
                                     double *B, double *C, void *stream)
 {

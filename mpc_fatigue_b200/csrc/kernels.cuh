@@ -122,6 +122,42 @@ size_t tree_jvp_workspace_bytes(int n, int npat, long U);
 cudaError_t launch_step_jvp_tree(const LaunchModel &m, int npat, long U, long cnt, const double *q, const double *qd, const double *tau,
                                  const double *f, double dt, const double *dt_u, double *qn, double *qdn, double *fn, double *jac, long UJ,
                                  double *ws, size_t ws_bytes, cudaStream_t s);
+// Vector-Jacobian product of the RK4 step (reverse mode): the adjoint lambda = (lq, lqd, lf) and the addend (aq, aqd, af) of g_x
+// (both NULL = 0) come in, g_x = lambda^T d x+/d x + addend, g_tau and g_dt go out.  Every plane group has its own stride, so the
+// rollout adjoint can read a trajectory slice (stride N B) and write an O(B) buffer in one call.
+struct VjpArgs {
+    const double *lq = nullptr, *lqd = nullptr, *lf = nullptr;
+    long ldl = 0;
+    const double *aq = nullptr, *aqd = nullptr, *af = nullptr;
+    long lda = 0;
+    double *gq = nullptr, *gqd = nullptr, *gf = nullptr;
+    long ldg = 0;
+    double *gtau = nullptr;
+    long ldgt = 0;
+    double *gdt = nullptr;  // [units] or NULL
+    // the same planes from joint j0 on (forests: one chain per launch)
+    __host__ VjpArgs rows(int j0) const
+    {
+        auto sh = [](auto *p, long ld, int j) { return p ? p + (size_t)j * ld : p; };
+        VjpArgs r = *this;
+        r.lq = sh(lq, ldl, j0); r.lqd = sh(lqd, ldl, j0); r.lf = sh(lf, ldl, j0);
+        r.aq = sh(aq, lda, j0); r.aqd = sh(aqd, lda, j0); r.af = sh(af, lda, j0);
+        r.gq = sh(gq, ldg, j0); r.gqd = sh(gqd, ldg, j0); r.gf = sh(gf, ldg, j0);
+        r.gtau = sh(gtau, ldgt, j0);
+        return r;
+    }
+};
+// static families (kernels_jvp2.cu): K1 + K2 of the Jacobian pipeline, then the reverse sweep; caller workspace as for the JVP
+cudaError_t launch_step_vjp_ws(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
+                               double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, double *ws,
+                               size_t ws_bytes, cudaStream_t s);
+// run-time trees with n <= 40 (kernels_tree.cu): T1, T2, the factor with L^-1, then the reverse sweep
+cudaError_t launch_step_vjp_tree(const LaunchModel &m, int npat, long U, long cnt, const double *q, const double *qd, const double *tau,
+                                 const double *f, double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn,
+                                 double *ws, size_t ws_bytes, cudaStream_t s);
+// run-time models with n > 40 (kernels_jvp.cu): one dual-number sweep per input direction, contracted with lambda
+cudaError_t launch_step_vjp_dual(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
+                                 double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, cudaStream_t s);
 void jvp_profile_enable(bool on);
 int jvp_profile_read(double *ms3, long *launches);
 cudaError_t launch_fp64_probe(long iters, int blocks, double *out, cudaStream_t s);

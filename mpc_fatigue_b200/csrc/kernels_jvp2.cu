@@ -593,6 +593,94 @@ struct ColumnState {
     }
 };
 
+// ------------------------------------------------------------------------------------------------ reverse sweep
+// Vector-Jacobian product of the step, thread = unit, in place of K3 (DESIGN.md §4d).  Stages walked 4 -> 1 with
+// rho_s = w_s lambda + c_s J_{s+1}^T r_{s+1}, r_s = h rho_s:
+//   J_s^T r = (A_s^T r_v, r_q + B_s^T r_v + 2 kappa cv qd_s r_f, -Lambda r_f),   g_tau += C_s r_v + 2 kappa ctau tau r_f,
+//   g_x = lambda + sum_s J_s^T r_s (+ addend),   g_dt = sum_s rho_s^T k_s.
+// Every workspace load is one coalesced warp access (lane = unit of the 32-unit tile); 3 n^2 FMAs per stage.
+// gdt_add: a forest's second chain adds its share of g_dt to the first chain's (stream order, no atomics).
+template <int N, int L>
+__global__ void __launch_bounds__(kThreads) k_step_vjp(const __grid_constant__ StaticParams<N> P, long U, long u0, long cnt,
+                                                      const double *__restrict__ tau, double dt, const double *__restrict__ dt_u,
+                                                      const VjpArgs a, int gdt_add, const double *__restrict__ ws)
+{
+    static_assert(N == L, "the reverse sweep runs one serial chain at a time (forests: one launch per chain)");
+    using W = WsLayout<N>;
+    const long lu = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (lu >= cnt) return;
+    const long u = u0 + lu;
+    const double h = dt_u ? dt_u[u] : dt;
+    double lam[3 * N], gx[3 * N], ad[3 * N], gt[N], kt[N];
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+        lam[i] = a.lq ? a.lq[i * a.ldl + u] : 0.0;
+        lam[N + i] = a.lqd ? a.lqd[i * a.ldl + u] : 0.0;
+        lam[2 * N + i] = a.lf ? a.lf[i * a.ldl + u] : 0.0;
+        gx[i] = lam[i] + (a.aq ? a.aq[i * a.lda + u] : 0.0);
+        gx[N + i] = lam[N + i] + (a.aqd ? a.aqd[i * a.lda + u] : 0.0);
+        gx[2 * N + i] = lam[2 * N + i] + (a.af ? a.af[i * a.lda + u] : 0.0);
+        kt[i] = 2.0 * P.fat[i][1] * P.fat[i][2] * tau[i * U + u];
+        gt[i] = 0.0;
+    }
+#pragma unroll
+    for (int i = 0; i < 3 * N; ++i) ad[i] = 0.0;
+    double gh = 0.0;
+#pragma unroll 1
+    for (int s = 3; s >= 0; --s) {
+        const double cs = s < 2 ? 0.5 : (s == 2 ? 1.0 : 0.0);  // x_{s+1} = x + c_s h k_s (ad = 0 at the last stage)
+        const double wt = (s == 0 || s == 3) ? 1.0 / 6.0 : 1.0 / 3.0;
+        const double *w = ws + W::chunk(lu / 32, s) + (lu & 31);
+        const double *v = w + W::kPlanes2 * 32;
+        double rq[N], rv[N], rf[N], nq[N], nv[N];
+#pragma unroll
+        for (int i = 0; i < N; ++i) {
+            const double qds = __ldcs(v + (W::kQd + i) * 32);
+            const double pq = fma(wt, lam[i], cs * ad[i]), pv = fma(wt, lam[N + i], cs * ad[N + i]),
+                         pf = fma(wt, lam[2 * N + i], cs * ad[2 * N + i]);
+            gh = fma(pq, qds, gh);
+            gh = fma(pv, __ldcs(v + (W::kQdd + i) * 32), gh);
+            gh = fma(pf, __ldcs(v + (W::kFd + i) * 32), gh);
+            rq[i] = h * pq;
+            rv[i] = h * pv;
+            rf[i] = h * pf;
+            nq[i] = 0.0;
+            nv[i] = fma(2.0 * P.fat[i][1] * P.fat[i][3] * qds, rf[i], rq[i]);
+            gt[i] = fma(kt[i], rf[i], gt[i]);
+        }
+        // one basic block per row (the never-taken fence, cf. StaticModel::skip): ptxas would otherwise hoist all 3 n^2 loads of the
+        // stage and take the whole register file
+#pragma unroll
+        for (int r = 0; r < N; ++r) {
+            if (P.fence0 > r) continue;
+            const double x = rv[r];
+#pragma unroll
+            for (int c = 0; c < N; ++c) {
+                nq[c] = fma(__ldcs(w + (r * N + c) * 32), x, nq[c]);
+                nv[c] = fma(__ldcs(w + (N * N + r * N + c) * 32), x, nv[c]);
+                gt[c] = fma(__ldcs(w + (2 * N * N + r * N + c) * 32), x, gt[c]);
+            }
+        }
+#pragma unroll
+        for (int i = 0; i < N; ++i) {
+            ad[i] = nq[i];
+            ad[N + i] = nv[i];
+            ad[2 * N + i] = -P.fat[i][0] * rf[i];
+            gx[i] += ad[i];
+            gx[N + i] += ad[N + i];
+            gx[2 * N + i] += ad[2 * N + i];
+        }
+    }
+#pragma unroll
+    for (int i = 0; i < N; ++i) {
+        a.gq[i * a.ldg + u] = gx[i];
+        a.gqd[i * a.ldg + u] = gx[N + i];
+        a.gf[i * a.ldg + u] = gx[2 * N + i];
+        a.gtau[i * a.ldgt + u] = gt[i];
+    }
+    if (a.gdt) a.gdt[u] = gdt_add ? a.gdt[u] + gh : gh;
+}
+
 // ---- mbarrier / bulk-copy primitives (PTX ISA 8.0, sm_90+; forms as in <cuda/ptx>) ----
 MPCF_DI unsigned smem_u32(const void *p) { return (unsigned)__cvta_generic_to_shared(p); }
 MPCF_DI void mbar_init(unsigned long long *bar, unsigned count)
@@ -781,6 +869,39 @@ static int sm_count()
     return n[dev];
 }
 
+// K2 launch shape: 2 blocks per SM with the link slab in shared memory
+template <int N, int L>
+struct K2Config {
+    static constexpr int kThreadsK2 = (2 * (18 * (N - 1) + N * (N + 1) / 2) * kThreads * (int)sizeof(double) <= 227 * 1024) ? kThreads : 96;
+    static constexpr int kSlab = (18 * (N - 1) + N * (N + 1) / 2) * kThreadsK2 * (int)sizeof(double);
+    static constexpr bool kSmem = N == L && 2 * kSlab <= 227 * 1024;
+};
+
+// K1 + K2 of one chunk of units [u0, u0 + cnt): what the Jacobian (K3) and the reverse sweep (k_step_vjp) read.  The caller has set
+// K2's shared-memory attribute.
+template <int N, int L>
+static void launch_stages_derivs(const StaticParams<N> &P, long U, long u0, long cnt, const double *q, const double *qd, const double *tau,
+                                 const double *theat, long UT, const double *f, double dt, const double *dt_u, double *qn, double *qdn,
+                                 double *fn, double *ws, cudaStream_t s)
+{
+    using K2 = K2Config<N, L>;
+    const unsigned gb = (unsigned)((cnt + kThreads - 1) / kThreads);
+    cudaEvent_t pe = prof_begin(0, s);
+    k_step_stages<N, L><<<gb, kThreads, 0, s>>>(P, U, u0, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, ws);
+    prof_end(pe, s);
+    pe = prof_begin(1, s);
+    static const int k2smem = getenv("MPCF_K2_SMEM") ? atoi(getenv("MPCF_K2_SMEM")) : 1;
+    bool k2done = false;
+    if constexpr (K2::kSmem) {
+        if (k2smem) {
+            k_stage_derivs<N, L, true><<<dim3((unsigned)((cnt + K2::kThreadsK2 - 1) / K2::kThreadsK2), 4), K2::kThreadsK2, K2::kSlab, s>>>(P, cnt, ws);
+            k2done = true;
+        }
+    }
+    if (!k2done) k_stage_derivs<N, L, false><<<dim3(gb, 4), kThreads, 0, s>>>(P, cnt, ws);
+    prof_end(pe, s);
+}
+
 template <int N, int L>
 static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const double *q, const double *qd, const double *tau, const double *theat,
                             long UT, const double *f,
@@ -796,10 +917,8 @@ static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const d
     constexpr int NBUF = kTma ? (kRingMax > 5 ? 5 : kRingMax) : 0;  // measured on chain6: 5 slots 11.74 ms, 4: 11.89, 6: 12.08, 7: 12.93 (L1 gets what the ring leaves)
     constexpr int kCpwDefault = (3 * N + 1 <= 19) ? 1 : 2;
     constexpr size_t smem = (size_t)NBUF * W::kRingBytes + 2 * NBUF * sizeof(unsigned long long);
-    // derivative kernel: 2 blocks per SM with the link slab in shared memory
-    constexpr int kK2Threads = (2 * (18 * (N - 1) + N * (N + 1) / 2) * kThreads * (int)sizeof(double) <= 227 * 1024) ? kThreads : 96;
-    constexpr int kK2Slab = (18 * (N - 1) + N * (N + 1) / 2) * kK2Threads * (int)sizeof(double);
-    constexpr bool kK2Smem = N == L && 2 * kK2Slab <= 227 * 1024;
+    using K2 = K2Config<N, L>;
+    constexpr bool kK2Smem = K2::kSmem;
     if constexpr (kTma) {
         // function attributes are per device: set them once on each device a process uses (idempotent, so two threads
         // racing through the first call is harmless; the flag is atomic)
@@ -818,7 +937,7 @@ static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const d
             e = cudaFuncSetAttribute(k_chain_rule_tma<N, L, NBUF, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
             if (e != cudaSuccess) return e;
             if constexpr (kK2Smem) {
-                e = cudaFuncSetAttribute(k_stage_derivs<N, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, kK2Slab);
+                e = cudaFuncSetAttribute(k_stage_derivs<N, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2::kSlab);
                 if (e != cudaSuccess) return e;
             }
             attr_set[dev].store(true, std::memory_order_release);
@@ -826,23 +945,9 @@ static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const d
     }
     for (long u0 = 0; u0 < Ucnt; u0 += Uc) {
         const long cnt = (Ucnt - u0) < Uc ? (Ucnt - u0) : Uc;
-        const unsigned gb = (unsigned)((cnt + kThreads - 1) / kThreads);
         const long ntiles = (cnt + 31) / 32;
-        cudaEvent_t pe = prof_begin(0, s);
-        k_step_stages<N, L><<<gb, kThreads, 0, s>>>(P, U, u0, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, ws);
-        prof_end(pe, s);
-        pe = prof_begin(1, s);
-        static const int k2smem = getenv("MPCF_K2_SMEM") ? atoi(getenv("MPCF_K2_SMEM")) : 1;
-        bool k2done = false;
-        if constexpr (kK2Smem) {
-            if (k2smem) {
-                k_stage_derivs<N, L, true><<<dim3((unsigned)((cnt + kK2Threads - 1) / kK2Threads), 4), kK2Threads, kK2Slab, s>>>(P, cnt, ws);
-                k2done = true;
-            }
-        }
-        if (!k2done) k_stage_derivs<N, L, false><<<dim3(gb, 4), kThreads, 0, s>>>(P, cnt, ws);
-        prof_end(pe, s);
-        pe = prof_begin(2, s);
+        launch_stages_derivs<N, L>(P, U, u0, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, ws, s);
+        cudaEvent_t pe = prof_begin(2, s);
         if constexpr (kTma) {
             const unsigned g3 = (unsigned)(ntiles < sm_count() ? ntiles : sm_count());
             static const int cpw_env = getenv("MPCF_K3_CPW") ? atoi(getenv("MPCF_K3_CPW")) : 1;
@@ -935,6 +1040,64 @@ cudaError_t launch_step_jvp_ws(const LaunchModel &m, long U, const double *q, co
         return run_forest<7>(m, U, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, jac, UJ, ws, Uc, s);
     default:
         return cudaErrorInvalidValue;
+    }
+}
+
+// Reverse sweep of one serial chain: K1 and K2 unchanged over the same chunks as run_jvp2, then k_step_vjp in place of K3.
+// gdt_add: this chain's g_dt is added to what an earlier chain's launch wrote.
+template <int N, int L>
+static cudaError_t run_vjp2(const StaticParams<N> &P, long U, long Ucnt, const double *q, const double *qd, const double *tau, const double *f,
+                            double dt, const double *dt_u, const VjpArgs &a, int gdt_add, double *qn, double *qdn, double *fn, double *ws, long Uc,
+                            cudaStream_t s)
+{
+    using K2 = K2Config<N, L>;
+    if constexpr (K2::kSmem) {
+        static std::atomic<bool> attr_set[64];
+        const int dev = current_device();
+        if (!attr_set[dev].load(std::memory_order_acquire)) {
+            const cudaError_t e = cudaFuncSetAttribute(k_stage_derivs<N, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2::kSlab);
+            if (e != cudaSuccess) return e;
+            attr_set[dev].store(true, std::memory_order_release);
+        }
+    }
+    for (long u0 = 0; u0 < Ucnt; u0 += Uc) {
+        const long cnt = (Ucnt - u0) < Uc ? (Ucnt - u0) : Uc;
+        launch_stages_derivs<N, L>(P, U, u0, cnt, q, qd, tau, tau, U, f, dt, dt_u, qn, qdn, fn, ws, s);
+        k_step_vjp<N, L><<<(unsigned)((cnt + kThreads - 1) / kThreads), kThreads, 0, s>>>(P, U, u0, cnt, tau, dt, dt_u, a, gdt_add, ws);
+        g_launches.fetch_add(3);
+    }
+    return cudaGetLastError();
+}
+
+template <int L>
+static cudaError_t vjp_chains(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
+                              double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, double *ws, long Uc,
+                              cudaStream_t s)
+{
+    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params);
+    for (int c = 0; c < m.n / L; ++c) {
+        const size_t off = (size_t)c * L * U;
+        const cudaError_t e = run_vjp2<L, L>(cp[c], U, cnt, q + off, qd + off, tau + off, f + off, dt, dt_u, a.rows(c * L), c > 0,
+                                             qn ? qn + off : nullptr, qdn ? qdn + off : nullptr, fn ? fn + off : nullptr, ws, Uc, s);
+        if (e != cudaSuccess) return e;
+    }
+    return cudaSuccess;
+}
+
+cudaError_t launch_step_vjp_ws(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
+                               double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, double *ws,
+                               size_t ws_bytes, cudaStream_t s)
+{
+    if (cnt <= 0) return cudaSuccess;
+    const size_t per_unit = jvp_ws_doubles_per_unit(family_chain_len(m.fam)) * sizeof(double);
+    long Uc = (long)(ws_bytes / per_unit);
+    Uc -= Uc % 32;  // whole 32-unit tiles
+    if (Uc < 32) return cudaErrorInvalidValue;
+    switch (family_chain_len(m.fam)) {
+    case 3: return vjp_chains<3>(m, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, Uc, s);
+    case 6: return vjp_chains<6>(m, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, Uc, s);
+    case 7: return vjp_chains<7>(m, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, Uc, s);
+    default: return cudaErrorInvalidValue;
     }
 }
 

@@ -270,6 +270,113 @@ __global__ void __launch_bounds__(256) k_tree_factor(GenericBlob blob, TreeWs W,
     }
 }
 
+// ------------------------------------------------------------------------------------------------ reverse sweep
+// Vector-Jacobian product of the step (DESIGN.md §4d), thread = unit, over the unit's contiguous (unit, stage) blocks after T1, T2
+// and k_tree_factor (with L^-1).  Per stage, with r = h rho and r_v its qd part:
+//   mu = M^-1 r_v = L^-1 D^-1 L^-T r_v        two triangular matvecs on the packed ancestor pattern
+//   A^T r_v = -(dID/dq)^T mu,  B^T r_v = -(dID/dqd)^T mu,  C r_v = mu
+// O(npat) work per stage.  The fatigue states of the stages are recomputed from f, tau and the stored qd_s with the same
+// arithmetic as T1 (the rows are per joint and linear in f).
+template <int MAXN>
+__global__ void __launch_bounds__(kThreads) k_tree_vjp(GenericBlob blob, TreeWs W, long U, long u0, long cnt, const double *tau, const double *f,
+                                                       double dt, const double *dt_u, const VjpArgs a, const double *ws)
+{
+    extern __shared__ double smem[];
+    const int n = blob.n;
+    const int nd = 27 * n + 3;
+    int *si = reinterpret_cast<int *>(smem + nd);
+    for (int k = threadIdx.x; k < nd; k += blockDim.x) smem[k] = blob.dbl[k];
+    for (int k = threadIdx.x; k < blob_ints(n); k += blockDim.x) si[k] = blob.ints[k];
+    __syncthreads();
+    const GenericModel<MAXN> m{n, smem, si};
+    using D = Dyn<double, GenericModel<MAXN>>;
+    const long lu = (long)blockIdx.x * blockDim.x + threadIdx.x;
+    if (lu >= cnt) return;
+    const long u = u0 + lu;
+    const double h = dt_u ? dt_u[u] : dt;
+    double lam[3 * MAXN], gx[3 * MAXN], ad[3 * MAXN], gt[MAXN], y[MAXN], fd[4 * MAXN];
+    for (int i = 0; i < n; ++i) {
+        lam[i] = a.lq ? a.lq[i * a.ldl + u] : 0.0;
+        lam[n + i] = a.lqd ? a.lqd[i * a.ldl + u] : 0.0;
+        lam[2 * n + i] = a.lf ? a.lf[i * a.ldl + u] : 0.0;
+        gx[i] = lam[i] + (a.aq ? a.aq[i * a.lda + u] : 0.0);
+        gx[n + i] = lam[n + i] + (a.aqd ? a.aqd[i * a.lda + u] : 0.0);
+        gx[2 * n + i] = lam[2 * n + i] + (a.af ? a.af[i * a.lda + u] : 0.0);
+        ad[i] = 0.0; ad[n + i] = 0.0; ad[2 * n + i] = 0.0;
+        gt[i] = 0.0;
+        // stage fatigue derivatives fdot_s, as T1 forms them: f_1 = f, f_{s+1} = f + (c_s h) fdot_s
+        const double ti = tau[i * U + u], fi = f[i * U + u];
+        double fs = fi;
+        for (int s = 0; s < 4; ++s) {
+            const double cs = s < 2 ? 0.5 : (s == 2 ? 1.0 : 0.0);
+            const double k = D::fatigue_rhs(m, i, fs, ti, ws[W.at(lu, s) + (size_t)W.vec(0, i)]);
+            fd[s * n + i] = k;
+            fs = fi + (h * cs) * k;
+        }
+    }
+    double gh = 0.0;
+#pragma unroll 1
+    for (int s = 3; s >= 0; --s) {
+        const double cs = s < 2 ? 0.5 : (s == 2 ? 1.0 : 0.0);
+        const double wt = (s == 0 || s == 3) ? 1.0 / 6.0 : 1.0 / 3.0;
+        const double *o = ws + W.at(lu, s);  // the workspace is chunk-local
+        // rho_s and r_s = h rho_s (r overwrites ad), g_dt += rho_s^T k_s
+        for (int i = 0; i < n; ++i) {
+            const double pq = fma(wt, lam[i], cs * ad[i]), pv = fma(wt, lam[n + i], cs * ad[n + i]), pf = fma(wt, lam[2 * n + i], cs * ad[2 * n + i]);
+            gh = fma(pq, o[W.vec(0, i)], gh);
+            gh = fma(pv, o[W.vec(1, i)], gh);
+            gh = fma(pf, fd[s * n + i], gh);
+            ad[i] = h * pq;
+            ad[n + i] = h * pv;
+            ad[2 * n + i] = h * pf;
+        }
+        // y = L^-T r_v (scatter to the ancestors), then D^-1 (diagonal entries hold 1 / D_k)
+        for (int k = 0; k < n; ++k) y[k] = ad[n + k];
+        for (int k = 0; k < n; ++k) {
+            const double rk = ad[n + k];
+            const int rp = m.rowptr(k);
+            for (int j = m.parent(k); j >= 0; j = m.parent(j)) y[j] = fma(o[W.lf(rp + m.depth(j))], rk, y[j]);
+        }
+        for (int k = 0; k < n; ++k) y[k] *= o[W.lf(m.rowptr(k) + m.depth(k))];
+        // mu = L^-1 y, in place from the leaves up (row k reads only its ancestors, which come earlier)
+        for (int k = n - 1; k >= 0; --k) {
+            double acc = y[k];
+            const int rp = m.rowptr(k);
+            for (int j = m.parent(k); j >= 0; j = m.parent(j)) acc = fma(o[W.lf(rp + m.depth(j))], y[j], acc);
+            y[k] = acc;
+        }
+        // J_s^T r: own-joint terms, then the ancestor-pattern scatter of -(dID/dq)^T mu and -(dID/dqd)^T mu
+        for (int i = 0; i < n; ++i) {
+            const double rf = ad[2 * n + i];
+            gt[i] += fma(2.0 * m.fat(i, 1) * m.fat(i, 2) * tau[i * U + u], rf, y[i]);
+            ad[n + i] = fma(2.0 * m.fat(i, 1) * m.fat(i, 3) * o[W.vec(0, i)], rf, ad[i]);
+            ad[2 * n + i] = -m.fat(i, 0) * rf;
+            ad[i] = 0.0;
+        }
+        for (int k = 0; k < n; ++k) {
+            const int rp = m.rowptr(k);
+            const double mk = y[k];
+            for (int j = k; j >= 0; j = m.parent(j)) {
+                const int e = rp + m.depth(j);
+                ad[j] -= o[W.dqkj(e)] * mk;
+                ad[n + j] -= o[W.dvkj(e)] * mk;
+                if (j != k) {
+                    ad[k] -= o[W.dqjk(e)] * y[j];
+                    ad[n + k] -= o[W.dvjk(e)] * y[j];
+                }
+            }
+        }
+        for (int i = 0; i < 3 * n; ++i) gx[i] += ad[i];
+    }
+    for (int i = 0; i < n; ++i) {
+        a.gq[i * a.ldg + u] = gx[i];
+        a.gqd[i * a.ldg + u] = gx[n + i];
+        a.gf[i * a.ldg + u] = gx[2 * n + i];
+        a.gtau[i * a.ldgt + u] = gt[i];
+    }
+    if (a.gdt) a.gdt[u] = gh;
+}
+
 // ------------------------------------------------------------------------------------------------ T3
 MPCF_DI void cp_async8s(unsigned smem_addr, const double *gmem)
 {
@@ -975,6 +1082,55 @@ static cudaError_t run_tree(const LaunchModel &m, int npat, long U, long cnt, co
         g_launches.fetch_add(3);
     }
     return cudaGetLastError();
+}
+
+// Reverse sweep: T1, T2 and k_tree_factor (with L^-1) unchanged, then k_tree_vjp.  It needs no chain-kernel scratch and no fatigue
+// columns, so the whole workspace holds stage data.
+template <int MAXN>
+static cudaError_t run_tree_vjp(const LaunchModel &m, int npat, long U, long cnt, const double *q, const double *qd, const double *tau,
+                                const double *f, double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, double *ws,
+                                size_t ws_bytes, cudaStream_t s)
+{
+    const int n = m.n;
+    TreeWs W{n, npat, TreeWs::planes(n, npat)};
+    int dev = 0, nsm = 148;
+    cudaGetDevice(&dev);
+    cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
+    static std::atomic<bool> attr_set[64];
+    if (dev >= 0 && dev < 64 && !attr_set[dev].load(std::memory_order_acquire)) {
+        const cudaError_t e = cudaFuncSetAttribute(k_tree_factor<MAXN>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAXN > 16 ? 128 * 1024 : 48 * 1024);
+        if (e != cudaSuccess) return e;
+        attr_set[dev].store(true, std::memory_order_release);
+    }
+    const size_t per_unit = tree_ws_doubles_per_unit(n, npat) * sizeof(double);
+    long Uc = (long)(ws_bytes / per_unit);
+    Uc -= Uc % 32;
+    if (Uc < 32) return cudaErrorInvalidValue;
+    const long wave = (long)nsm * MPCF_T2_BLOCKS * 32;  // whole waves of the derivative kernel (see run_tree)
+    if (Uc > wave) Uc -= Uc % wave;
+    const size_t smem12 = blob_smem_bytes(n);
+    for (long u0 = 0; u0 < cnt; u0 += Uc) {
+        const long c = (cnt - u0) < Uc ? (cnt - u0) : Uc;
+        const unsigned gb = (unsigned)((c + kThreads - 1) / kThreads);
+        k_tree_stages<MAXN><<<gb, kThreads, smem12, s>>>(m.blob, W, U, c, q + u0, qd + u0, tau + u0, f + u0, dt, dt_u ? dt_u + u0 : nullptr,
+                                                        qn ? qn + u0 : nullptr, qdn ? qdn + u0 : nullptr, fn ? fn + u0 : nullptr, ws);
+        k_tree_derivs<MAXN><<<dim3(gb, 4), kThreads, smem12, s>>>(m.blob, W, c, ws);
+        const long blocks = (c * 4 + 7) / 8, cap = (long)nsm * 4;
+        k_tree_factor<MAXN><<<(unsigned)(blocks < cap ? blocks : cap), 256, tree_factor_smem(n, npat), s>>>(m.blob, W, c, ws, 1);
+        k_tree_vjp<MAXN><<<gb, kThreads, smem12, s>>>(m.blob, W, U, u0, c, tau, f, dt, dt_u, a, ws);
+        g_launches.fetch_add(4);
+    }
+    return cudaGetLastError();
+}
+
+cudaError_t launch_step_vjp_tree(const LaunchModel &m, int npat, long U, long cnt, const double *q, const double *qd, const double *tau,
+                                 const double *f, double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn,
+                                 double *ws, size_t ws_bytes, cudaStream_t s)
+{
+    if (cnt <= 0) return cudaSuccess;
+    if (m.n <= 16) return run_tree_vjp<16>(m, npat, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, ws_bytes, s);
+    if (m.n <= 40) return run_tree_vjp<40>(m, npat, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, ws_bytes, s);
+    return cudaErrorInvalidValue;
 }
 
 size_t tree_jvp_workspace_bytes(int n, int npat, long U)

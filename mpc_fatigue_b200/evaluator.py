@@ -224,6 +224,43 @@ class BatchEvaluator:
                 C.c_void_p(fn.data_ptr()), C.c_void_p(jac.data_ptr()), ws, ws_bytes, _stream()))
         return qn, qdn, fn, jac
 
+    def step_rk4_vjp(self, q, qd, tau, f, dt, lq=None, lqd=None, lf=None, want_dt=False):
+        """Reverse mode of `step_rk4`: with the adjoint lambda = (lq, lqd, lf) ([n, U] each; None = 0) returns
+        (gq, gqd, gtau, gf) = lambda^T d(q+, qd+, f+)/d(q, qd, tau, f), and gdt [U] = lambda^T d x+/d dt as a fifth element with
+        want_dt=True.  dt is a scalar or a per-unit tensor [U], as in `step_rk4`.  No dense Jacobian is formed."""
+        U, n = self._U(q), self.n
+        g = [self._out(None, n, U, nm) for nm in ("gq", "gqd", "gtau", "gf")]
+        gdt = self._out(None, 1, U, "gdt").view(U) if want_dt else None
+        dts, dtu = self._dt(dt, U)
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        with torch.cuda.device(self.device):
+            ws, ws_bytes = self._workspace(U)
+            _capi.check(_capi.lib.mpcf_step_rk4_vjp_batch(
+                self.model.handle, U, self._in(q, n, U, "q"), self._in(qd, n, U, "qd"), self._in(tau, n, U, "tau"),
+                self._in(f, n, U, "f"), dts, dtu, self._in(lq, n, U, "lq", True), self._in(lqd, n, U, "lqd", True),
+                self._in(lf, n, U, "lf", True), *[p(t) for t in g], p(gdt), None, None, None, ws, ws_bytes, _stream()))
+        return (*g, gdt) if want_dt else tuple(g)
+
+    def rollout_rk4_vjp(self, q0, qd0, f0, tau, N: int, dt: float, traj, gqt=None, gqdt=None, gft=None):
+        """Adjoint of `rollout_rk4`: `traj` = the (qt, qdt, ft) it returned for the same inputs, gqt/gqdt/gft [n, N*B] = dL/d(trajectory)
+        (None = 0).  Returns (gtau [n, N*B], gq0, gqd0, gf0 [n, B]) = dL/d(tau, x0).  One step VJP per node in reverse order; nothing
+        of size N*B is allocated besides gtau."""
+        if q0.dim() != 2:
+            raise ValueError("expected [n, B] initial states")
+        n, B = self.n, q0.shape[1]
+        U = B * int(N)
+        qt, qdt, ft = traj
+        gtau = self._out(None, n, U, "gtau")
+        g0 = [self._out(None, n, B, nm) for nm in ("gq0", "gqd0", "gf0")]
+        with torch.cuda.device(self.device):
+            ws, ws_bytes = self._workspace(B)
+            _capi.check(_capi.lib.mpcf_rollout_rk4_vjp_batch(
+                self.model.handle, B, int(N), self._in(q0, n, B, "q0"), self._in(qd0, n, B, "qd0"), self._in(f0, n, B, "f0"),
+                self._in(tau, n, U, "tau"), float(dt), self._in(qt, n, U, "qt"), self._in(qdt, n, U, "qdt"), self._in(ft, n, U, "ft"),
+                self._in(gqt, n, U, "gqt", True), self._in(gqdt, n, U, "gqdt", True), self._in(gft, n, U, "gft", True),
+                C.c_void_p(gtau.data_ptr()), *[C.c_void_p(t.data_ptr()) for t in g0], ws, ws_bytes, _stream()))
+        return (gtau, *g0)
+
     def step_rk4_jvp_range(self, q, qd, tau, f, dt: float, u0: int, cnt: int, out, jac):
         """Units [u0, u0 + cnt) of a larger batch: states go to columns [u0, u0 + cnt) of the full-size `out` = (qn, qdn, fn),
         the Jacobian to the chunk-local buffer jac[3n, 4n+1, cap] (cap >= cnt) — one Jacobian buffer is reused over the
