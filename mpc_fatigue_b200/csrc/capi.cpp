@@ -291,10 +291,10 @@ static int get_launch_model(const mpcf_model *m, LaunchModel &lm)
     lm.chain_params = nullptr;
     lm.blob = GenericBlob{nullptr, nullptr, h.n};
     switch (m->fam) {
-    case FAM_CHAIN3: lm.static_params = &m->sp3; return MPCF_OK;
-    case FAM_CHAIN6: lm.static_params = &m->sp6; return MPCF_OK;
+    case FAM_CHAIN3: lm.static_params = lm.chain_params = &m->sp3; return MPCF_OK;
+    case FAM_CHAIN6: lm.static_params = lm.chain_params = &m->sp6; return MPCF_OK;
     case FAM_FOREST12x6: lm.static_params = &m->sp12; lm.chain_params = m->chain6; return MPCF_OK;
-    case FAM_CHAIN7: lm.static_params = &m->sp7; return MPCF_OK;
+    case FAM_CHAIN7: lm.static_params = lm.chain_params = &m->sp7; return MPCF_OK;
     case FAM_FOREST14x7: lm.static_params = &m->sp14; lm.chain_params = m->chain7; return MPCF_OK;
     default: break;
     }
@@ -521,8 +521,34 @@ extern "C" size_t mpcf_step_rk4_jvp_workspace_bytes(const mpcf_model *model, lon
     if (!jvp2_supported(lm)) return 0;
     long units = U < kJvpChunkUnits ? U : kJvpChunkUnits;
     units = (units + 31) / 32 * 32;
-    const int nchain = family_chain_len(model->fam);  // forests run one chain at a time
-    return (size_t)units * jvp_ws_doubles_per_unit(nchain) * sizeof(double);
+    return (size_t)units * jvp_ws_bytes_per_unit(lm);
+}
+
+// The step-derivative entries' workspace: the caller's, checked (128-byte aligned, at least one 32-unit tile), or one from the
+// device's stream-ordered memory pool sized for U units (no synchronisation; the pool keeps the block after the first call, so
+// steady-state calls cost two pool look-ups).  *owned: the caller frees it with cudaFreeAsync.  Models without a workspace
+// pipeline need none.
+static int get_workspace(const mpcf_model *model, const LaunchModel &lm, long U, void *workspace, size_t workspace_bytes, cudaStream_t st,
+                         const char *alloc_what, double **ws, size_t *bytes, bool *owned)
+{
+    *ws = nullptr; *bytes = 0; *owned = false;
+    const bool tree = tree_jvp_supported(lm);
+    if (!tree && !jvp2_supported(lm)) return MPCF_OK;
+    if (workspace) {
+        const size_t min_ws = tree ? tree_jvp_workspace_bytes(model->h.n, model->npat, 32) : 32 * jvp_ws_bytes_per_unit(lm);
+        // the chain-rule kernel streams the workspace with cp.async.bulk: 16-byte aligned global addresses; chunk offsets
+        // are multiples of 256 B, so the base decides.  128 keeps every plane on a full cache line.
+        if (reinterpret_cast<uintptr_t>(workspace) % 128) return fail(MPCF_EINVAL, "workspace must be 128-byte aligned");
+        if (workspace_bytes < min_ws) return fail(MPCF_EINVAL, "workspace too small: see mpcf_step_rk4_jvp_workspace_bytes");
+        *ws = static_cast<double *>(workspace);
+        *bytes = workspace_bytes;
+        return MPCF_OK;
+    }
+    *bytes = mpcf_step_rk4_jvp_workspace_bytes(model, U);
+    const cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(ws), *bytes, st);
+    if (e != cudaSuccess) return cuda_fail(e, alloc_what);
+    *owned = true;
+    return MPCF_OK;
 }
 
 // analytic pipeline on `cnt` units (plane strides ld / ld_jac), with the coupled-fatigue pre / post kernels around it when the
@@ -564,29 +590,16 @@ extern "C" int mpcf_step_rk4_jvp_ws_batch(const mpcf_model *model, long U, const
     PROLOGUE(q && qd && tau && f && jac)
     if ((qn || qdn || fn) && !(qn && qdn && fn)) return fail(MPCF_EINVAL, "qn/qdn/fn must be all set or all NULL");
     if (int rc = check_forward_dynamics(model)) return rc;
-    const bool tree = tree_jvp_supported(lm);
-    if (!jvp2_supported(lm) && !tree)  // run-time topology with n > 40: no workspace pipeline; the workspace argument is ignored
+    if (!jvp2_supported(lm) && !tree_jvp_supported(lm))  // run-time topology with n > 40: no workspace pipeline; the workspace argument is ignored
         return done(launch_step_jvp(lm, U, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, st), "step_rk4_jvp_batch");
     if (U == 0) return MPCF_OK;
-    const size_t min_ws = tree ? tree_jvp_workspace_bytes(model->h.n, model->npat, 32)
-                               : (size_t)32 * jvp_ws_doubles_per_unit(family_chain_len(model->fam)) * sizeof(double);
-    if (workspace) {
-        // the chain-rule kernel streams the workspace with cp.async.bulk: 16-byte aligned global addresses; chunk offsets
-        // are multiples of 256 B, so the base decides.  128 keeps every plane on a full cache line.
-        if (reinterpret_cast<uintptr_t>(workspace) % 128) return fail(MPCF_EINVAL, "workspace must be 128-byte aligned");
-        if (workspace_bytes < min_ws) return fail(MPCF_EINVAL, "workspace too small: see mpcf_step_rk4_jvp_workspace_bytes");
-        return done(run_pipeline(model, lm, U, U, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, U, static_cast<double *>(workspace), workspace_bytes, st),
-                    "step_rk4_jvp_ws_batch");
-    }
-    // no caller workspace: stream-ordered allocation from the device's memory pool (no synchronisation; the pool keeps the
-    // block after the first call, so steady-state calls cost two pool look-ups)
-    const size_t bytes = mpcf_step_rk4_jvp_workspace_bytes(model, U);
-    void *ws = nullptr;
-    cudaError_t e = cudaMallocAsync(&ws, bytes, st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMallocAsync(jvp workspace)");
-    e = run_pipeline(model, lm, U, U, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, U, static_cast<double *>(ws), bytes, st);
-    const cudaError_t e2 = cudaFreeAsync(ws, st);
-    return done(e != cudaSuccess ? e : e2, "step_rk4_jvp_batch");
+    double *ws;
+    size_t bytes;
+    bool owned;
+    if (int rc = get_workspace(model, lm, U, workspace, workspace_bytes, st, "cudaMallocAsync(jvp workspace)", &ws, &bytes, &owned)) return rc;
+    const cudaError_t e = run_pipeline(model, lm, U, U, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, U, ws, bytes, st);
+    const cudaError_t e2 = owned ? cudaFreeAsync(ws, st) : cudaSuccess;
+    return done(e != cudaSuccess ? e : e2, owned ? "step_rk4_jvp_batch" : "step_rk4_jvp_ws_batch");
 }
 
 // Unit-range form: `cnt` units whose input / state planes have stride `ld` (base pointers already shifted to the range) and a
@@ -603,16 +616,14 @@ extern "C" int mpcf_step_rk4_jvp_strided_batch(const mpcf_model *model, long cnt
     if ((qn || qdn || fn) && !(qn && qdn && fn)) return fail(MPCF_EINVAL, "qn/qdn/fn must be all set or all NULL");
     if (int rc = check_forward_dynamics(model)) return rc;
     if (cnt == 0) return MPCF_OK;
-    const bool tree = tree_jvp_supported(lm);
-    if (!jvp2_supported(lm) && !tree)
+    if (!jvp2_supported(lm) && !tree_jvp_supported(lm))
         return done(launch_step_jvp(lm, ld, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, st, cnt, ld_jac), "step_rk4_jvp_strided_batch");
-    const size_t min_ws = tree ? tree_jvp_workspace_bytes(model->h.n, model->npat, 32)
-                               : (size_t)32 * jvp_ws_doubles_per_unit(family_chain_len(model->fam)) * sizeof(double);
     if (!workspace) return fail(MPCF_EINVAL, "the strided entry needs a caller workspace (mpcf_step_rk4_jvp_workspace_bytes)");
-    if (reinterpret_cast<uintptr_t>(workspace) % 128) return fail(MPCF_EINVAL, "workspace must be 128-byte aligned");
-    if (workspace_bytes < min_ws) return fail(MPCF_EINVAL, "workspace too small: see mpcf_step_rk4_jvp_workspace_bytes");
-    return done(run_pipeline(model, lm, cnt, ld, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, ld_jac, static_cast<double *>(workspace), workspace_bytes, st),
-                "step_rk4_jvp_strided_batch");
+    double *ws;
+    size_t bytes;
+    bool owned;  // false: the caller's workspace is never replaced
+    if (int rc = get_workspace(model, lm, cnt, workspace, workspace_bytes, st, "cudaMallocAsync(jvp workspace)", &ws, &bytes, &owned)) return rc;
+    return done(run_pipeline(model, lm, cnt, ld, q, qd, tau, f, dt, dt_u, qn, qdn, fn, jac, ld_jac, ws, bytes, st), "step_rk4_jvp_strided_batch");
 }
 
 extern "C" int mpcf_step_rk4_jvp_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,
@@ -631,30 +642,6 @@ static cudaError_t run_vjp(const mpcf_model *model, const LaunchModel &lm, long 
     if (tree_jvp_supported(lm)) return launch_step_vjp_tree(lm, model->npat, ld, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, ws_bytes, st);
     if (jvp2_supported(lm)) return launch_step_vjp_ws(lm, ld, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, ws_bytes, st);
     return launch_step_vjp_dual(lm, ld, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, st);
-}
-
-// the reverse entries' workspace: the caller's (checked as for mpcf_step_rk4_jvp_ws_batch) or one from the stream-ordered pool
-// (*owned set: the caller frees it with cudaFreeAsync); models without a workspace path need none
-static int vjp_workspace(const mpcf_model *model, const LaunchModel &lm, long U, void *workspace, size_t workspace_bytes, cudaStream_t st,
-                         double **ws, size_t *bytes, bool *owned)
-{
-    *ws = nullptr; *bytes = 0; *owned = false;
-    const bool tree = tree_jvp_supported(lm);
-    if (!tree && !jvp2_supported(lm)) return MPCF_OK;
-    if (workspace) {
-        const size_t min_ws = tree ? tree_jvp_workspace_bytes(model->h.n, model->npat, 32)
-                                   : (size_t)32 * jvp_ws_doubles_per_unit(family_chain_len(model->fam)) * sizeof(double);
-        if (reinterpret_cast<uintptr_t>(workspace) % 128) return fail(MPCF_EINVAL, "workspace must be 128-byte aligned");
-        if (workspace_bytes < min_ws) return fail(MPCF_EINVAL, "workspace too small: see mpcf_step_rk4_jvp_workspace_bytes");
-        *ws = static_cast<double *>(workspace);
-        *bytes = workspace_bytes;
-        return MPCF_OK;
-    }
-    *bytes = mpcf_step_rk4_jvp_workspace_bytes(model, U);
-    const cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(ws), *bytes, st);
-    if (e != cudaSuccess) return cuda_fail(e, "cudaMallocAsync(vjp workspace)");
-    *owned = true;
-    return MPCF_OK;
 }
 
 extern "C" int mpcf_step_rk4_vjp_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau, const double *f,
@@ -676,7 +663,7 @@ extern "C" int mpcf_step_rk4_vjp_batch(const mpcf_model *model, long U, const do
     double *ws;
     size_t bytes;
     bool owned;
-    if (int rc = vjp_workspace(model, lm, U, workspace, workspace_bytes, st, &ws, &bytes, &owned)) return rc;
+    if (int rc = get_workspace(model, lm, U, workspace, workspace_bytes, st, "cudaMallocAsync(vjp workspace)", &ws, &bytes, &owned)) return rc;
     const cudaError_t e = run_vjp(model, lm, U, U, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, bytes, st);
     const cudaError_t e2 = owned ? cudaFreeAsync(ws, st) : cudaSuccess;
     return done(e != cudaSuccess ? e : e2, "step_rk4_vjp_batch");
@@ -701,7 +688,7 @@ extern "C" int mpcf_rollout_rk4_vjp_batch(const mpcf_model *model, long B, int N
     double *ws;
     size_t bytes;
     bool owned;
-    if (int rc = vjp_workspace(model, lm, B, workspace, workspace_bytes, st, &ws, &bytes, &owned)) return rc;
+    if (int rc = get_workspace(model, lm, B, workspace, workspace_bytes, st, "cudaMallocAsync(vjp workspace)", &ws, &bytes, &owned)) return rc;
     double *scr = nullptr;  // [3n][B] adjoint of the odd nodes | [n][B] tau of node 0
     cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&scr), (size_t)4 * n * B * sizeof(double), st);
     if (e != cudaSuccess) {

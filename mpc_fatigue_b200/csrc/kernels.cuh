@@ -53,7 +53,7 @@ struct LaunchModel {
     int n;
     GenericBlob blob;
     const void *static_params;  // host pointer to StaticParams<N> for static families
-    const void *chain_params;   // forests: host array of StaticParams<L>, one per chain
+    const void *chain_params;   // static families: host array of StaticParams<L>, one per serial chain
 };
 
 struct CostArgs {
@@ -97,7 +97,7 @@ cudaError_t launch_cost_residual_table(int n, long B, int N, const double *q, co
 cudaError_t launch_gather_planes(const double *src, double *dst, const int *map, int nplanes, long U, long ld_src, cudaStream_t s);
 // analytic Jacobian pipeline (kernels_jvp2.cu): static chain families, caller-provided workspace
 bool jvp2_supported(const LaunchModel &m);
-size_t jvp_ws_doubles_per_unit(int n);
+size_t jvp_ws_bytes_per_unit(const LaunchModel &m);  // forests run one chain at a time: the chain length sizes it
 cudaError_t launch_step_jvp_ws(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, const double *f,
                                double dt, const double *dt_u, double *qn, double *qdn, double *fn, double *jac, double *ws,
                                size_t ws_bytes, cudaStream_t s, long cnt = -1, long UJ = 0, const double *theat = nullptr, long UT = 0);

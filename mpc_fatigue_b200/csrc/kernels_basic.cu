@@ -289,10 +289,11 @@ cudaError_t launch_cost_residual_table(int n, long B, int N, const double *q, co
                                        const double *table, double *out, long ld_out, cudaStream_t s)
 {
     if (B <= 0) return cudaSuccess;
+    constexpr int kMaxSmem = 200 * 1024;
     const size_t smem = (size_t)2 * n * N * sizeof(double);
-    if (smem > 200 * 1024) return cudaErrorInvalidValue;
-    if (smem > 48 * 1024) {
-        cudaError_t e = cudaFuncSetAttribute(cost_residual_table_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+    if (smem > kMaxSmem) return cudaErrorInvalidValue;
+    if (smem > 48 * 1024) {  // one limit for every table size: the largest accepted
+        const cudaError_t e = raise_smem_limit<cost_residual_table_kernel>(kMaxSmem);
         if (e != cudaSuccess) return e;
     }
     cost_residual_table_kernel<<<(unsigned)((B + 255) / 256), 256, smem, s>>>(n, B, N, q, qd, f, tau, qn, qdn, fn, w_qd, w_tau, f_max, table, out,
@@ -500,63 +501,32 @@ __global__ void __launch_bounds__(kThreads) jtw_chain_kernel(const __grid_consta
         if (i < c0 || i >= c0 + N) out[(long)i * U + u] = 0.0;
 }
 
-// frame on a chain of a static family: which chain, its parameters, the frame with the joint index made chain-relative
-template <int L>
-static bool chain_frame(const LaunchModel &m, const FrameArg &f, const StaticParams<L> *&cp, FrameArg &fc, int &c0)
-{
-    if (f.joint < 0) return false;  // world-fixed frame: constant pose, the generic body handles it
-    const int c = f.joint / L;
-    c0 = c * L;
-    cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params) + c;
-    fc = f;
-    fc.joint = f.joint - c0;
-    return true;
-}
-
-template <int L>
-static cudaError_t frames_chain(int what, const LaunchModel &m, const FrameArg &f, long U, const double *q, const double *W, double *o0,
-                                double *o1, cudaStream_t s, bool &done)
-{
-    const StaticParams<L> *cp;
-    FrameArg fc;
-    int c0;
-    done = chain_frame<L>(m, f, cp, fc, c0);
-    if (!done) return cudaSuccess;
-    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
-    const double *qc = q + (size_t)c0 * U;
-    if (what == 0) fk_chain_kernel<L><<<gb, kThreads, 0, s>>>(*cp, U, fc, qc, o0, o1);
-    else if (what == 1) jac_chain_kernel<L><<<gb, kThreads, 0, s>>>(*cp, U, fc, qc, o0, m.n, c0);
-    else jtw_chain_kernel<L><<<gb, kThreads, 0, s>>>(*cp, U, fc, qc, W, o0, m.n, c0);
-    g_launches.fetch_add(1);
-    return cudaGetLastError();
-}
-
-// what: 0 = pose, 1 = Jacobian, 2 = J^T W.  Returns true when a static-chain kernel took the call.
-static bool frames_static(int what, const LaunchModel &m, const FrameArg &f, long U, const double *q, const double *W, double *o0, double *o1,
-                          cudaStream_t s, cudaError_t &e)
-{
-    bool done = false;
-    switch (family_chain_len(m.fam)) {
-    case 3: e = frames_chain<3>(what, m, f, U, q, W, o0, o1, s, done); break;
-    case 6: e = frames_chain<6>(what, m, f, U, q, W, o0, o1, s, done); break;
-    case 7: e = frames_chain<7>(what, m, f, U, q, W, o0, o1, s, done); break;
-    default: break;
-    }
-    return done;
-}
-
+// A frame on a chain of a static family goes to that chain's kernel (chain f.joint / L, joint index made chain-relative); a
+// world-fixed frame (f.joint < 0) has a constant pose and takes the generic body.
 cudaError_t launch_fk(const LaunchModel &m, const FrameArg &f, long U, const double *q, double *pos, double *rot, cudaStream_t s)
 {
     if (U <= 0) return cudaSuccess;
-    cudaError_t e = cudaSuccess;
-    if (frames_static(0, m, f, U, q, nullptr, pos, rot, s, e)) return e;
+    if (f.joint >= 0 && with_chains(m, [&](auto L, const auto *chains, auto) {
+            FrameArg fc = f;
+            fc.joint = f.joint % L;
+            const int c0 = f.joint - fc.joint;
+            fk_chain_kernel<L><<<(unsigned)((U + kThreads - 1) / kThreads), kThreads, 0, s>>>(chains[c0 / L], U, fc, q + (size_t)c0 * U, pos, rot);
+            g_launches.fetch_add(1);
+        }))
+        return cudaGetLastError();
     return dispatch<FkBody>(m, U, 1, s, f, q, pos, rot);
 }
 cudaError_t launch_jac(const LaunchModel &m, const FrameArg &f, long U, const double *q, double *J, cudaStream_t s)
 {
     if (U <= 0) return cudaSuccess;
-    cudaError_t e = cudaSuccess;
-    if (frames_static(1, m, f, U, q, nullptr, J, nullptr, s, e)) return e;
+    if (f.joint >= 0 && with_chains(m, [&](auto L, const auto *chains, auto) {
+            FrameArg fc = f;
+            fc.joint = f.joint % L;
+            const int c0 = f.joint - fc.joint;
+            jac_chain_kernel<L><<<(unsigned)((U + kThreads - 1) / kThreads), kThreads, 0, s>>>(chains[c0 / L], U, fc, q + (size_t)c0 * U, J, m.n, c0);
+            g_launches.fetch_add(1);
+        }))
+        return cudaGetLastError();
     return dispatch<JacBody>(m, U, 1, s, f, q, J);
 }
 // Contact wrenches as external link forces of the RNEA (serial chain): W_e = [F ; n] is given in world axes at the frame
@@ -656,45 +626,36 @@ __global__ void __launch_bounds__(kThreads, 3) node_eval_chain_kernel(const __gr
     }
 }
 
-template <int L>
-static cudaError_t node_eval_chains(const LaunchModel &m, const EeArgs &ee, double wsign, long U, const double *q, const double *qd,
-                                    const double *qdd, const double *W, const double *T, double h, const ZohArg &zoh, double *tau,
-                                    double *qnext, double *Tnext, cudaStream_t s)
-{
-    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params);
-    for (int c = 0; c < m.n / L; ++c) {
-        const size_t off = (size_t)c * L * U;
-        auto at = [off](auto *p) { return p ? p + off : p; };
-        auto go = [&](auto kern) {
-            kern<<<gb, kThreads, 0, s>>>(cp[c], U, ee, wsign, q + off, at(qd), at(qdd), W, at(T), h, zoh, tau + off, at(qnext), at(Tnext), c * L);
-        };
-        if (ee.nee == 0) go(node_eval_chain_kernel<L, 0>);
-        else if (ee.nee == 1) go(node_eval_chain_kernel<L, 1>);
-        else if (ee.nee == 2) go(node_eval_chain_kernel<L, 2>);
-        else go(node_eval_chain_kernel<L, MPCF_MAX_EE>);
-        g_launches.fetch_add(1);
-    }
-    return cudaGetLastError();
-}
-
 cudaError_t launch_node_eval(const LaunchModel &m, const EeArgs &ee, double wsign, long U, const double *q, const double *qd,
                              const double *qdd, const double *W, const double *T, double h, const ZohArg &zoh, double *tau,
                              double *qnext, double *Tnext, bool jtw_only, cudaStream_t s)
 {
     if (U <= 0) return cudaSuccess;
-    if (jtw_only && ee.nee == 1 && wsign == 1.0) {
-        cudaError_t e = cudaSuccess;
-        if (frames_static(2, m, ee.f[0], U, q, W, tau, nullptr, s, e)) return e;
-    }
-    if (!jtw_only) {
-        switch (family_chain_len(m.fam)) {
-        case 3: return node_eval_chains<3>(m, ee, wsign, U, q, qd, qdd, W, T, h, zoh, tau, qnext, Tnext, s);
-        case 6: return node_eval_chains<6>(m, ee, wsign, U, q, qd, qdd, W, T, h, zoh, tau, qnext, Tnext, s);
-        case 7: return node_eval_chains<7>(m, ee, wsign, U, q, qd, qdd, W, T, h, zoh, tau, qnext, Tnext, s);
-        default: break;
-        }
-    }
+    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
+    const FrameArg &f = ee.f[0];
+    if (jtw_only && ee.nee == 1 && wsign == 1.0 && f.joint >= 0 && with_chains(m, [&](auto L, const auto *chains, auto) {
+            FrameArg fc = f;
+            fc.joint = f.joint % L;
+            const int c0 = f.joint - fc.joint;
+            jtw_chain_kernel<L><<<gb, kThreads, 0, s>>>(chains[c0 / L], U, fc, q + (size_t)c0 * U, W, tau, m.n, c0);
+            g_launches.fetch_add(1);
+        }))
+        return cudaGetLastError();
+    if (!jtw_only && with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+            for (int c = 0; c < nchains; ++c) {
+                const size_t off = (size_t)c * L * U;
+                auto at = [off](auto *p) { return p ? p + off : p; };
+                auto go = [&](auto kern) {
+                    kern<<<gb, kThreads, 0, s>>>(chains[c], U, ee, wsign, q + off, at(qd), at(qdd), W, at(T), h, zoh, tau + off, at(qnext), at(Tnext), c * L);
+                };
+                if (ee.nee == 0) go(node_eval_chain_kernel<L, 0>);
+                else if (ee.nee == 1) go(node_eval_chain_kernel<L, 1>);
+                else if (ee.nee == 2) go(node_eval_chain_kernel<L, 2>);
+                else go(node_eval_chain_kernel<L, MPCF_MAX_EE>);
+                g_launches.fetch_add(1);
+            }
+        }))
+        return cudaGetLastError();
     return dispatch<NodeEvalBody>(m, U, 1, s, ee, wsign, q, qd, qdd, W, T, h, zoh, tau, qnext, Tnext, jtw_only);
 }
 cudaError_t launch_node_eval_jvp_dual(const LaunchModel &m, const EeArgs &ee, double wsign, long U, const double *q, const double *qd,

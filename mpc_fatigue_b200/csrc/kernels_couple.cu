@@ -138,18 +138,6 @@ __global__ void __launch_bounds__(kThreads) k_couple(const __grid_constant__ Sta
     }
 }
 
-template <int L>
-static cudaError_t couple_launch(const LaunchModel &m, const CoupleArgs &ca, long cnt, long ld, const double *q, const double *f,
-                                 const double *tau, double *theat, long ld_t, int mode, double dt, const double *dt_u, double *jac, long UJ,
-                                 cudaStream_t s)
-{
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.chain_params);
-    k_couple<L><<<(unsigned)((cnt + kThreads - 1) / kThreads), kThreads, 0, s>>>(cp[0], cp[1], ca, cnt, ld, q, f, tau, theat, ld_t, mode, dt, dt_u, jac,
-                                                                                UJ);
-    g_launches.fetch_add(1);
-    return cudaGetLastError();
-}
-
 // mode 0: theat[n][ld_t] = tau + share * g(q).  mode 1: patch the fatigue rows of jac (plane stride UJ) after the pipeline.
 cudaError_t launch_couple(const LaunchModel &m, const CoupleHost &ch, long cnt, long ld, const double *q, const double *f, const double *tau,
                           double *theat, long ld_t, int mode, double dt, const double *dt_u, double *jac, long UJ, cudaStream_t s)
@@ -161,11 +149,16 @@ cudaError_t launch_couple(const LaunchModel &m, const CoupleHost &ch, long cnt, 
         ca.ee_joint[c] = ch.ee_joint[c];
         for (int k = 0; k < 3; ++k) ca.ee_p[c][k] = ch.ee_p[c][k];
     }
-    switch (m.fam) {
-    case FAM_FOREST12x6: return couple_launch<6>(m, ca, cnt, ld, q, f, tau, theat, ld_t, mode, dt, dt_u, jac, UJ, s);
-    case FAM_FOREST14x7: return couple_launch<7>(m, ca, cnt, ld, q, f, tau, theat, ld_t, mode, dt, dt_u, jac, UJ, s);
-    default: return cudaErrorInvalidValue;
-    }
+    cudaError_t e = cudaErrorInvalidValue;  // the two-arm families only
+    with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+        if constexpr (decltype(nchains)::value == 2) {
+            k_couple<L><<<(unsigned)((cnt + kThreads - 1) / kThreads), kThreads, 0, s>>>(chains[0], chains[1], ca, cnt, ld, q, f, tau, theat, ld_t,
+                                                                                        mode, dt, dt_u, jac, UJ);
+            g_launches.fetch_add(1);
+            e = cudaGetLastError();
+        }
+    });
+    return e;
 }
 
 }  // namespace mpcf

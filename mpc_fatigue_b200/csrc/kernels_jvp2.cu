@@ -43,7 +43,6 @@ struct WsLayout {
     // chunk of (tile, stage)
     static MPCF_DI size_t chunk(long tile, int s) { return ((size_t)tile * 4 + s) * kStageDoubles; }
 };
-size_t jvp_ws_doubles_per_unit(int n) { return (size_t)4 * (3 * n * n + 4 * n); }
 
 // ------------------------------------------------------------------------------------------------ K1
 template <int N, int L>
@@ -877,20 +876,25 @@ struct K2Config {
     static constexpr bool kSmem = N == L && 2 * kSlab <= 227 * 1024;
 };
 
-// K1 + K2 of one chunk of units [u0, u0 + cnt): what the Jacobian (K3) and the reverse sweep (k_step_vjp) read.  The caller has set
-// K2's shared-memory attribute.
+// K1 + K2 of one chunk of units [u0, u0 + cnt): what the Jacobian (K3) and the reverse sweep (k_step_vjp) read
 template <int N, int L>
-static void launch_stages_derivs(const StaticParams<N> &P, long U, long u0, long cnt, const double *q, const double *qd, const double *tau,
+static cudaError_t launch_stages_derivs(const StaticParams<N> &P, long U, long u0, long cnt, const double *q, const double *qd, const double *tau,
                                  const double *theat, long UT, const double *f, double dt, const double *dt_u, double *qn, double *qdn,
                                  double *fn, double *ws, cudaStream_t s)
 {
     using K2 = K2Config<N, L>;
+    static const int k2smem = getenv("MPCF_K2_SMEM") ? atoi(getenv("MPCF_K2_SMEM")) : 1;
+    if constexpr (K2::kSmem) {
+        if (k2smem) {
+            const cudaError_t e = raise_smem_limit<k_stage_derivs<N, L, true>>(K2::kSlab);
+            if (e != cudaSuccess) return e;
+        }
+    }
     const unsigned gb = (unsigned)((cnt + kThreads - 1) / kThreads);
     cudaEvent_t pe = prof_begin(0, s);
     k_step_stages<N, L><<<gb, kThreads, 0, s>>>(P, U, u0, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, ws);
     prof_end(pe, s);
     pe = prof_begin(1, s);
-    static const int k2smem = getenv("MPCF_K2_SMEM") ? atoi(getenv("MPCF_K2_SMEM")) : 1;
     bool k2done = false;
     if constexpr (K2::kSmem) {
         if (k2smem) {
@@ -900,13 +904,14 @@ static void launch_stages_derivs(const StaticParams<N> &P, long U, long u0, long
     }
     if (!k2done) k_stage_derivs<N, L, false><<<dim3(gb, 4), kThreads, 0, s>>>(P, cnt, ws);
     prof_end(pe, s);
+    return cudaSuccess;
 }
 
 template <int N, int L>
 static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const double *q, const double *qd, const double *tau, const double *theat,
                             long UT, const double *f,
                             double dt, const double *dt_u, double *qn, double *qdn, double *fn, double *jac, long UJ, double *ws, long Uc,
-                            cudaStream_t s, int ntot = N, int c0 = 0)
+                            cudaStream_t s, int ntot, int c0)
 {
     using W = WsLayout<N>;
     // chain-rule kernel: bulk-copy ring of up to 5 slots (a deeper ring takes the shared-memory carve-out from L1, which the
@@ -917,36 +922,20 @@ static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const d
     constexpr int NBUF = kTma ? (kRingMax > 5 ? 5 : kRingMax) : 0;  // measured on chain6: 5 slots 11.74 ms, 4: 11.89, 6: 12.08, 7: 12.93 (L1 gets what the ring leaves)
     constexpr int kCpwDefault = (3 * N + 1 <= 19) ? 1 : 2;
     constexpr size_t smem = (size_t)NBUF * W::kRingBytes + 2 * NBUF * sizeof(unsigned long long);
-    using K2 = K2Config<N, L>;
-    constexpr bool kK2Smem = K2::kSmem;
     if constexpr (kTma) {
-        // function attributes are per device: set them once on each device a process uses (idempotent, so two threads
-        // racing through the first call is harmless; the flag is atomic)
-        static std::atomic<bool> attr_set[64];
-        const int dev = current_device();
-        if (!attr_set[dev].load(std::memory_order_acquire)) {
-            cudaError_t e = cudaSuccess;
-            if constexpr (kCpwDefault == 1) {
-                e = cudaFuncSetAttribute(k_chain_rule_tma<N, L, NBUF, 1, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e != cudaSuccess) return e;
-                e = cudaFuncSetAttribute(k_chain_rule_tma<N, L, NBUF, 1, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-                if (e != cudaSuccess) return e;
-            }
-            e = cudaFuncSetAttribute(k_chain_rule_tma<N, L, NBUF, 2, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            e = cudaFuncSetAttribute(k_chain_rule_tma<N, L, NBUF, 2, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
-            if (e != cudaSuccess) return e;
-            if constexpr (kK2Smem) {
-                e = cudaFuncSetAttribute(k_stage_derivs<N, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2::kSlab);
-                if (e != cudaSuccess) return e;
-            }
-            attr_set[dev].store(true, std::memory_order_release);
+        cudaError_t e = cudaSuccess;
+        if constexpr (kCpwDefault == 1) {
+            if ((e = raise_smem_limit<k_chain_rule_tma<N, L, NBUF, 1, true>>((int)smem)) != cudaSuccess) return e;
+            if ((e = raise_smem_limit<k_chain_rule_tma<N, L, NBUF, 1, false>>((int)smem)) != cudaSuccess) return e;
         }
+        if ((e = raise_smem_limit<k_chain_rule_tma<N, L, NBUF, 2, true>>((int)smem)) != cudaSuccess) return e;
+        if ((e = raise_smem_limit<k_chain_rule_tma<N, L, NBUF, 2, false>>((int)smem)) != cudaSuccess) return e;
     }
     for (long u0 = 0; u0 < Ucnt; u0 += Uc) {
         const long cnt = (Ucnt - u0) < Uc ? (Ucnt - u0) : Uc;
         const long ntiles = (cnt + 31) / 32;
-        launch_stages_derivs<N, L>(P, U, u0, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, ws, s);
+        const cudaError_t e = launch_stages_derivs<N, L>(P, U, u0, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, ws, s);
+        if (e != cudaSuccess) return e;
         cudaEvent_t pe = prof_begin(2, s);
         if constexpr (kTma) {
             const unsigned g3 = (unsigned)(ntiles < sm_count() ? ntiles : sm_count());
@@ -968,8 +957,6 @@ static cudaError_t run_jvp2(const StaticParams<N> &P, long U, long Ucnt, const d
     return cudaGetLastError();
 }
 
-// Forests: the chains are dynamically decoupled, so each runs the single-chain pipeline on its own input planes and writes its
-// block of the whole-model Jacobian (plus the zeros of the cross blocks).
 // Forest Jacobians: every entry between joints of different chains is structurally zero (columns q, qd, tau, f; the dt column
 // is dense).  One coalesced pass: thread = unit, blockIdx.y = Jacobian row, loop over the columns of the other chains.
 template <int L, class V>
@@ -991,28 +978,24 @@ __global__ void __launch_bounds__(256) k_forest_fill_cross(int ntot, long cntv, 
         }
 }
 
-template <int L>
-static cudaError_t run_forest(const LaunchModel &m, long U, long Ucnt, const double *q, const double *qd, const double *tau, const double *theat,
-                              long UT, const double *f, double dt,
-                              const double *dt_u, double *qn, double *qdn, double *fn, double *jac, long UJ, double *ws, long Uc, cudaStream_t s)
-{
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.chain_params);
-    for (int c = 0; c < m.n / L; ++c) {
-        const size_t off = (size_t)c * L * U;
-        cudaError_t e = run_jvp2<L, L>(cp[c], U, Ucnt, q + off, qd + off, tau + off, theat + (size_t)c * L * UT, UT, f + off, dt, dt_u, qn ? qn + off : nullptr,
-                                       qdn ? qdn + off : nullptr, fn ? fn + off : nullptr, jac, UJ, ws, Uc, s, m.n, L * c);
-        if (e != cudaSuccess) return e;
-    }
-    if (Ucnt % 2 == 0 && UJ % 2 == 0 && (reinterpret_cast<size_t>(jac) & 15) == 0)
-        k_forest_fill_cross<L, double2><<<dim3((unsigned)((Ucnt / 2 + 255) / 256), 3 * m.n), 256, 0, s>>>(m.n, Ucnt / 2, UJ, jac);
-    else
-        k_forest_fill_cross<L, double><<<dim3((unsigned)((Ucnt + 255) / 256), 3 * m.n), 256, 0, s>>>(m.n, Ucnt, UJ, jac);
-    g_launches.fetch_add(1);
-    return cudaGetLastError();
-}
-
 bool jvp2_supported(const LaunchModel &m) { return family_chain_len(m.fam) > 0; }
 
+size_t jvp_ws_bytes_per_unit(const LaunchModel &m)
+{
+    size_t bytes = 0;
+    with_chains(m, [&](auto L, const auto *, auto) { bytes = WsLayout<L>::kUnitDoubles * sizeof(double); });
+    return bytes;
+}
+
+// units per chunk of the pipeline in ws_bytes of workspace: whole 32-unit tiles
+static long jvp_chunk_units(const LaunchModel &m, size_t ws_bytes)
+{
+    const long Uc = (long)(ws_bytes / jvp_ws_bytes_per_unit(m));
+    return Uc - Uc % 32;
+}
+
+// Forests: the chains are dynamically decoupled, so each runs the single-chain pipeline on its own input planes and writes its
+// block of the whole-model Jacobian; k_forest_fill_cross then writes the zeros of the cross blocks.
 cudaError_t launch_step_jvp_ws(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, const double *f,
                                double dt, const double *dt_u, double *qn, double *qdn, double *fn, double *jac, double *ws,
                                size_t ws_bytes, cudaStream_t s, long cnt, long UJ, const double *theat, long UT)
@@ -1023,24 +1006,26 @@ cudaError_t launch_step_jvp_ws(const LaunchModel &m, long U, const double *q, co
     if (cnt < 0) cnt = U;
     if (UJ <= 0) UJ = U;
     if (cnt <= 0) return cudaSuccess;
-    const size_t per_unit = jvp_ws_doubles_per_unit(family_chain_len(m.fam)) * sizeof(double);
-    long Uc = (long)(ws_bytes / per_unit);
-    Uc -= Uc % 32;  // whole 32-unit tiles
+    const long Uc = jvp_chunk_units(m, ws_bytes);
     if (Uc < 32) return cudaErrorInvalidValue;
-    switch (m.fam) {
-    case FAM_CHAIN3:
-        return run_jvp2<3, 3>(*static_cast<const StaticParams<3> *>(m.static_params), U, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, jac, UJ, ws, Uc, s);
-    case FAM_CHAIN6:
-        return run_jvp2<6, 6>(*static_cast<const StaticParams<6> *>(m.static_params), U, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, jac, UJ, ws, Uc, s);
-    case FAM_CHAIN7:
-        return run_jvp2<7, 7>(*static_cast<const StaticParams<7> *>(m.static_params), U, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, jac, UJ, ws, Uc, s);
-    case FAM_FOREST12x6:
-        return run_forest<6>(m, U, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, jac, UJ, ws, Uc, s);
-    case FAM_FOREST14x7:
-        return run_forest<7>(m, U, cnt, q, qd, tau, theat, UT, f, dt, dt_u, qn, qdn, fn, jac, UJ, ws, Uc, s);
-    default:
-        return cudaErrorInvalidValue;
-    }
+    cudaError_t e = cudaErrorInvalidValue;
+    with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+        for (int c = 0; c < nchains; ++c) {
+            const size_t off = (size_t)c * L * U;
+            e = run_jvp2<L, L>(chains[c], U, cnt, q + off, qd + off, tau + off, theat + (size_t)c * L * UT, UT, f + off, dt, dt_u,
+                               qn ? qn + off : nullptr, qdn ? qdn + off : nullptr, fn ? fn + off : nullptr, jac, UJ, ws, Uc, s, m.n, c * L);
+            if (e != cudaSuccess) return;
+        }
+        if constexpr (decltype(nchains)::value > 1) {
+            if (cnt % 2 == 0 && UJ % 2 == 0 && (reinterpret_cast<size_t>(jac) & 15) == 0)
+                k_forest_fill_cross<L, double2><<<dim3((unsigned)((cnt / 2 + 255) / 256), 3 * m.n), 256, 0, s>>>(m.n, cnt / 2, UJ, jac);
+            else
+                k_forest_fill_cross<L, double><<<dim3((unsigned)((cnt + 255) / 256), 3 * m.n), 256, 0, s>>>(m.n, cnt, UJ, jac);
+            g_launches.fetch_add(1);
+            e = cudaGetLastError();
+        }
+    });
+    return e;
 }
 
 // Reverse sweep of one serial chain: K1 and K2 unchanged over the same chunks as run_jvp2, then k_step_vjp in place of K3.
@@ -1050,38 +1035,14 @@ static cudaError_t run_vjp2(const StaticParams<N> &P, long U, long Ucnt, const d
                             double dt, const double *dt_u, const VjpArgs &a, int gdt_add, double *qn, double *qdn, double *fn, double *ws, long Uc,
                             cudaStream_t s)
 {
-    using K2 = K2Config<N, L>;
-    if constexpr (K2::kSmem) {
-        static std::atomic<bool> attr_set[64];
-        const int dev = current_device();
-        if (!attr_set[dev].load(std::memory_order_acquire)) {
-            const cudaError_t e = cudaFuncSetAttribute(k_stage_derivs<N, L, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, K2::kSlab);
-            if (e != cudaSuccess) return e;
-            attr_set[dev].store(true, std::memory_order_release);
-        }
-    }
     for (long u0 = 0; u0 < Ucnt; u0 += Uc) {
         const long cnt = (Ucnt - u0) < Uc ? (Ucnt - u0) : Uc;
-        launch_stages_derivs<N, L>(P, U, u0, cnt, q, qd, tau, tau, U, f, dt, dt_u, qn, qdn, fn, ws, s);
+        const cudaError_t e = launch_stages_derivs<N, L>(P, U, u0, cnt, q, qd, tau, tau, U, f, dt, dt_u, qn, qdn, fn, ws, s);
+        if (e != cudaSuccess) return e;
         k_step_vjp<N, L><<<(unsigned)((cnt + kThreads - 1) / kThreads), kThreads, 0, s>>>(P, U, u0, cnt, tau, dt, dt_u, a, gdt_add, ws);
         g_launches.fetch_add(3);
     }
     return cudaGetLastError();
-}
-
-template <int L>
-static cudaError_t vjp_chains(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
-                              double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, double *ws, long Uc,
-                              cudaStream_t s)
-{
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params);
-    for (int c = 0; c < m.n / L; ++c) {
-        const size_t off = (size_t)c * L * U;
-        const cudaError_t e = run_vjp2<L, L>(cp[c], U, cnt, q + off, qd + off, tau + off, f + off, dt, dt_u, a.rows(c * L), c > 0,
-                                             qn ? qn + off : nullptr, qdn ? qdn + off : nullptr, fn ? fn + off : nullptr, ws, Uc, s);
-        if (e != cudaSuccess) return e;
-    }
-    return cudaSuccess;
 }
 
 cudaError_t launch_step_vjp_ws(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
@@ -1089,110 +1050,86 @@ cudaError_t launch_step_vjp_ws(const LaunchModel &m, long U, long cnt, const dou
                                size_t ws_bytes, cudaStream_t s)
 {
     if (cnt <= 0) return cudaSuccess;
-    const size_t per_unit = jvp_ws_doubles_per_unit(family_chain_len(m.fam)) * sizeof(double);
-    long Uc = (long)(ws_bytes / per_unit);
-    Uc -= Uc % 32;  // whole 32-unit tiles
+    const long Uc = jvp_chunk_units(m, ws_bytes);
     if (Uc < 32) return cudaErrorInvalidValue;
-    switch (family_chain_len(m.fam)) {
-    case 3: return vjp_chains<3>(m, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, Uc, s);
-    case 6: return vjp_chains<6>(m, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, Uc, s);
-    case 7: return vjp_chains<7>(m, U, cnt, q, qd, tau, f, dt, dt_u, a, qn, qdn, fn, ws, Uc, s);
-    default: return cudaErrorInvalidValue;
-    }
+    cudaError_t e = cudaErrorInvalidValue;
+    with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+        for (int c = 0; c < nchains; ++c) {
+            const size_t off = (size_t)c * L * U;
+            e = run_vjp2<L, L>(chains[c], U, cnt, q + off, qd + off, tau + off, f + off, dt, dt_u, a.rows(c * L), c > 0, qn ? qn + off : nullptr,
+                               qdn ? qdn + off : nullptr, fn ? fn + off : nullptr, ws, Uc, s);
+            if (e != cudaSuccess) return;
+        }
+    });
+    return e;
 }
 
 // shared-memory slab of the streaming derivative kernels: (S, xi, eta) of links 0 .. n-2, one column per thread
 static constexpr int link_slab_bytes(int n) { return 18 * (n - 1) * kThreads * (int)sizeof(double); }
 
-template <int L>
-static cudaError_t node_eval_jvp_chains(const LaunchModel &m, const EeArgs &ee, double wsign, long U, const double *q, const double *qd,
-                                        const double *qdd, const double *W, double *dtau_dq, double *dtau_dqd, cudaStream_t s)
-{
-    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params);
-    for (int c = 0; c < m.n / L; ++c) {
-        const size_t off = (size_t)c * L * U;
-        auto go = [&](auto kern) {
-            cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, link_slab_bytes(L));
-            if (e != cudaSuccess) return e;
-            kern<<<gb, kThreads, link_slab_bytes(L), s>>>(cp[c], U, ee, wsign, q + off, qd + off, qdd ? qdd + off : nullptr, W, dtau_dq, dtau_dqd,
-                                                         m.n, c * L);
-            return cudaSuccess;
-        };
-        const cudaError_t e = ee.nee == 0 ? go(k_node_eval_jvp<L, 0>) : ee.nee == 1 ? go(k_node_eval_jvp<L, 1>)
-                              : ee.nee == 2 ? go(k_node_eval_jvp<L, 2>) : go(k_node_eval_jvp<L, MPCF_MAX_EE>);
-        if (e != cudaSuccess) return e;
-        g_launches.fetch_add(1);
-    }
-    return cudaGetLastError();
-}
-
 cudaError_t launch_node_eval_jvp(const LaunchModel &m, const EeArgs &ee, double wsign, long U, const double *q, const double *qd,
                                  const double *qdd, const double *W, double *dtau_dq, double *dtau_dqd, cudaStream_t s)
 {
     if (U <= 0) return cudaSuccess;
-    switch (family_chain_len(m.fam)) {
-    case 3: return node_eval_jvp_chains<3>(m, ee, wsign, U, q, qd, qdd, W, dtau_dq, dtau_dqd, s);
-    case 6: return node_eval_jvp_chains<6>(m, ee, wsign, U, q, qd, qdd, W, dtau_dq, dtau_dqd, s);
-    case 7: return node_eval_jvp_chains<7>(m, ee, wsign, U, q, qd, qdd, W, dtau_dq, dtau_dqd, s);
-    default: return launch_node_eval_jvp_dual(m, ee, wsign, U, q, qd, qdd, W, dtau_dq, dtau_dqd, s);
-    }
-}
-
-template <int L>
-static cudaError_t rnea_derivs_chains(const LaunchModel &m, long U, const double *q, const double *qd, const double *qdd, double *Dq, double *Dv,
-                                      double *M, cudaStream_t s)
-{
-    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params);
-    const cudaError_t e = cudaFuncSetAttribute(k_rnea_derivs<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, link_slab_bytes(L));
-    if (e != cudaSuccess) return e;
-    for (int c = 0; c < m.n / L; ++c) {
-        const size_t off = (size_t)c * L * U;
-        k_rnea_derivs<L><<<gb, kThreads, link_slab_bytes(L), s>>>(cp[c], U, q + off, qd + off, qdd ? qdd + off : nullptr, Dq, Dv, M, m.n, c * L);
-        g_launches.fetch_add(1);
-    }
-    return cudaGetLastError();
+    cudaError_t e = cudaSuccess;
+    if (with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+            auto go = [&](auto nee) {
+                constexpr auto kern = k_node_eval_jvp<L, decltype(nee)::value>;
+                if ((e = raise_smem_limit<kern>(link_slab_bytes(L))) != cudaSuccess) return;
+                for (int c = 0; c < nchains; ++c) {
+                    const size_t off = (size_t)c * L * U;
+                    kern<<<(unsigned)((U + kThreads - 1) / kThreads), kThreads, link_slab_bytes(L), s>>>(
+                        chains[c], U, ee, wsign, q + off, qd + off, qdd ? qdd + off : nullptr, W, dtau_dq, dtau_dqd, m.n, c * L);
+                    g_launches.fetch_add(1);
+                }
+                e = cudaGetLastError();
+            };
+            using std::integral_constant;
+            if (ee.nee == 0) go(integral_constant<int, 0>{});
+            else if (ee.nee == 1) go(integral_constant<int, 1>{});
+            else if (ee.nee == 2) go(integral_constant<int, 2>{});
+            else go(integral_constant<int, MPCF_MAX_EE>{});
+        }))
+        return e;
+    return launch_node_eval_jvp_dual(m, ee, wsign, U, q, qd, qdd, W, dtau_dq, dtau_dqd, s);
 }
 
 cudaError_t launch_rnea_derivs(const LaunchModel &m, long U, const double *q, const double *qd, const double *qdd, double *Dq, double *Dv,
                                double *M, cudaStream_t s)
 {
     if (U <= 0) return cudaSuccess;
-    switch (family_chain_len(m.fam)) {
-    case 3: return rnea_derivs_chains<3>(m, U, q, qd, qdd, Dq, Dv, M, s);
-    case 6: return rnea_derivs_chains<6>(m, U, q, qd, qdd, Dq, Dv, M, s);
-    case 7: return rnea_derivs_chains<7>(m, U, q, qd, qdd, Dq, Dv, M, s);
-    default: return dispatch_generic<RneaDerivsDualBody>(m, U, 3 * m.n, s, q, qd, qdd, Dq, Dv, M);
-    }
-}
-
-template <int L>
-static cudaError_t fd_derivs_chains(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, double *A, double *B,
-                                    double *C, cudaStream_t s)
-{
-    const unsigned gb = (unsigned)((U + kThreads - 1) / kThreads);
-    const StaticParams<L> *cp = static_cast<const StaticParams<L> *>(m.n == L ? m.static_params : m.chain_params);
-    const cudaError_t e = cudaFuncSetAttribute(k_fd_derivs<L>, cudaFuncAttributeMaxDynamicSharedMemorySize, link_slab_bytes(L));
-    if (e != cudaSuccess) return e;
-    for (int c = 0; c < m.n / L; ++c) {
-        const size_t off = (size_t)c * L * U;
-        k_fd_derivs<L><<<gb, kThreads, link_slab_bytes(L), s>>>(cp[c], U, q + off, qd + off, tau + off, A, B, C, m.n, c * L);
-        g_launches.fetch_add(1);
-    }
-    return cudaGetLastError();
+    cudaError_t e = cudaSuccess;
+    if (with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+            if ((e = raise_smem_limit<k_rnea_derivs<L>>(link_slab_bytes(L))) != cudaSuccess) return;
+            for (int c = 0; c < nchains; ++c) {
+                const size_t off = (size_t)c * L * U;
+                k_rnea_derivs<L><<<(unsigned)((U + kThreads - 1) / kThreads), kThreads, link_slab_bytes(L), s>>>(
+                    chains[c], U, q + off, qd + off, qdd ? qdd + off : nullptr, Dq, Dv, M, m.n, c * L);
+                g_launches.fetch_add(1);
+            }
+            e = cudaGetLastError();
+        }))
+        return e;
+    return dispatch_generic<RneaDerivsDualBody>(m, U, 3 * m.n, s, q, qd, qdd, Dq, Dv, M);
 }
 
 cudaError_t launch_fd_derivs(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, double *A, double *B,
                              double *C, cudaStream_t s)
 {
     if (U <= 0) return cudaSuccess;
-    switch (family_chain_len(m.fam)) {
-    case 3: return fd_derivs_chains<3>(m, U, q, qd, tau, A, B, C, s);
-    case 6: return fd_derivs_chains<6>(m, U, q, qd, tau, A, B, C, s);
-    case 7: return fd_derivs_chains<7>(m, U, q, qd, tau, A, B, C, s);
-    default: return dispatch_generic<FdDerivsDualBody>(m, U, 3 * m.n, s, q, qd, tau, A, B, C);
-    }
+    cudaError_t e = cudaSuccess;
+    if (with_chains(m, [&](auto L, const auto *chains, auto nchains) {
+            if ((e = raise_smem_limit<k_fd_derivs<L>>(link_slab_bytes(L))) != cudaSuccess) return;
+            for (int c = 0; c < nchains; ++c) {
+                const size_t off = (size_t)c * L * U;
+                k_fd_derivs<L><<<(unsigned)((U + kThreads - 1) / kThreads), kThreads, link_slab_bytes(L), s>>>(
+                    chains[c], U, q + off, qd + off, tau + off, A, B, C, m.n, c * L);
+                g_launches.fetch_add(1);
+            }
+            e = cudaGetLastError();
+        }))
+        return e;
+    return dispatch_generic<FdDerivsDualBody>(m, U, 3 * m.n, s, q, qd, tau, A, B, C);
 }
 
 }  // namespace mpcf

@@ -28,7 +28,6 @@
 //   d f+_i/dz = sum_{s<=3} fnext_s[i] Yv_s[i] (+ closed-form terms), fnext_s = c_s gamma_{s+1}(lambda_i h) (h/6) 2 kappa_i cv_i qd_{s+1,i}
 //               with gamma = (1 - z + z^2/2 - z^3/4, 2 - z + z^2/2, 2 - z, 1): the RK4 response of the linear fatigue rows
 //               to a forcing applied at stage s, so the rows need no per-column recursion state.
-#include <atomic>
 #include <cstdlib>
 
 #include "launch.cuh"
@@ -994,7 +993,6 @@ __global__ void __launch_bounds__(256) k_tree_fill_fatigue_cols(int n, long cnt,
 #define MPCF_TC_NJ 2
 #endif
 static constexpr int TC_NJ = MPCF_TC_NJ;  // n-tiles per warp of the tensor-core chain kernel: 1 -> 8 warps per CTA, 2 -> 4 warps
-static std::atomic<bool> g_tree_attr[64];
 
 bool tree_jvp_supported(const LaunchModel &m) { return (m.fam == FAM_GENERIC16 || m.fam == FAM_GENERIC64) && m.n <= 40; }
 
@@ -1002,6 +1000,7 @@ static size_t tree_factor_smem(int n, int npat)
 {
     return (size_t)8 * 2 * npat * sizeof(double) + ((size_t)n * n + npat + (n + 2) + (n + 1)) * sizeof(unsigned short) + (size_t)n * (n + 1) + 2 * npat + n + 16;
 }
+static constexpr int tree_factor_smem_limit(int maxn) { return maxn > 16 ? 128 * 1024 : 48 * 1024; }
 static size_t tree_chain_smem(int n, int NR, int npat)
 {
     const int NC = 3 * n + 1, XS = (NC + 15) & ~15;
@@ -1019,22 +1018,11 @@ static cudaError_t run_tree(const LaunchModel &m, int npat, long U, long cnt, co
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
     const size_t smem3 = tree_chain_smem(n, NR, npat);
-    if (dev >= 0 && dev < 64 && !g_tree_attr[dev].load(std::memory_order_acquire)) {
-        // n <= 38 fits two CTAs per SM (<= 113 KB each); n = 39, 40 run one CTA per SM
-        cudaError_t e = cudaFuncSetAttribute(k_tree_chain<40>, cudaFuncAttributeMaxDynamicSharedMemorySize, 160 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_tree_chain<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 56 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_tree_factor<40>, cudaFuncAttributeMaxDynamicSharedMemorySize, 128 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_tree_factor<16>, cudaFuncAttributeMaxDynamicSharedMemorySize, 48 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_tree_chain_tc<40, TC_NJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, 113 * 1024);
-        if (e != cudaSuccess) return e;
-        e = cudaFuncSetAttribute(k_tree_chain_tc<16, TC_NJ>, cudaFuncAttributeMaxDynamicSharedMemorySize, 56 * 1024);
-        if (e != cudaSuccess) return e;
-        g_tree_attr[dev].store(true, std::memory_order_release);
-    }
+    // n <= 38 fits two CTAs per SM (<= 113 KB each); n = 39, 40 run one CTA per SM
+    cudaError_t e;
+    if ((e = raise_smem_limit<k_tree_chain<NR>>(NR > 16 ? 160 * 1024 : 56 * 1024)) != cudaSuccess) return e;
+    if ((e = raise_smem_limit<k_tree_factor<MAXN>>(tree_factor_smem_limit(MAXN))) != cudaSuccess) return e;
+    if ((e = raise_smem_limit<k_tree_chain_tc<NR, TC_NJ>>(NR > 16 ? 113 * 1024 : 56 * 1024)) != cudaSuccess) return e;
     const int ctas_per_sm = smem3 <= 113 * 1024 ? 2 : 1;
     const long grid3_max = (long)nsm * ctas_per_sm;
     // workspace = [stage data of the chunk][fatigue-row scratch of the chain kernel's CTAs]
@@ -1096,12 +1084,8 @@ static cudaError_t run_tree_vjp(const LaunchModel &m, int npat, long U, long cnt
     int dev = 0, nsm = 148;
     cudaGetDevice(&dev);
     cudaDeviceGetAttribute(&nsm, cudaDevAttrMultiProcessorCount, dev);
-    static std::atomic<bool> attr_set[64];
-    if (dev >= 0 && dev < 64 && !attr_set[dev].load(std::memory_order_acquire)) {
-        const cudaError_t e = cudaFuncSetAttribute(k_tree_factor<MAXN>, cudaFuncAttributeMaxDynamicSharedMemorySize, MAXN > 16 ? 128 * 1024 : 48 * 1024);
-        if (e != cudaSuccess) return e;
-        attr_set[dev].store(true, std::memory_order_release);
-    }
+    const cudaError_t e = raise_smem_limit<k_tree_factor<MAXN>>(tree_factor_smem_limit(MAXN));
+    if (e != cudaSuccess) return e;
     const size_t per_unit = tree_ws_doubles_per_unit(n, npat) * sizeof(double);
     long Uc = (long)(ws_bytes / per_unit);
     Uc -= Uc % 32;

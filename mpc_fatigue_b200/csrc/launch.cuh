@@ -10,6 +10,7 @@
 #include "kernels.cuh"
 
 #include <atomic>
+#include <type_traits>
 
 #include "dyn.cuh"
 
@@ -157,5 +158,37 @@ static cudaError_t dispatch(const LaunchModel &m, long U, int grid_y, cudaStream
     return cudaGetLastError();
 }
 
+// Static families run their dedicated kernels once per serial chain: f(L, chains, nchains) with the chain length L and the chain
+// count as std::integral_constant (so forest-only kernels are instantiated for the forests alone) and chains = the parameter blocks
+// of the m.n / L chains, chain c owning joints [c L, (c + 1) L).  Returns false without calling f for run-time-topology families.
+template <class F>
+static bool with_chains(const LaunchModel &m, F &&f)
+{
+    using std::integral_constant;
+    const void *p = m.chain_params;
+    switch (m.fam) {
+    case FAM_CHAIN3: f(integral_constant<int, 3>{}, static_cast<const StaticParams<3> *>(p), integral_constant<int, 1>{}); return true;
+    case FAM_CHAIN6: f(integral_constant<int, 6>{}, static_cast<const StaticParams<6> *>(p), integral_constant<int, 1>{}); return true;
+    case FAM_FOREST12x6: f(integral_constant<int, 6>{}, static_cast<const StaticParams<6> *>(p), integral_constant<int, 2>{}); return true;
+    case FAM_CHAIN7: f(integral_constant<int, 7>{}, static_cast<const StaticParams<7> *>(p), integral_constant<int, 1>{}); return true;
+    case FAM_FOREST14x7: f(integral_constant<int, 7>{}, static_cast<const StaticParams<7> *>(p), integral_constant<int, 2>{}); return true;
+    default: return false;
+    }
+}
+
+// Raises Kernel's dynamic shared-memory limit to `bytes` once per device (function attributes are per device).  Every call site of
+// a kernel asks for the same limit, so threads racing through the first call set the same value.
+template <auto Kernel>
+static cudaError_t raise_smem_limit(int bytes)
+{
+    static std::atomic<bool> done[64];
+    int dev = 0;
+    cudaGetDevice(&dev);
+    const bool cached = dev >= 0 && dev < 64;
+    if (cached && done[dev].load(std::memory_order_acquire)) return cudaSuccess;
+    const cudaError_t e = cudaFuncSetAttribute(Kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, bytes);
+    if (e == cudaSuccess && cached) done[dev].store(true, std::memory_order_release);
+    return e;
+}
 
 }  // namespace mpcf
