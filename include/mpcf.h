@@ -196,6 +196,23 @@ int mpcf_rollout_rk4_vjp_batch(const mpcf_model *model, long B, int N, const dou
                                const double *f0, const double *tau, double dt, const double *qt, const double *qdt,
                                const double *ft, const double *gqt, const double *gqdt, const double *gft, double *gtau,
                                double *gq0, double *gqd0, double *gf0, void *workspace, size_t workspace_bytes, void *stream);
+/* Second order.  With z = (q, qd, tau, f, dt) (P = 4n + 1 components) and the adjoint lambda = (lq, lqd, lf) as for
+   mpcf_step_rk4_vjp_batch (any may be NULL = 0):
+   H[4n+1][4n+1][U] (plane r*(4n+1)+c, both triangles written) = d2(lambda^T x+)/dz dz, z = (q, qd, tau, f, dt).
+   The two mirrored planes hold the same double.  One hyper-dual sweep per pair of the 3n + 1 directions (q, qd, tau, dt); the f rows
+   and columns are closed form (zero except H[f_i][dt] = lf_i Lambda_i amp'(Lambda_i dt)).  No workspace.  dt_u: per-unit step or NULL.
+   Every kernel family; coupled models: MPCF_EINVAL.  A singular model gives NaN. */
+int mpcf_step_rk4_hess_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,
+                             const double *f, double dt, const double *dt_u, const double *lq, const double *lqd,
+                             const double *lf, double *H, void *stream);
+/* Hessian-vector product of the same H with v = (vq, vqd, vtau, vf [n][U], vdt [U]; any may be NULL = 0):
+   hq, hqd, htau, hf [n][U], hdt [U] (optional) = H v;  jq, jqd, jf [n][U] = J v (all or none), J = d(q+, qd+, f+)/dz.
+   One hyper-dual sweep per direction (3n + 1); no dense Hessian or Jacobian is formed.  Coupled models: MPCF_EINVAL. */
+int mpcf_step_rk4_hvp_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,
+                            const double *f, double dt, const double *dt_u, const double *lq, const double *lqd,
+                            const double *lf, const double *vq, const double *vqd, const double *vtau, const double *vf,
+                            const double *vdt, double *hq, double *hqd, double *htau, double *hf, double *hdt,
+                            double *jq, double *jqd, double *jf, void *stream);
 /* Forward-dynamics derivatives at (q, qd, tau): A = d qdd/d q, B = d qdd/d qd, C = M^-1 = d qdd/d tau,
    each [n*n][U] with plane index row*n + col. */
 int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,

@@ -726,6 +726,38 @@ extern "C" int mpcf_rollout_rk4_vjp_batch(const mpcf_model *model, long B, int N
     return done(e != cudaSuccess ? e : e2, "rollout_rk4_vjp_batch");
 }
 
+// ---- second order ----
+extern "C" int mpcf_step_rk4_hess_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,
+                                        const double *f, double dt, const double *dt_u, const double *lq, const double *lqd,
+                                        const double *lf, double *H, void *stream)
+{
+    PROLOGUE(q && qd && tau && f && H)
+    if (model->couple.on) return fail(MPCF_EINVAL, "the second-order entries do not support coupled fatigue");
+    if (int rc = check_forward_dynamics(model)) return rc;
+    HessArgs h;
+    h.lq = lq; h.lqd = lqd; h.lf = lf;
+    h.H = H;
+    return done(launch_step_hess(lm, U, q, qd, tau, f, dt, dt_u, h, st), "step_rk4_hess_batch");
+}
+
+extern "C" int mpcf_step_rk4_hvp_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,
+                                       const double *f, double dt, const double *dt_u, const double *lq, const double *lqd,
+                                       const double *lf, const double *vq, const double *vqd, const double *vtau, const double *vf,
+                                       const double *vdt, double *hq, double *hqd, double *htau, double *hf, double *hdt,
+                                       double *jq, double *jqd, double *jf, void *stream)
+{
+    PROLOGUE(q && qd && tau && f && hq && hqd && htau && hf)
+    if ((jq || jqd || jf) && !(jq && jqd && jf)) return fail(MPCF_EINVAL, "jq/jqd/jf must be all set or all NULL");
+    if (model->couple.on) return fail(MPCF_EINVAL, "the second-order entries do not support coupled fatigue");
+    if (int rc = check_forward_dynamics(model)) return rc;
+    HessArgs h;
+    h.lq = lq; h.lqd = lqd; h.lf = lf;
+    h.vq = vq; h.vqd = vqd; h.vtau = vtau; h.vf = vf; h.vdt = vdt;
+    h.hq = hq; h.hqd = hqd; h.htau = htau; h.hf = hf; h.hdt = hdt;
+    h.jq = jq; h.jqd = jqd; h.jf = jf;
+    return done(launch_step_hvp(lm, U, q, qd, tau, f, dt, dt_u, h, st), "step_rk4_hvp_batch");
+}
+
 extern "C" int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau, double *A,
                                     double *B, double *C, void *stream)
 {

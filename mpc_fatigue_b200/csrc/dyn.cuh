@@ -53,9 +53,50 @@ MPCF_DI void sincos_t(Dual q, Dual &s, Dual &c)
     s = Dual(sv, cv * q.d);
     c = Dual(cv, -sv * q.d);
 }
+// ---------------------------------------------------------------------------------------------
+// Hyper-dual numbers: two tangent directions a, b and the mixed second derivative ab, exact to rounding (no truncation error)
+// ---------------------------------------------------------------------------------------------
+struct HDual {
+    double v, a, b, ab;
+    MPCF_DI HDual() {}
+    MPCF_DI HDual(double v_) : v(v_), a(0.0), b(0.0), ab(0.0) {}
+    MPCF_DI HDual(double v_, double a_, double b_, double ab_) : v(v_), a(a_), b(b_), ab(ab_) {}
+};
+MPCF_DI HDual operator+(HDual x, HDual y) { return HDual(x.v + y.v, x.a + y.a, x.b + y.b, x.ab + y.ab); }
+MPCF_DI HDual operator+(HDual x, double y) { return HDual(x.v + y, x.a, x.b, x.ab); }
+MPCF_DI HDual operator+(double x, HDual y) { return HDual(x + y.v, y.a, y.b, y.ab); }
+MPCF_DI HDual operator-(HDual x, HDual y) { return HDual(x.v - y.v, x.a - y.a, x.b - y.b, x.ab - y.ab); }
+MPCF_DI HDual operator-(HDual x, double y) { return HDual(x.v - y, x.a, x.b, x.ab); }
+MPCF_DI HDual operator-(double x, HDual y) { return HDual(x - y.v, -y.a, -y.b, -y.ab); }
+MPCF_DI HDual operator-(HDual x) { return HDual(-x.v, -x.a, -x.b, -x.ab); }
+MPCF_DI HDual operator*(HDual x, HDual y)
+{
+    return HDual(x.v * y.v, fma(x.v, y.a, x.a * y.v), fma(x.v, y.b, x.b * y.v),
+                 fma(x.v, y.ab, fma(x.a, y.b, fma(x.b, y.a, x.ab * y.v))));
+}
+MPCF_DI HDual operator*(HDual x, double y) { return HDual(x.v * y, x.a * y, x.b * y, x.ab * y); }
+MPCF_DI HDual operator*(double x, HDual y) { return HDual(x * y.v, x * y.a, x * y.b, x * y.ab); }
+MPCF_DI HDual &operator+=(HDual &x, HDual y) { x = x + y; return x; }
+MPCF_DI HDual &operator-=(HDual &x, HDual y) { x = x - y; return x; }
+MPCF_DI HDual &operator+=(HDual &x, double y) { x.v += y; return x; }
+MPCF_DI HDual recip(HDual x)
+{
+    const double r = 1.0 / x.v, r2 = r * r;
+    return HDual(r, -x.a * r2, -x.b * r2, fma(-x.ab, r2, 2.0 * (x.a * x.b) * (r2 * r)));
+}
+MPCF_DI void sincos_t(HDual q, HDual &s, HDual &c)
+{
+    double sv, cv;
+    sincos(q.v, &sv, &cv);
+    const double ab = q.a * q.b;
+    s = HDual(sv, cv * q.a, cv * q.b, fma(cv, q.ab, -sv * ab));
+    c = HDual(cv, -sv * q.a, -sv * q.b, fma(-sv, q.ab, -cv * ab));
+}
+
 MPCF_DI double nan_value() { return __longlong_as_double(0x7ff8000000000000ll); }
 MPCF_DI double value_of(double a) { return a; }
 MPCF_DI double value_of(Dual a) { return a.v; }
+MPCF_DI double value_of(HDual a) { return a.v; }
 MPCF_DI double tangent_of(double) { return 0.0; }
 MPCF_DI double tangent_of(Dual a) { return a.d; }
 

@@ -158,6 +158,19 @@ cudaError_t launch_step_vjp_tree(const LaunchModel &m, int npat, long U, long cn
 // run-time models with n > 40 (kernels_jvp.cu): one dual-number sweep per input direction, contracted with lambda
 cudaError_t launch_step_vjp_dual(const LaunchModel &m, long U, long cnt, const double *q, const double *qd, const double *tau, const double *f,
                                  double dt, const double *dt_u, const VjpArgs &a, double *qn, double *qdn, double *fn, cudaStream_t s);
+// second derivatives of the RK4 step (kernels_hess.cu): hyper-dual sweeps, every family, no workspace; HessArgs holds the adjoint,
+// the HVP direction and the outputs, all [n][U] planes (vdt, hdt: [U]), NULL inputs = 0
+struct HessArgs {
+    const double *lq = nullptr, *lqd = nullptr, *lf = nullptr;
+    const double *vq = nullptr, *vqd = nullptr, *vtau = nullptr, *vf = nullptr, *vdt = nullptr;
+    double *H = nullptr;  // [4n+1][4n+1][U]
+    double *hq = nullptr, *hqd = nullptr, *htau = nullptr, *hf = nullptr, *hdt = nullptr;
+    double *jq = nullptr, *jqd = nullptr, *jf = nullptr;  // J v, all or none
+};
+cudaError_t launch_step_hess(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, const double *f,
+                             double dt, const double *dt_u, const HessArgs &h, cudaStream_t s);
+cudaError_t launch_step_hvp(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, const double *f,
+                            double dt, const double *dt_u, const HessArgs &h, cudaStream_t s);
 void jvp_profile_enable(bool on);
 int jvp_profile_read(double *ms3, long *launches);
 cudaError_t launch_fp64_probe(long iters, int blocks, double *out, cudaStream_t s);

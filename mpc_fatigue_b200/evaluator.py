@@ -241,6 +241,42 @@ class BatchEvaluator:
                 self._in(lf, n, U, "lf", True), *[p(t) for t in g], p(gdt), None, None, None, ws, ws_bytes, _stream()))
         return (*g, gdt) if want_dt else tuple(g)
 
+    def step_rk4_hess(self, q, qd, tau, f, dt, lq=None, lqd=None, lf=None):
+        """Second derivatives of `step_rk4`: H [4n+1, 4n+1, U] = d2(lambda^T x+)/dz dz with z = (q, qd, tau, f, dt) and the adjoint
+        lambda = (lq, lqd, lf) ([n, U] each; None = 0).  dt is a scalar or a per-unit tensor [U], as in `step_rk4`."""
+        U, n = self._U(q), self.n
+        P = 4 * n + 1
+        H = self._out(None, (P, P), U, "H")
+        dts, dtu = self._dt(dt, U)
+        with torch.cuda.device(self.device):
+            _capi.check(_capi.lib.mpcf_step_rk4_hess_batch(
+                self.model.handle, U, self._in(q, n, U, "q"), self._in(qd, n, U, "qd"), self._in(tau, n, U, "tau"),
+                self._in(f, n, U, "f"), dts, dtu, self._in(lq, n, U, "lq", True), self._in(lqd, n, U, "lqd", True),
+                self._in(lf, n, U, "lf", True), C.c_void_p(H.data_ptr()), _stream()))
+        return H
+
+    def step_rk4_hvp(self, q, qd, tau, f, dt, lam, v, want_dt=False, want_jv=False):
+        """Hessian-vector product of `step_rk4_hess` without forming H: lam = (lq, lqd, lf), v = (vq, vqd, vtau, vf, vdt) ([n, U] each,
+        vdt [U]; None entries = 0).  Returns (hq, hqd, htau, hf) = H v, then hdt [U] with want_dt=True, then (jq, jqd, jf) = J v of the
+        step Jacobian J = d(q+, qd+, f+)/dz with want_jv=True."""
+        U, n = self._U(q), self.n
+        lq, lqd, lf = lam
+        vq, vqd, vtau, vf, vdt = v
+        h = [self._out(None, n, U, nm) for nm in ("hq", "hqd", "htau", "hf")]
+        hdt = self._out(None, 1, U, "hdt").view(U) if want_dt else None
+        jv = [self._out(None, n, U, nm) for nm in ("jq", "jqd", "jf")] if want_jv else [None] * 3
+        dts, dtu = self._dt(dt, U)
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        with torch.cuda.device(self.device):
+            _capi.check(_capi.lib.mpcf_step_rk4_hvp_batch(
+                self.model.handle, U, self._in(q, n, U, "q"), self._in(qd, n, U, "qd"), self._in(tau, n, U, "tau"),
+                self._in(f, n, U, "f"), dts, dtu, self._in(lq, n, U, "lq", True), self._in(lqd, n, U, "lqd", True),
+                self._in(lf, n, U, "lf", True), self._in(vq, n, U, "vq", True), self._in(vqd, n, U, "vqd", True),
+                self._in(vtau, n, U, "vtau", True), self._in(vf, n, U, "vf", True),
+                None if vdt is None else self._in(vdt.view(1, -1), 1, U, "vdt"), *[p(t) for t in h], p(hdt), *[p(t) for t in jv],
+                _stream()))
+        return (*h, *((hdt,) if want_dt else ()), *((tuple(jv),) if want_jv else ()))
+
     def rollout_rk4_vjp(self, q0, qd0, f0, tau, N: int, dt: float, traj, gqt=None, gqdt=None, gft=None):
         """Adjoint of `rollout_rk4`: `traj` = the (qt, qdt, ft) it returned for the same inputs, gqt/gqdt/gft [n, N*B] = dL/d(trajectory)
         (None = 0).  Returns (gtau [n, N*B], gq0, gqd0, gf0 [n, B]) = dL/d(tau, x0).  One step VJP per node in reverse order; nothing
