@@ -455,7 +455,11 @@ extern "C" int mpcf_node_eval_ref_batch(const mpcf_model *model, int nee, const 
     for (int e = 0; e < nee; ++e)
         if (int rc = frame_arg(model, ee_frames[e], ee.f[e])) return rc;
     ZohArg zoh{};
-    for (int i = 0; i < model->h.n; ++i) zoh.a[i] = std::exp(-model->h.fat[4 * i] * h);
+    for (int i = 0; i < model->h.n; ++i) {
+        const double lam = model->h.fat[4 * i], kap = model->h.fat[4 * i + 1];
+        zoh.a[i] = std::exp(-lam * h);
+        zoh.g[i] = lam == 0.0 ? 0.0 : -std::expm1(-lam * h) * (kap / lam);
+    }
     return done(launch_node_eval(lm, ee, wsign, U, q, qd, qdd, W, T, h, zoh, tau, qnext, Tnext, false, st), "node_eval_ref_batch");
 }
 

@@ -41,6 +41,7 @@ struct EeArgs {
 };
 struct ZohArg {
     double a[MPCF_MAX_DOF];  // exp(-lambda_i h), computed once on the host
+    double g[MPCF_MAX_DOF];  // gain -expm1(-lambda_i h) kappa_i / lambda_i (lambda_i != 0): 1 - a_i cancels as lambda_i h -> 0
 };
 
 enum Family { FAM_GENERIC16 = 0, FAM_GENERIC64, FAM_CHAIN3, FAM_CHAIN6, FAM_FOREST12x6, FAM_CHAIN7, FAM_FOREST14x7, FAM_COUNT };

@@ -144,7 +144,7 @@ struct NodeEvalBody {
                 const double P = m.fat(i, 2) * t[i] * t[i] + m.fat(i, 3) * b[i] * b[i];
                 const double Ti = T[i * U + u];
                 const double lam = m.fat(i, 0);
-                Tnext[i * U + u] = (lam == 0.0) ? Ti + h * m.fat(i, 1) * P : zoh.a[i] * Ti + (1.0 - zoh.a[i]) * (m.fat(i, 1) / lam) * P;
+                Tnext[i * U + u] = (lam == 0.0) ? Ti + h * m.fat(i, 1) * P : zoh.a[i] * Ti + zoh.g[i] * P;
             }
         }
     }
@@ -621,7 +621,7 @@ __global__ void __launch_bounds__(kThreads, 3) node_eval_chain_kernel(const __gr
             const double Pl = m.fat(i, 2) * t[i] * t[i] + m.fat(i, 3) * b[i] * b[i];
             const double Ti = T[i * U + u];
             const double lam = m.fat(i, 0), za = zoh.a[c0 + i];
-            Tnext[i * U + u] = (lam == 0.0) ? Ti + h * m.fat(i, 1) * Pl : za * Ti + (1.0 - za) * (m.fat(i, 1) / lam) * Pl;
+            Tnext[i * U + u] = (lam == 0.0) ? Ti + h * m.fat(i, 1) * Pl : za * Ti + zoh.g[c0 + i] * Pl;
         }
     }
 }

@@ -155,7 +155,8 @@ struct RowsBody {
                 const double Pl = m.fat(i, 2) * t * t + m.fat(i, 3) * qdi * qdi;
                 const double Ti = T[(long)i * U + u];
                 const double za = exp(-lam * a.h);
-                const double gain = lam == 0.0 ? a.h * kap : (1.0 - za) * (kap / lam);
+                // expm1: 1 - za cancels as lam h -> 0 (lam h = 1e-12: ~1e-4 relative), and the gain must meet h kap there
+                const double gain = lam == 0.0 ? a.h * kap : -expm1(-lam * a.h) * (kap / lam);
                 const double Tn = za * Ti + gain * Pl;
                 const double Tnext = k + 1 < a.N ? T[(long)i * U + u + a.B] : (T_last ? T_last[(long)i * a.B + b] : Tn);
                 Tdef = Tn - Tnext;

@@ -394,14 +394,16 @@ static inline SC SUF(fatigue_rhs)(const mpcfo_model *m, int i, SC f, SC tau, SC 
     const double *c = m->fat + 4 * i;
     return -c[0] * f + c[1] * (c[2] * tau * tau + c[3] * qd * qd);
 }
-/* exact zero-order-hold map over h (the reference's T_next line, mpc_principal.py:301) */
+/* exact zero-order-hold map over h (the reference's T_next line, mpc_principal.py:301).  The gain (1 - a) kappa / lambda is
+ * formed as -expm1(-lambda h) kappa / lambda: 1 - exp(-lambda h) loses all but a few digits as lambda h -> 0 (lambda h = 1e-12:
+ * ~1e-4 relative), while expm1 keeps the gain continuous into the lambda = 0 branch. */
 static inline SC SUF(fatigue_zoh)(const mpcfo_model *m, int i, SC f, SC tau, SC qd, SC h)
 {
     const double *c = m->fat + 4 * i;
     SC P = c[2] * tau * tau + c[3] * qd * qd;
     if (c[0] == 0.0) return f + h * c[1] * P;
     SC a = EXP(-c[0] * h);
-    return a * f + (1.0 - a) * (c[1] / c[0]) * P;
+    return a * f + (-EXPM1(-c[0] * h)) * (c[1] / c[0]) * P;
 }
 
 /* xdot = (qd, ABA(q,qd,tau), fatigue_rhs) */

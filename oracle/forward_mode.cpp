@@ -52,6 +52,7 @@ inline bool operator==(const MDual &a, double b) { return a.v == b; }
 inline MDual md_sin(const MDual &a) { MDual r; const double c = std::cos(a.v); r.v = std::sin(a.v); LOOP3 r.d[k] = c * a.d[k]; return r; }
 inline MDual md_cos(const MDual &a) { MDual r; const double s = -std::sin(a.v); r.v = std::cos(a.v); LOOP3 r.d[k] = s * a.d[k]; return r; }
 inline MDual md_exp(const MDual &a) { MDual r; r.v = std::exp(a.v); LOOP3 r.d[k] = r.v * a.d[k]; return r; }
+inline MDual md_expm1(const MDual &a) { MDual r; const double e = std::exp(a.v); r.v = std::expm1(a.v); LOOP3 r.d[k] = e * a.d[k]; return r; }
 inline void seed(MDual &a, int lane) { reinterpret_cast<double *>(a.d)[lane] = 1.0; }
 inline double tangent(const MDual &a, int lane) { return reinterpret_cast<const double *>(a.d)[lane]; }
 
@@ -60,12 +61,14 @@ inline double tangent(const MDual &a, int lane) { return reinterpret_cast<const 
 #define SIN md_sin
 #define COS md_cos
 #define EXP md_exp
+#define EXPM1 md_expm1
 #include "core.inc.h"
 #undef SC
 #undef SUF
 #undef SIN
 #undef COS
 #undef EXP
+#undef EXPM1
 
 }  // namespace
 

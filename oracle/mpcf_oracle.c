@@ -20,12 +20,22 @@
 #define SIN sin
 #define COS cos
 #define EXP exp
+#define EXPM1 expm1
 #include "core.inc.h"
 #undef SC
 #undef SUF
 #undef SIN
 #undef COS
 #undef EXP
+#undef EXPM1
+
+/* exp(z) - 1 for complex z = x + i y without the cancellation of cexp(z) - 1 at small |z|:
+ * e^x cos y - 1 = expm1(x) cos y - 2 sin^2(y / 2) */
+static inline double complex cexpm1(double complex z)
+{
+    const double x = creal(z), y = cimag(z), s = sin(0.5 * y);
+    return CMPLX(expm1(x) * cos(y) - 2.0 * s * s, exp(x) * sin(y));
+}
 
 /* complex instantiation (complex-step derivatives) */
 #define SC double complex
@@ -33,12 +43,14 @@
 #define SIN csin
 #define COS ccos
 #define EXP cexp
+#define EXPM1 cexpm1
 #include "core.inc.h"
 #undef SC
 #undef SUF
 #undef SIN
 #undef COS
 #undef EXP
+#undef EXPM1
 
 static int g_threads = 0;
 

@@ -52,18 +52,21 @@ inline bool operator==(const HD &x, double y) { return x.v == y; }
 inline HD hd_sin(const HD &x) { const double s = std::sin(x.v), c = std::cos(x.v); return HD(s, c * x.a, c * x.b, c * x.ab - s * x.a * x.b); }
 inline HD hd_cos(const HD &x) { const double s = std::sin(x.v), c = std::cos(x.v); return HD(c, -s * x.a, -s * x.b, -s * x.ab - c * x.a * x.b); }
 inline HD hd_exp(const HD &x) { const double e = std::exp(x.v); return HD(e, e * x.a, e * x.b, e * (x.ab + x.a * x.b)); }
+inline HD hd_expm1(const HD &x) { const double e = std::exp(x.v); return HD(std::expm1(x.v), e * x.a, e * x.b, e * (x.ab + x.a * x.b)); }
 
 #define SC HD
 #define SUF(x) x##_h
 #define SIN hd_sin
 #define COS hd_cos
 #define EXP hd_exp
+#define EXPM1 hd_expm1
 #include "core.inc.h"
 #undef SC
 #undef SUF
 #undef SIN
 #undef COS
 #undef EXP
+#undef EXPM1
 
 inline double at(const double *p, long i) { return p ? p[i] : 0.0; }
 
