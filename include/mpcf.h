@@ -213,6 +213,30 @@ int mpcf_step_rk4_hvp_batch(const mpcf_model *model, long U, const double *q, co
                             const double *lf, const double *vq, const double *vqd, const double *vtau, const double *vf,
                             const double *vdt, double *hq, double *hqd, double *htau, double *hf, double *hdt,
                             double *jq, double *jqd, double *jf, void *stream);
+/* Riccati solve of the multiple-shooting linear-quadratic subproblem of B scenarios over N nodes (units u = k*B + b), with the state
+   x = (q, qd, f) (3n components, the row order of the step Jacobian) and the input u = tau (n components):
+     minimise  sum_{k<N} 1/2 z_k^T W_k z_k + g_k^T z_k + 1/2 dx_N^T W_N dx_N + g_N^T dx_N,   z_k = (dx_k, du_k)
+     s.t.      dx_0 = dx0,   dx_{k+1} = A_k dx_k + B_k du_k + d_k.
+   A_k = the q, qd and f columns of jac[3n][4n+1][N*B] (mpcf_step_rk4_jvp_batch: columns 0..2n and 3n..4n), B_k = its tau columns
+   2n..3n; the dt column is not read.  W_k = the (x, tau) rows and columns of H[4n+1][4n+1][N*B] in the layout of
+   mpcf_step_rk4_hess_batch (its output can be passed as is; the upper triangle in the order (tau, q, qd, f) is read, so H must be
+   symmetric) + diag(wx [3n][N*B], wu [n][N*B]) (e.g. interior-point barrier diagonals).  W_N = HN [3n*3n][B] (plane r*3n + c,
+   symmetric) + diag(wN [3n][B]).  g_k = (gx [3n][N*B], gu [n][N*B]), g_N [3n][B], the defect d_k = x+_k - x_{k+1} [3n][N*B] (the sign
+   of mpcf_cost_residual_batch) and dx0 [3n][B]: every one of H, wx, wu, gx, gu, d, HN, wN, gN, dx0 may be NULL (= 0).
+   Outputs, node-major: dx [3n][(N+1)*B], du [n][N*B] and, when lam is not NULL, the costates lam [3n][(N+1)*B]:
+     lambda_N = W_N dx_N + g_N,   lambda_k = Q_k dx_k + S_k^T du_k + gx_k + A_k^T lambda_{k+1}
+   (W_k = [Q_k S_k^T; S_k R_k]), the multipliers of the dynamics in
+     L = obj - lambda_0^T (dx_0 - dx0) - sum_k lambda_{k+1}^T (dx_{k+1} - A_k dx_k - B_k du_k - d_k),
+   i.e. the adjoint that the next mpcf_step_rk4_hess_batch call takes.  No regularisation: a scenario whose R + B^T P B is not
+   positive definite at some node gets NaN in all its outputs; the other scenarios are unaffected.  Models with n <= 16 (every
+   family but generic64, coupled models included: only jac is read); n > 16 is MPCF_ELIMIT.  B = 0 launches nothing.
+   Workspace (one per stream): mpcf_riccati_workspace_bytes() gives the size for B scenarios (bounded: scenarios run in chunks);
+   it must be 128-byte aligned and hold at least one chunk of one CTA's scenarios (a smaller size gives more, smaller chunks);
+   NULL takes it from the stream-ordered pool.  One warp per scenario, the nodes serially. */
+size_t mpcf_riccati_workspace_bytes(const mpcf_model *model, long B, int N);
+int mpcf_riccati_batch(const mpcf_model *model, long B, int N, const double *jac, const double *H, const double *wx, const double *wu,
+                       const double *gx, const double *gu, const double *d, const double *HN, const double *wN, const double *gN,
+                       const double *dx0, double *dx, double *du, double *lam, void *workspace, size_t workspace_bytes, void *stream);
 /* Forward-dynamics derivatives at (q, qd, tau): A = d qdd/d q, B = d qdd/d qd, C = M^-1 = d qdd/d tau,
    each [n*n][U] with plane index row*n + col. */
 int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,

@@ -78,6 +78,8 @@ _sig = {
                                    + [C.c_void_p, C.c_size_t, C.c_void_p]),
     "mpcf_step_rk4_hess_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, C.c_double, _dp] + [_dp] * 4 + [C.c_void_p]),
     "mpcf_step_rk4_hvp_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, C.c_double, _dp] + [_dp] * 16 + [C.c_void_p]),
+    "mpcf_riccati_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_long, C.c_int]),
+    "mpcf_riccati_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 14 + [C.c_void_p, C.c_size_t, C.c_void_p]),
     "mpcf_fd_derivs_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, _dp, _dp, C.c_void_p]),
     "mpcf_rnea_derivs_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, _dp, _dp, C.c_void_p]),
     "mpcf_cost_residual_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 7 + [C.c_double] * 7 + [_dp, C.c_void_p]),

@@ -762,6 +762,62 @@ extern "C" int mpcf_step_rk4_hvp_batch(const mpcf_model *model, long U, const do
     return done(launch_step_hvp(lm, U, q, qd, tau, f, dt, dt_u, h, st), "step_rk4_hvp_batch");
 }
 
+// ---- Riccati solve of the LQ subproblem ----
+// Scenarios run in chunks; the workspace holds the chunk's feedback gains, riccati_ws_bytes_per_scenario(n, N) per scenario.  A
+// chunk is a multiple of the scenarios of one CTA and, for the default size, at most 4 GiB of gains (more only when one CTA's
+// scenarios need more), so the request is bounded however large B is.
+static const size_t kRiccatiChunkBytes = (size_t)1 << 32;
+static const int kRiccatiMaxDof = 16;
+extern "C" size_t mpcf_riccati_workspace_bytes(const mpcf_model *model, long B, int N)
+{
+    if (!model || B <= 0 || N <= 0 || model->h.n > kRiccatiMaxDof) return 0;
+    const int n = model->h.n, w = riccati_warps_per_cta(n);
+    const size_t per = riccati_ws_bytes_per_scenario(n, N);
+    long chunk = (long)(kRiccatiChunkBytes / per) / w * w;
+    if (chunk < w) chunk = w;
+    long scen = (B + w - 1) / w * w;
+    if (scen > chunk) scen = chunk;
+    return (size_t)scen * per;
+}
+
+extern "C" int mpcf_riccati_batch(const mpcf_model *model, long B, int N, const double *jac, const double *H, const double *wx,
+                                  const double *wu, const double *gx, const double *gu, const double *d, const double *HN,
+                                  const double *wN, const double *gN, const double *dx0, double *dx, double *du, double *lam,
+                                  void *workspace, size_t workspace_bytes, void *stream)
+{
+    if (!model) return fail(MPCF_EINVAL, "null model");
+    if (B < 0 || N <= 0) return fail(MPCF_EINVAL, "bad B / N");
+    if (!(jac && dx && du)) return fail(MPCF_EINVAL, "null array argument");
+    const int n = model->h.n;
+    if (n > kRiccatiMaxDof) return fail(MPCF_ELIMIT, "the Riccati solve supports n <= 16 (one warp per scenario); this model has n = " + std::to_string(n));
+    if (B == 0) return MPCF_OK;
+    const int w = riccati_warps_per_cta(n);
+    const size_t per = riccati_ws_bytes_per_scenario(n, N);
+    cudaStream_t st = static_cast<cudaStream_t>(stream);
+    double *ws = static_cast<double *>(workspace);
+    size_t bytes = workspace_bytes;
+    bool owned = false;
+    if (workspace) {
+        if (reinterpret_cast<uintptr_t>(workspace) % 128) return fail(MPCF_EINVAL, "workspace must be 128-byte aligned");
+        if (workspace_bytes < (size_t)w * per) return fail(MPCF_EINVAL, "workspace too small: see mpcf_riccati_workspace_bytes");
+    } else {
+        bytes = mpcf_riccati_workspace_bytes(model, B, N);
+        const cudaError_t e = cudaMallocAsync(reinterpret_cast<void **>(&ws), bytes, st);
+        if (e != cudaSuccess) return cuda_fail(e, "cudaMallocAsync(riccati workspace)");
+        owned = true;
+    }
+    const long chunk = (long)(bytes / per) / w * w;
+    RiccatiArgs a;
+    a.n = n; a.N = N; a.B = B;
+    a.jac = jac; a.H = H; a.wx = wx; a.wu = wu; a.gx = gx; a.gu = gu; a.d = d;
+    a.HN = HN; a.wN = wN; a.gN = gN; a.dx0 = dx0;
+    a.dx = dx; a.du = du; a.lam = lam; a.ws = ws;
+    cudaError_t e = cudaSuccess;
+    for (long b0 = 0; b0 < B && e == cudaSuccess; b0 += chunk) e = launch_riccati(a, b0, B - b0 < chunk ? B - b0 : chunk, st);
+    const cudaError_t e2 = owned ? cudaFreeAsync(ws, st) : cudaSuccess;
+    return done(e != cudaSuccess ? e : e2, "riccati_batch");
+}
+
 extern "C" int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau, double *A,
                                     double *B, double *C, void *stream)
 {

@@ -172,6 +172,19 @@ cudaError_t launch_step_hess(const LaunchModel &m, long U, const double *q, cons
                              double dt, const double *dt_u, const HessArgs &h, cudaStream_t s);
 cudaError_t launch_step_hvp(const LaunchModel &m, long U, const double *q, const double *qd, const double *tau, const double *f,
                             double dt, const double *dt_u, const HessArgs &h, cudaStream_t s);
+// Riccati solve of the multiple-shooting LQ subproblem (kernels_riccati.cu): one warp per scenario, n <= 16.  Every pointer is a
+// device plane set as in include/mpcf.h (mpcf_riccati_batch); NULL optional inputs are zero.  ws: K_k and k_k of the chunk's
+// scenarios, riccati_ws_bytes_per_scenario(n, N) each, scenario b0 + i at offset i.
+struct RiccatiArgs {
+    int n = 0, N = 0;
+    long B = 0;
+    const double *jac = nullptr, *H = nullptr, *wx = nullptr, *wu = nullptr, *gx = nullptr, *gu = nullptr, *d = nullptr;
+    const double *HN = nullptr, *wN = nullptr, *gN = nullptr, *dx0 = nullptr;
+    double *dx = nullptr, *du = nullptr, *lam = nullptr, *ws = nullptr;
+};
+int riccati_warps_per_cta(int n);  // scenarios per CTA: chunk sizes are multiples of it
+size_t riccati_ws_bytes_per_scenario(int n, int N);
+cudaError_t launch_riccati(const RiccatiArgs &a, long b0, long cnt, cudaStream_t s);
 void jvp_profile_enable(bool on);
 int jvp_profile_read(double *ms3, long *launches);
 cudaError_t launch_fp64_probe(long iters, int blocks, double *out, cudaStream_t s);

@@ -297,6 +297,37 @@ class BatchEvaluator:
                 C.c_void_p(gtau.data_ptr()), *[C.c_void_p(t.data_ptr()) for t in g0], ws, ws_bytes, _stream()))
         return (gtau, *g0)
 
+    def riccati(self, jac, B: int, N: int, *, H=None, wx=None, wu=None, gx=None, gu=None, d=None, HN=None, wN=None, gN=None, dx0=None,
+                want_lam=False):
+        """Riccati solve of the multiple-shooting LQ subproblem of B scenarios over N nodes (include/mpcf.h: mpcf_riccati_batch).
+        jac [3n, 4n+1, N*B] is the step Jacobian (`step_rk4_jvp`); H [4n+1, 4n+1, N*B] the step Hessian (`step_rk4_hess`);
+        wx [3n, N*B], wu [n, N*B] diagonal weights; gx [3n, N*B], gu [n, N*B] gradients; d [3n, N*B] = x+_k - x_{k+1};
+        HN [3n*3n, B], wN, gN, dx0 [3n, B]; None = 0.  Returns (dx [3n, (N+1)*B], du [n, N*B]) and, with want_lam=True, the
+        costates lam [3n, (N+1)*B] (the adjoint of the next `step_rk4_hess` call).  Node-major units u = k*B + b throughout."""
+        n, B, N = self.n, int(B), int(N)
+        U, nx, P = N * B, 3 * n, 4 * n + 1
+        if not (jac.is_cuda and jac.dtype == torch.float64 and jac.is_contiguous() and tuple(jac.shape) == (nx, P, U)
+                and jac.device == self.device):
+            raise ValueError("jac must be a contiguous CUDA float64 tensor of shape %s" % ((nx, P, U),))
+        if H is not None and not (H.is_cuda and H.dtype == torch.float64 and H.is_contiguous() and tuple(H.shape) == (P, P, U)
+                                  and H.device == self.device):
+            raise ValueError("H must be a contiguous CUDA float64 tensor of shape %s" % ((P, P, U),))
+        dx, du = self._out(None, nx, (N + 1) * B, "dx"), self._out(None, n, U, "du")
+        lam = self._out(None, nx, (N + 1) * B, "lam") if want_lam else None
+        need = int(_capi.lib.mpcf_riccati_workspace_bytes(self.model.handle, B, N))
+        ws = getattr(self, "_rws", None)
+        if need and (ws is None or ws.numel() * 8 < need):
+            self._rws = ws = torch.empty(need // 8, dtype=torch.float64, device=self.device)
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        with torch.cuda.device(self.device):
+            _capi.check(_capi.lib.mpcf_riccati_batch(
+                self.model.handle, B, N, p(jac), p(H), self._in(wx, nx, U, "wx", True), self._in(wu, n, U, "wu", True),
+                self._in(gx, nx, U, "gx", True), self._in(gu, n, U, "gu", True), self._in(d, nx, U, "d", True),
+                self._in(HN, nx * nx, B, "HN", True), self._in(wN, nx, B, "wN", True), self._in(gN, nx, B, "gN", True),
+                self._in(dx0, nx, B, "dx0", True), p(dx), p(du), p(lam), p(ws) if need else None, ws.numel() * 8 if need else 0,
+                _stream()))
+        return (dx, du, lam) if want_lam else (dx, du)
+
     def step_rk4_jvp_range(self, q, qd, tau, f, dt: float, u0: int, cnt: int, out, jac):
         """Units [u0, u0 + cnt) of a larger batch: states go to columns [u0, u0 + cnt) of the full-size `out` = (qn, qdn, fn),
         the Jacobian to the chunk-local buffer jac[3n, 4n+1, cap] (cap >= cnt) — one Jacobian buffer is reused over the
