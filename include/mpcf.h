@@ -256,7 +256,8 @@ int mpcf_rnea_derivs_batch(const mpcf_model *model, long U, const double *q, con
                     bound_k = max(tau0 exp(-alpha k dt), tau_floor)
                                                         (python/Pilz_6_DOF/force_optimization_pilz_6DOF.py:136-148)
      resid[2][b]  = max_k max_i (f+_ki - f_max)+        fatigue / temperature bound
-   out[4][B] = (cost, resid0, resid1, resid2): written directly into the caller's (all-gather send) buffer. */
+   out[4][B] = (cost, resid0, resid1, resid2): written directly into the caller's (all-gather send) buffer.
+   A row is NaN when any entry it reads is NaN (a failed step's NaN is never dropped from a maximum). */
 int mpcf_cost_residual_batch(const mpcf_model *model, long B, int N, const double *q, const double *qd,
                              const double *f, const double *tau, const double *qn, const double *qdn,
                              const double *fn, double dt, double w_qd, double w_tau, double tau0,
@@ -268,7 +269,8 @@ int mpcf_cost_residual_batch(const mpcf_model *model, long B, int N, const doubl
    F3 joint switch-off |tau_i| <= C_i after the first third for the joints selected by S (Centauro_dynamics.py:327-348).
      resid[1][b] = max_k max_i max(lb_ki - tau_ki, tau_ki - ub_ki, 0)
    out has row stride ld_out >= B (0 = B): a scenario chunk can write its columns of a larger [4][B_total] send buffer.
-   2 n N doubles must fit 200 KB of shared memory (MPCF_ELIMIT otherwise). */
+   2 n N doubles must fit 200 KB of shared memory (MPCF_ELIMIT otherwise).  As above, a row is NaN when any entry it reads
+   (the bound table's included) is NaN. */
 int mpcf_cost_residual_table_batch(const mpcf_model *model, long B, int N, const double *q, const double *qd,
                                    const double *f, const double *tau, const double *qn, const double *qdn,
                                    const double *fn, double w_qd, double w_tau, const double *bound_table,
@@ -331,7 +333,8 @@ int mpcf_memcpy2d_async(void *dst, size_t dpitch, const void *src, size_t spitch
 
 /* dst[k][u] = src[plane_map[k]][u] for k < nplanes, u < U (src planes have stride ld_src >= U; plane_map is a DEVICE int32
    array; src and dst 16-byte aligned): packs the planes a host consumer wants (states + the structurally non-zero Jacobian
-   planes) into one contiguous device buffer, so that a scenario chunk goes back to the host in ONE copy. */
+   planes) into one contiguous device buffer, so that a scenario chunk goes back to the host in ONE copy.  Every plane_map
+   entry must be a valid plane index of src: the entry cannot check a device array without a synchronising copy. */
 int mpcf_gather_planes(const double *src, long ld_src, const int *plane_map, int nplanes, long U, double *dst,
                        void *stream);
 

@@ -214,6 +214,21 @@ struct NodeEvalJvpBody {
 // per-scenario cost / residual reduction: thread b walks the N nodes of scenario b (u = k*B + b,
 // coalesced across b) and writes (cost, defect, torque-bound, fatigue-bound) into out[4][B]
 // ---------------------------------------------------------------------------------------------
+// Running maximum of a residual row from +0.0 that keeps NaN: value() is NaN when any operand was NaN, otherwise the largest
+// operand, and +0.0 when none exceeds 0 (-0.0 included).  fmax(m, NaN) returns m (IEEE maxNum), so a NaN is remembered in a
+// predicate beside the fmax chain; the + 0.0 turns a -0.0 that fmax may keep into +0.0.  A select-based maximum gives the same
+// values but made ptxas interleave the loads with the selects: 2.3x the table kernel's time (B200, 1000 W power limit).
+struct RowMax {
+    double m = 0.0;
+    bool nan = false;
+    MPCF_DI void add(double x)
+    {
+        m = fmax(m, x);
+        nan |= isnan(x);
+    }
+    MPCF_DI double value() const { return nan ? NAN : m + 0.0; }
+};
+
 __global__ void __launch_bounds__(256) cost_residual_kernel(int n, long B, int N, const double *q, const double *qd, const double *f,
                                                           const double *tau, const double *qn, const double *qdn, const double *fn,
                                                           CostArgs c, double *out)
@@ -221,7 +236,8 @@ __global__ void __launch_bounds__(256) cost_residual_kernel(int n, long B, int N
     const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     const long U = B * N;
-    double cost = 0.0, r0 = 0.0, r1 = 0.0, r2 = 0.0;
+    double cost = 0.0;
+    RowMax r0, r1, r2;
     for (int k = 0; k < N; ++k) {
         const long u = (long)k * B + b;
         const double bound = fmax(c.tau0 * exp(-c.alpha * k * c.dt), c.tau_floor);
@@ -229,20 +245,20 @@ __global__ void __launch_bounds__(256) cost_residual_kernel(int n, long B, int N
             const long o = (long)i * U + u;
             const double v = qd[o], t = tau[o];
             cost += c.w_qd * v * v + c.w_tau * t * t;
-            r1 = fmax(r1, fabs(t) - bound);
-            r2 = fmax(r2, fn[o] - c.f_max);
+            r1.add(fabs(t) - bound);
+            r2.add(fn[o] - c.f_max);
             if (k + 1 < N) {
                 const long o1 = o + B;
-                r0 = fmax(r0, fabs(qn[o] - q[o1]));
-                r0 = fmax(r0, fabs(qdn[o] - qd[o1]));
-                r0 = fmax(r0, fabs(fn[o] - f[o1]));
+                r0.add(fabs(qn[o] - q[o1]));
+                r0.add(fabs(qdn[o] - qd[o1]));
+                r0.add(fabs(fn[o] - f[o1]));
             }
         }
     }
     out[b] = cost;
-    out[B + b] = r0;
-    out[2 * B + b] = r1;
-    out[3 * B + b] = r2;
+    out[B + b] = r0.value();
+    out[2 * B + b] = r1.value();
+    out[3 * B + b] = r2.value();
 }
 
 // Same reduction with a per-node, per-joint bound table [N][n][2] = (lb, ub) instead of the closed-form F0 schedule, which
@@ -250,7 +266,10 @@ __global__ void __launch_bounds__(256) cost_residual_kernel(int n, long B, int N
 // ub = b_k), F2 stepwise over segments of the horizon (both_robots_torque_limited_2_pilz.py:129-147, Box_Pilz_6DOF2.py:303-433)
 // and F3 joint switch-off (Centauro_dynamics.py:327-348: |tau_i| <= C_i after the first third for the joints selected by S).
 // The table (2 n N doubles) is staged in shared memory once per block.  resid[1] = max violation max(lb - tau, tau - ub, 0).
-__global__ void __launch_bounds__(256) cost_residual_table_kernel(int n, long B, int N, const double *q, const double *qd, const double *f,
+// The minimum of 3 blocks per SM keeps ptxas from sinking the loads towards their uses (one thread per scenario leaves few
+// warps per SM, so the loads each thread has in flight set the bandwidth): at 65,536 x 100 (pilz6), 0.35 ms with it and 0.55 ms
+// without on a B200 at a 1000 W power limit.
+__global__ void __launch_bounds__(256, 3) cost_residual_table_kernel(int n, long B, int N, const double *q, const double *qd, const double *f,
                                                                 const double *tau, const double *qn, const double *qdn,
                                                                 const double *fn, double w_qd, double w_tau, double f_max,
                                                                 const double *__restrict__ table, double *out, long ld_out)
@@ -261,27 +280,29 @@ __global__ void __launch_bounds__(256) cost_residual_table_kernel(int n, long B,
     const long b = (long)blockIdx.x * blockDim.x + threadIdx.x;
     if (b >= B) return;
     const long U = B * N;
-    double cost = 0.0, r0 = 0.0, r1 = 0.0, r2 = 0.0;
+    double cost = 0.0;
+    RowMax r0, r1, r2;
     for (int k = 0; k < N; ++k) {
         const long u = (long)k * B + b;
         for (int i = 0; i < n; ++i) {
             const long o = (long)i * U + u;
             const double v = qd[o], t = tau[o];
             cost += w_qd * v * v + w_tau * t * t;
-            r1 = fmax(r1, fmax(tb[2 * (k * n + i)] - t, t - tb[2 * (k * n + i) + 1]));
-            r2 = fmax(r2, fn[o] - f_max);
+            r1.add(tb[2 * (k * n + i)] - t);
+            r1.add(t - tb[2 * (k * n + i) + 1]);
+            r2.add(fn[o] - f_max);
             if (k + 1 < N) {
                 const long o1 = o + B;
-                r0 = fmax(r0, fabs(qn[o] - q[o1]));
-                r0 = fmax(r0, fabs(qdn[o] - qd[o1]));
-                r0 = fmax(r0, fabs(fn[o] - f[o1]));
+                r0.add(fabs(qn[o] - q[o1]));
+                r0.add(fabs(qdn[o] - qd[o1]));
+                r0.add(fabs(fn[o] - f[o1]));
             }
         }
     }
     out[b] = cost;
-    out[ld_out + b] = r0;
-    out[2 * ld_out + b] = r1;
-    out[3 * ld_out + b] = r2;
+    out[ld_out + b] = r0.value();
+    out[2 * ld_out + b] = r1.value();
+    out[3 * ld_out + b] = r2.value();
 }
 
 cudaError_t launch_cost_residual_table(int n, long B, int N, const double *q, const double *qd, const double *f, const double *tau,

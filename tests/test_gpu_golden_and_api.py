@@ -159,50 +159,104 @@ def test_singular_forward_dynamics_is_an_error_not_a_nan(torch_mod):
     assert tuple(ev.rnea(z[:, :0].contiguous(), z[:, :0].contiguous()).shape) == (6, 0)  # empty batch
 
 
-def test_host_pipeline_matches_direct_calls(torch_mod):
-    torch = torch_mod
+# Host pipeline cases beyond the three of test_host_pipeline_matches_direct_calls:
+# (B, N, chunk_units, skip_structural_zeros, outputs, with_jacobian).  B = 1009, N = 5, chunk_units = 505: Bc = 101 scenarios and
+# 505 units per chunk, odd, so the plane gather takes its scalar path and the 2-D copies odd pitches; chunk_units < N: one
+# scenario per chunk (Bc = 1); "reused": one pipeline object run again with the same (B, N), then another (B, N), then the first.
+PIPELINE_CASES = {
+    "1009x5": (1009, 5, 505, False, "all", True),
+    "1009x5_skip": (1009, 5, 505, True, "all", True),
+    "1009x5_reduced": (1009, 5, 505, False, "reduced", True),
+    "1009x5_skip_reduced": (1009, 5, 505, True, "reduced", True),
+    "no_jacobian": (300, 6, 6 * 64, False, "all", False),
+    "no_jacobian_reduced": (300, 6, 6 * 64, True, "reduced", False),
+    "one_scenario_per_chunk": (9, 7, 3, False, "all", True),
+    "one_scenario_per_chunk_skip": (9, 7, 3, True, "all", True),
+    "reused": (1009, 5, 505, False, "all", True),
+    "reused_skip": (1009, 5, 505, True, "all", True),
+}
+
+
+def _pipeline_check(torch, pipe, m, B, N, seed):
+    """One run of `pipe` against direct step_rk4_jvp (step_rk4 without Jacobian) plus cost_residual calls on the device:
+    every returned chunk and the reduced rows bit for bit, and the byte counts."""
     from mpc_fatigue_b200.evaluator import BatchEvaluator
-    from mpc_fatigue_b200.model import Model, data_urdf
-    from mpc_fatigue_b200.pipeline import HostStepPipeline
     from mpc_fatigue_b200.synth import synth_batch
-    m = Model.from_urdf(data_urdf("pilz6"), armature=1e-2)
     ev = BatchEvaluator(m)
-    B, N, dt = 700, 7, 0.02
+    n, dt = m.n, 0.02
     lim = {k: m.export(k) for k in ("q_lo", "q_hi", "v_max", "tau_max")}
-    q, qd, tau, f = synth_batch(lim, 0, B, N, device="cuda")
-    qn, qdn, fn, jac = ev.step_rk4_jvp(q, qd, tau, f, dt)
+    q, qd, tau, f = synth_batch(lim, 0, B, N, seed=seed, device="cuda")
+    if pipe.with_jacobian:
+        qn, qdn, fn, jac = ev.step_rk4_jvp(q, qd, tau, f, dt)
+        full = torch.cat([qn, qdn, fn, jac.reshape(-1, B * N)])
+    else:
+        qn, qdn, fn = ev.step_rk4(q, qd, tau, f, dt)
+        full = torch.cat([qn, qdn, fn])
     red = ev.cost_residual(B, N, q, qd, f, tau, qn, qdn, fn, dt)
-    pipe = HostStepPipeline(m, "cuda:0", chunk_units=N * 256)  # 3 ragged chunks
+    full = full.reshape(-1, N, B).cpu()
     host = [t.cpu().pin_memory() for t in (q, qd, tau, f)]
     got = {}
-
-    def consume(view, b0, b1):
-        got[(b0, b1)] = view.clone()
-    stats = pipe.run(*host, dt, B, N, consume=consume)
-    assert stats["chunks"] == 3 and sorted(got) == [(0, 256), (256, 512), (512, 700)]
-    assert stats["h2d_bytes"] == 4 * 6 * B * N * 8 and stats["d2h_bytes"] == (18 + 450) * B * N * 8 + 4 * B * 8
-    full = torch.cat([qn, qdn, fn, jac.reshape(450, B * N)]).reshape(468, N, B).cpu()
-    for (b0, b1), v in got.items():
-        assert torch.equal(v, full[:, :, b0:b1])
+    stats = pipe.run(*host, dt, B, N, consume=lambda v, b0, b1: got.__setitem__((b0, b1), v.clone()))
+    Bc = max(1, min(B, pipe.chunk_units // N))
+    bounds = [(b0, min(B, b0 + Bc)) for b0 in range(0, B, Bc)]
+    hrows = len(pipe.plane_map)
+    assert stats["chunks"] == len(bounds) and stats["h2d_bytes"] == 4 * n * B * N * 8
     assert torch.equal(pipe.h_red, red.cpu())
-    # structural zeros stay on the device: 348 of 450 Jacobian planes travel, mapped by plane_map
-    pz = HostStepPipeline(m, "cuda:0", chunk_units=N * 256, skip_structural_zeros=True)
-    assert len(pz.plane_map) == 18 + 348 and not pz.identity_map and pipe.identity_map  # packed on the device, one D2H per chunk
-    gz = {}
-    st2 = pz.run(*host, dt, B, N, consume=lambda v, b0, b1: gz.__setitem__((b0, b1), v.clone()))
+    if pipe.outputs == "reduced":
+        assert not got and stats["d2h_bytes"] == 4 * B * 8
+        return full, stats
+    assert sorted(got) == bounds and stats["d2h_bytes"] == hrows * B * N * 8 + 4 * B * 8
+    sel = torch.tensor(pipe.plane_map)
+    for (b0, b1), v in got.items():
+        assert torch.equal(v, full[sel][:, :, b0:b1]), (b0, b1)
+    return full, stats
+
+
+def _pipeline_case(torch, m, B, N, chunk, skip, outputs, with_jac):
+    """a pipeline of these options against the direct calls, plus what its plane selection implies"""
+    from mpc_fatigue_b200.pipeline import HostStepPipeline
+    pipe = HostStepPipeline(m, "cuda:0", chunk_units=chunk, with_jacobian=with_jac, skip_structural_zeros=skip, outputs=outputs)
+    full, stats = _pipeline_check(torch, pipe, m, B, N, seed=B + N)
+    if skip and with_jac:  # structural zeros stay on the device: 348 of 450 Jacobian planes travel, packed on the device
+        assert len(pipe.plane_map) == 18 + 348 and not pipe.identity_map
+        if outputs == "all":
+            dropped = sorted(set(range(468)) - set(pipe.plane_map))
+            assert len(dropped) == 102 and float(full[torch.tensor(dropped)].abs().max()) == 0.0
+    if not with_jac:
+        assert pipe.plane_map == list(range(18)) and pipe.identity_map
+    return pipe, stats
+
+
+def test_host_pipeline_matches_direct_calls(torch_mod):
+    torch = torch_mod
+    from mpc_fatigue_b200.model import Model, data_urdf
+    from mpc_fatigue_b200.pipeline import HostStepPipeline
+    m = Model.from_urdf(data_urdf("pilz6"), armature=1e-2)
+    B, N = 700, 7
+    pipe, stats = _pipeline_case(torch, m, B, N, N * 256, False, "all", True)
+    assert stats["chunks"] == 3 and pipe.identity_map  # 3 ragged chunks
+    assert stats["d2h_bytes"] == (18 + 450) * B * N * 8 + 4 * B * 8
+    _, st2 = _pipeline_case(torch, m, B, N, N * 256, True, "all", True)
     assert st2["d2h_bytes"] == (18 + 348) * B * N * 8 + 4 * B * 8
-    sel = torch.tensor(pz.plane_map)
-    for (b0, b1), v in gz.items():
-        assert torch.equal(v, full[sel][:, :, b0:b1])
-    dropped = sorted(set(range(468)) - set(pz.plane_map))
-    assert len(dropped) == 102 and float(full[torch.tensor(dropped)].abs().max()) == 0.0
     # outputs="reduced": same computation, only the per-scenario rows come back
-    pr = HostStepPipeline(m, "cuda:0", chunk_units=N * 256, outputs="reduced")
-    st3 = pr.run(*host, dt, B, N)
+    _, st3 = _pipeline_case(torch, m, B, N, N * 256, False, "reduced", True)
     assert st3["d2h_bytes"] == 4 * B * 8 and st3["h2d_bytes"] == stats["h2d_bytes"]
-    assert torch.equal(pr.h_red, red.cpu())
     with pytest.raises(ValueError):
         HostStepPipeline(m, "cuda:0", outputs="none")
+
+
+@pytest.mark.parametrize("case", list(PIPELINE_CASES))
+def test_host_pipeline_edge_cases_match_direct_calls(torch_mod, case):
+    torch = torch_mod
+    from mpc_fatigue_b200.model import Model, data_urdf
+    B, N, chunk, skip, outputs, with_jac = PIPELINE_CASES[case]
+    m = Model.from_urdf(data_urdf("pilz6"), armature=1e-2)
+    pipe, stats = _pipeline_case(torch, m, B, N, chunk, skip, outputs, with_jac)
+    if case.startswith("reused"):
+        for B2, N2, seed in ((B, N, 2), (257, 3, 3), (B, N, 4)):
+            _pipeline_check(torch, pipe, m, B2, N2, seed)
+    if case.startswith("one_scenario_per_chunk"):
+        assert stats["chunks"] == B
 
 
 def test_full_size_properties(torch_mod):
