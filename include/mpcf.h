@@ -237,6 +237,48 @@ size_t mpcf_riccati_workspace_bytes(const mpcf_model *model, long B, int N);
 int mpcf_riccati_batch(const mpcf_model *model, long B, int N, const double *jac, const double *H, const double *wx, const double *wu,
                        const double *gx, const double *gu, const double *d, const double *HN, const double *wN, const double *gN,
                        const double *dx0, double *dx, double *du, double *lam, void *workspace, size_t workspace_bytes, void *stream);
+/* The same backward pass with the feedback gains as an output and no workspace: K [n][3n+1][N*B], plane t*(3n+1) + j, unit k*B + b,
+   holds row t of [K_k | k_k] (columns j < 3n: K_k, column 3n: the feedforward k_k), so that du_k = K_k dx_k + k_k in the solve.
+   Inputs as for mpcf_riccati_batch.  dx and du are optional, both or neither: when both are NULL only the backward pass runs (all
+   that iLQR needs); lam needs dx.  When dx is given, dx, du and lam are bit-identical to mpcf_riccati_batch's.  A scenario whose
+   R + B^T P B is not positive definite at some node gets NaN in all its K planes (and in dx, du, lam); the others are unaffected.
+   n > 16 is MPCF_ELIMIT. */
+int mpcf_riccati_gains_batch(const mpcf_model *model, long B, int N, const double *jac, const double *H, const double *wx,
+                             const double *wu, const double *gx, const double *gu, const double *d, const double *HN, const double *wN,
+                             const double *gN, const double *dx0, double *K, double *dx, double *du, double *lam, void *stream);
+
+/* iLQR on the device (DESIGN.md §4g).  State x = (q, qd, f) [3n], input u = tau [n]; units node-major u = k*B + b; trajectories
+   x / xbar [3n][(N+1)*B] (nodes 0..N), torques [n][N*B], x0 [3n][B].  The tracking cost of one scenario, with every pointer of
+   mpcf_track_cost a DEVICE array or NULL (= 0, or absent for bound_table):
+     J = sum_{k<N} [ 1/2 sum_i wx_i (x_ki - x_ref_ki)^2 + 1/2 sum_j wu_j (tau_kj - tau_ref_kj)^2
+                     + 1/2 rho_tau sum_j ((lb_kj - tau_kj)+^2 + (tau_kj - ub_kj)+^2) + 1/2 rho_f sum_j (f_kj - f_max)+^2 ]
+         + 1/2 sum_i wN_i (x_Ni - x_ref_Ni)^2 + 1/2 rho_f sum_j (f_Nj - f_max)+^2
+   x_ref [3n][(N+1)*B], tau_ref [n][N*B], wx, wN [3n], wu [n], bound_table [N][n][2] = (lb, ub) (the table of
+   mpcf_cost_residual_table_batch).  A NaN in any state, torque or reference makes J NaN.  Under the feedback law
+     tau_k = taubar_k + alpha k_k + K_k (x_k - xbar_k),   x_{k+1} = RK4(x_k, tau_k, dt),   x_0 = x0,
+   with K the gains of mpcf_riccati_gains_batch.  alpha == 0 reads neither K nor xbar: tau_k = taubar_k exactly, so a rejected step
+   reproduces the trajectory it started from bit for bit, even where the gains are NaN.  Every kernel family; coupled models:
+   MPCF_EINVAL. */
+typedef struct {
+    const double *x_ref, *tau_ref, *wx, *wu, *wN, *bound_table;
+    double rho_tau, f_max, rho_f;
+} mpcf_track_cost;
+/* Line-search pass: J [na][B] = the cost of the closed-loop rollout for each of the na step lengths alphas[0..na) (host array,
+   1 <= na <= 16, finite, >= 0), one thread per (step length, scenario).  K == NULL: the open-loop cost of taubar for every entry
+   (xbar may then be NULL).  No trajectory is stored.  J of step length a has the same bits as mpcf_feedback_rollout_batch's J with
+   alpha = a. */
+int mpcf_ilqr_costs_batch(const mpcf_model *model, const mpcf_track_cost *cost, long B, int N, const double *x0, const double *xbar,
+                          const double *taubar, const double *K, const double *alphas, int na, double dt, double *J, void *stream);
+/* Accept pass: the closed-loop rollout with the per-scenario step length alpha [B] (DEVICE); K == NULL (alpha and xbar may then be
+   NULL) rolls taubar out open loop from x0, bit-identical to mpcf_rollout_rk4_batch.  Writes x [3n][(N+1)*B] (node 0 = x0),
+   tau [n][N*B] and J [B].  Optionally (all or none) the Riccati inputs of the cost at the new trajectory, to pass straight to
+   mpcf_riccati_gains_batch: the gradient gx [3n][N*B], gu [n][N*B], gN [3n][B] and the Gauss-Newton curvature wx_out [3n][N*B] =
+   wx + rho_f [f > f_max] on the f rows, wu_out [n][N*B] = wu + rho_tau [tau outside (lb, ub)], wN_out [3n][B]. */
+int mpcf_feedback_rollout_batch(const mpcf_model *model, const mpcf_track_cost *cost, long B, int N, const double *x0,
+                                const double *xbar, const double *taubar, const double *K, const double *alpha, double dt, double *x,
+                                double *tau, double *J, double *gx, double *gu, double *wx_out, double *wu_out, double *gN,
+                                double *wN_out, void *stream);
+
 /* Forward-dynamics derivatives at (q, qd, tau): A = d qdd/d q, B = d qdd/d qd, C = M^-1 = d qdd/d tau,
    each [n*n][U] with plane index row*n + col. */
 int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau,

@@ -37,6 +37,11 @@ class RowsOpts(C.Structure):
                 ("p_ref", C.c_double * 3), ("w_box", C.c_double), ("w_qd", C.c_double), ("w_F", C.c_double), ("h", C.c_double)]
 
 
+class TrackCost(C.Structure):
+    _fields_ = [("x_ref", C.c_void_p), ("tau_ref", C.c_void_p), ("wx", C.c_void_p), ("wu", C.c_void_p), ("wN", C.c_void_p),
+                ("bound_table", C.c_void_p), ("rho_tau", C.c_double), ("f_max", C.c_double), ("rho_f", C.c_double)]
+
+
 _dp = C.c_void_p  # device pointers travel as integers
 _sig = {
     "mpcf_opts_default": (None, [C.POINTER(Opts)]),
@@ -80,6 +85,11 @@ _sig = {
     "mpcf_step_rk4_hvp_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, C.c_double, _dp] + [_dp] * 16 + [C.c_void_p]),
     "mpcf_riccati_workspace_bytes": (C.c_size_t, [C.c_void_p, C.c_long, C.c_int]),
     "mpcf_riccati_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 14 + [C.c_void_p, C.c_size_t, C.c_void_p]),
+    "mpcf_riccati_gains_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 15 + [C.c_void_p]),
+    "mpcf_ilqr_costs_batch": (C.c_int, [C.c_void_p, C.POINTER(TrackCost), C.c_long, C.c_int, _dp, _dp, _dp, _dp, C.POINTER(C.c_double),
+                                        C.c_int, C.c_double, _dp, C.c_void_p]),
+    "mpcf_feedback_rollout_batch": (C.c_int, [C.c_void_p, C.POINTER(TrackCost), C.c_long, C.c_int, _dp, _dp, _dp, _dp, _dp, C.c_double]
+                                    + [_dp] * 9 + [C.c_void_p]),
     "mpcf_fd_derivs_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, _dp, _dp, C.c_void_p]),
     "mpcf_rnea_derivs_batch": (C.c_int, [C.c_void_p, C.c_long, _dp, _dp, _dp, _dp, _dp, _dp, C.c_void_p]),
     "mpcf_cost_residual_batch": (C.c_int, [C.c_void_p, C.c_long, C.c_int] + [_dp] * 7 + [C.c_double] * 7 + [_dp, C.c_void_p]),

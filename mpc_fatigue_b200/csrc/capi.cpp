@@ -818,6 +818,80 @@ extern "C" int mpcf_riccati_batch(const mpcf_model *model, long B, int N, const 
     return done(e != cudaSuccess ? e : e2, "riccati_batch");
 }
 
+extern "C" int mpcf_riccati_gains_batch(const mpcf_model *model, long B, int N, const double *jac, const double *H, const double *wx,
+                                        const double *wu, const double *gx, const double *gu, const double *d, const double *HN,
+                                        const double *wN, const double *gN, const double *dx0, double *K, double *dx, double *du,
+                                        double *lam, void *stream)
+{
+    if (!model) return fail(MPCF_EINVAL, "null model");
+    if (B < 0 || N <= 0) return fail(MPCF_EINVAL, "bad B / N");
+    if (!(jac && K)) return fail(MPCF_EINVAL, "null array argument");
+    if (!dx != !du) return fail(MPCF_EINVAL, "dx and du are both given or both NULL");
+    if (lam && !dx) return fail(MPCF_EINVAL, "lam needs dx and du");
+    const int n = model->h.n;
+    if (n > kRiccatiMaxDof) return fail(MPCF_ELIMIT, "the Riccati solve supports n <= 16 (one warp per scenario); this model has n = " + std::to_string(n));
+    if (B == 0) return MPCF_OK;
+    RiccatiArgs a;
+    a.n = n; a.N = N; a.B = B;
+    a.jac = jac; a.H = H; a.wx = wx; a.wu = wu; a.gx = gx; a.gu = gu; a.d = d;
+    a.HN = HN; a.wN = wN; a.gN = gN; a.dx0 = dx0;
+    a.dx = dx; a.du = du; a.lam = lam; a.ws = K;
+    return done(launch_riccati_gains(a, static_cast<cudaStream_t>(stream)), "riccati_gains_batch");
+}
+
+// ---- iLQR rollouts ----
+static int ilqr_prologue(const mpcf_model *model, const mpcf_track_cost *cost, long B, int N, const double *x0, const double *taubar,
+                         double *J, IlqrArgs &a)
+{
+    if (!model) return fail(MPCF_EINVAL, "null model");
+    if (!cost) return fail(MPCF_EINVAL, "null cost");
+    if (B < 0 || N <= 0) return fail(MPCF_EINVAL, "bad B / N");
+    if (B > 0 && !(x0 && taubar && J)) return fail(MPCF_EINVAL, "null array argument");
+    if (model->couple.on) return fail(MPCF_EINVAL, "the iLQR rollouts do not support coupled fatigue");
+    if (int rc = check_forward_dynamics(model)) return rc;
+    a.N = N; a.B = B;
+    a.cost.x_ref = cost->x_ref; a.cost.tau_ref = cost->tau_ref; a.cost.wx = cost->wx; a.cost.wu = cost->wu; a.cost.wN = cost->wN;
+    a.cost.bound = cost->bound_table;
+    a.cost.rho_tau = cost->rho_tau; a.cost.f_max = cost->f_max; a.cost.rho_f = cost->rho_f;
+    a.x0 = x0; a.taubar = taubar; a.J = J;
+    return MPCF_OK;
+}
+
+extern "C" int mpcf_ilqr_costs_batch(const mpcf_model *model, const mpcf_track_cost *cost, long B, int N, const double *x0,
+                                     const double *xbar, const double *taubar, const double *K, const double *alphas, int na, double dt,
+                                     double *J, void *stream)
+{
+    IlqrArgs a;
+    if (int rc = ilqr_prologue(model, cost, B, N, x0, taubar, J, a)) return rc;
+    if (!alphas || na < 1 || na > kIlqrMaxAlphas) return fail(MPCF_EINVAL, "na must be in [1, 16] with a host array of step lengths");
+    for (int i = 0; i < na; ++i)
+        if (!(std::isfinite(alphas[i]) && alphas[i] >= 0.0)) return fail(MPCF_EINVAL, "step lengths must be finite and >= 0");
+    if (K && B > 0 && !xbar) return fail(MPCF_EINVAL, "the feedback law needs xbar");
+    LaunchModel lm;
+    if (int rc = get_launch_model(model, lm)) return rc;
+    a.dt = dt; a.xbar = xbar; a.K = K; a.na = na;
+    for (int i = 0; i < na; ++i) a.alphas[i] = alphas[i];
+    return done(launch_ilqr_costs(lm, a, static_cast<cudaStream_t>(stream)), "ilqr_costs_batch");
+}
+
+extern "C" int mpcf_feedback_rollout_batch(const mpcf_model *model, const mpcf_track_cost *cost, long B, int N, const double *x0,
+                                           const double *xbar, const double *taubar, const double *K, const double *alpha, double dt,
+                                           double *x, double *tau, double *J, double *gx, double *gu, double *wx_out, double *wu_out,
+                                           double *gN, double *wN_out, void *stream)
+{
+    IlqrArgs a;
+    if (int rc = ilqr_prologue(model, cost, B, N, x0, taubar, J, a)) return rc;
+    if (B > 0 && !(x && tau)) return fail(MPCF_EINVAL, "null array argument");
+    if (K && B > 0 && !(xbar && alpha)) return fail(MPCF_EINVAL, "the feedback law needs xbar and alpha");
+    const int nd = !!gx + !!gu + !!wx_out + !!wu_out + !!gN + !!wN_out;
+    if (nd != 0 && nd != 6) return fail(MPCF_EINVAL, "the derivative outputs gx, gu, wx_out, wu_out, gN, wN_out are all given or all NULL");
+    LaunchModel lm;
+    if (int rc = get_launch_model(model, lm)) return rc;
+    a.dt = dt; a.xbar = xbar; a.K = K; a.alpha = alpha; a.x = x; a.tau = tau;
+    a.gx = gx; a.gu = gu; a.wxo = wx_out; a.wuo = wu_out; a.gN = gN; a.wNo = wN_out;
+    return done(launch_feedback_rollout(lm, a, static_cast<cudaStream_t>(stream)), "feedback_rollout_batch");
+}
+
 extern "C" int mpcf_fd_derivs_batch(const mpcf_model *model, long U, const double *q, const double *qd, const double *tau, double *A,
                                     double *B, double *C, void *stream)
 {

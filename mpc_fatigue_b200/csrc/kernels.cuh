@@ -185,6 +185,30 @@ struct RiccatiArgs {
 int riccati_warps_per_cta(int n);  // scenarios per CTA: chunk sizes are multiples of it
 size_t riccati_ws_bytes_per_scenario(int n, int N);
 cudaError_t launch_riccati(const RiccatiArgs &a, long b0, long cnt, cudaStream_t s);
+// mpcf_riccati_gains_batch: every scenario in one launch, the gains written to the planes a.ws = K [n][3n+1][N B] (dx, du, lam optional)
+cudaError_t launch_riccati_gains(const RiccatiArgs &a, cudaStream_t s);
+// iLQR rollouts (kernels_ilqr.cu): the tracking cost of include/mpcf.h (mpcf_track_cost; NULL pointers = 0 or absent) and the
+// arguments of both passes.  Every [.][N B] plane has units k B + b, x / xbar are [3n][(N+1) B], x0 [3n][B].
+constexpr int kIlqrMaxAlphas = 16;
+struct TrackCost {
+    const double *x_ref = nullptr, *tau_ref = nullptr, *wx = nullptr, *wu = nullptr, *wN = nullptr, *bound = nullptr;
+    double rho_tau = 0.0, f_max = 0.0, rho_f = 0.0;
+};
+struct IlqrArgs {
+    int N = 0;
+    long B = 0;
+    double dt = 0.0;
+    TrackCost cost;
+    const double *x0 = nullptr, *xbar = nullptr, *taubar = nullptr, *K = nullptr;  // K [n][3n+1][N B] or NULL (open loop)
+    double *J = nullptr;                                                            // [na][B] (costs) or [B] (accept)
+    int na = 0;                                                                     // costs pass: the step lengths
+    double alphas[kIlqrMaxAlphas] = {};
+    const double *alpha = nullptr;                                                  // accept pass: alpha [B]
+    double *x = nullptr, *tau = nullptr;
+    double *gx = nullptr, *gu = nullptr, *wxo = nullptr, *wuo = nullptr, *gN = nullptr, *wNo = nullptr;  // all or none
+};
+cudaError_t launch_ilqr_costs(const LaunchModel &m, const IlqrArgs &a, cudaStream_t s);
+cudaError_t launch_feedback_rollout(const LaunchModel &m, const IlqrArgs &a, cudaStream_t s);
 void jvp_profile_enable(bool on);
 int jvp_profile_read(double *ms3, long *launches);
 cudaError_t launch_fp64_probe(long iters, int blocks, double *out, cudaStream_t s);

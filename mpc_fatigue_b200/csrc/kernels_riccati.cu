@@ -47,7 +47,10 @@ MPCF_DI double w_entry(const RiccatiArgs &a, int i, int c, long u, long U)
 
 }  // namespace
 
-template <int MAXN, int WPC>
+// PLANES = false: mpcf_riccati_batch, the gains go to the chunk-local workspace and the forward pass always runs.  PLANES = true:
+// mpcf_riccati_gains_batch, the gains go to the caller's planes a.ws = K [n][3n+1][N B] (plane t (3n+1) + j, unit k B + b; b0 = 0) and
+// the forward pass and the costates run only when a.dx is given.
+template <int MAXN, int WPC, bool PLANES = false>
 __global__ void __launch_bounds__(32 * WPC) k_riccati(const RiccatiArgs a, long b0, long cnt)
 {
     constexpr int MX = 3 * MAXN;
@@ -132,8 +135,9 @@ __global__ void __launch_bounds__(32 * WPC) k_riccati(const RiccatiArgs a, long 
             }
             __syncwarp();
         }
-        // K = -L^-T Y_x and k = -L^-T y_u by back substitution (lane = column), into the workspace; the new (P, p)
-        double *K = a.ws + ((bl * N + k) * (long)nu) * ldk;
+        // K = -L^-T Y_x and k = -L^-T y_u by back substitution (lane = column), into the workspace or the planes; the new (P, p)
+        double *K = a.ws + (PLANES ? u : ((bl * N + k) * (long)nu) * ldk);
+        const long sk = PLANES ? U : 1;  // stride of the gain entries
         for (int c = nu + lane; c <= nc; c += 32) {
             double kc[MAXN];
 #pragma unroll
@@ -144,7 +148,7 @@ __global__ void __launch_bounds__(32 * WPC) k_riccati(const RiccatiArgs a, long 
                     for (int q = t + 1; q < MAXN; ++q)
                         if (q < nu) s = fma(Z[t * ld + q], kc[q], s);
                     kc[t] = -s / Z[t * ld + t];
-                    K[t * ldk + (c - nu)] = kc[t];
+                    K[(t * ldk + (c - nu)) * sk] = kc[t];
                 }
             }
             if (c < nc)
@@ -158,6 +162,11 @@ __global__ void __launch_bounds__(32 * WPC) k_riccati(const RiccatiArgs a, long 
     // ---- forward pass ----
     const double qnan = __longlong_as_double(0x7ff8000000000000LL);
     if (bad) {  // Quu not positive definite at some node: the whole scenario is NaN
+        if constexpr (PLANES) {
+            for (int idx = lane; idx < nu * ldk; idx += 32)
+                for (int k = 0; k < N; ++k) a.ws[(long)idx * U + (long)k * B + b] = qnan;
+            if (!a.dx) return;
+        }
         for (int r = lane; r < nx; r += 32)
             for (int k = 0; k <= N; ++k) {
                 a.dx[(long)r * (N + 1) * B + (long)k * B + b] = qnan;
@@ -167,6 +176,7 @@ __global__ void __launch_bounds__(32 * WPC) k_riccati(const RiccatiArgs a, long 
             for (int k = 0; k < N; ++k) a.du[(long)t * U + (long)k * B + b] = qnan;
         return;
     }
+    if (PLANES && !a.dx) return;
     const long UX = (long)(N + 1) * B;
     for (int r = lane; r < nx; r += 32) {
         const double x0 = ld_or0(a.dx0, (long)r * B + b);
@@ -175,8 +185,8 @@ __global__ void __launch_bounds__(32 * WPC) k_riccati(const RiccatiArgs a, long 
     }
     for (int k = 0; k < N; ++k) {
         const long u = (long)k * B + b;
-        const double *K = a.ws + ((bl * N + k) * (long)nu) * ldk;
-        for (int idx = lane; idx < nu * ldk; idx += 32) Z[idx] = K[idx];
+        const double *K = a.ws + (PLANES ? u : ((bl * N + k) * (long)nu) * ldk);
+        for (int idx = lane; idx < nu * ldk; idx += 32) Z[idx] = K[idx * (PLANES ? U : 1)];
         load_ab(a, u, U, AB, lane);
         for (int r = lane; r < nx; r += 32) dd[r] = ld_or0(a.d, (long)r * U + u);
         __syncwarp();
@@ -246,13 +256,13 @@ int riccati_warps_per_cta(int n) { return n <= 8 ? 4 : 2; }
 
 size_t riccati_ws_bytes_per_scenario(int n, int N) { return (size_t)N * n * (3 * n + 1) * sizeof(double); }
 
-template <int MAXN, int WPC>
+template <int MAXN, int WPC, bool PLANES = false>
 static cudaError_t launch_bucket(const RiccatiArgs &a, long b0, long cnt, cudaStream_t s)
 {
     // the limit is set once per device, for the largest n of the bucket
-    if (cudaError_t e = raise_smem_limit<k_riccati<MAXN, WPC>>(WPC * riccati_warp_doubles(MAXN) * (int)sizeof(double))) return e;
+    if (cudaError_t e = raise_smem_limit<k_riccati<MAXN, WPC, PLANES>>(WPC * riccati_warp_doubles(MAXN) * (int)sizeof(double))) return e;
     const unsigned grid = (unsigned)((cnt + WPC - 1) / WPC);
-    k_riccati<MAXN, WPC><<<grid, 32 * WPC, (size_t)WPC * riccati_warp_doubles(a.n) * sizeof(double), s>>>(a, b0, cnt);
+    k_riccati<MAXN, WPC, PLANES><<<grid, 32 * WPC, (size_t)WPC * riccati_warp_doubles(a.n) * sizeof(double), s>>>(a, b0, cnt);
     g_launches.fetch_add(1);
     return cudaGetLastError();
 }
@@ -263,6 +273,14 @@ cudaError_t launch_riccati(const RiccatiArgs &a, long b0, long cnt, cudaStream_t
     if (a.n <= 4) return launch_bucket<4, 4>(a, b0, cnt, s);
     if (a.n <= 8) return launch_bucket<8, 4>(a, b0, cnt, s);
     return launch_bucket<16, 2>(a, b0, cnt, s);
+}
+
+cudaError_t launch_riccati_gains(const RiccatiArgs &a, cudaStream_t s)
+{
+    if (a.B <= 0) return cudaSuccess;
+    if (a.n <= 4) return launch_bucket<4, 4, true>(a, 0, a.B, s);
+    if (a.n <= 8) return launch_bucket<8, 4, true>(a, 0, a.B, s);
+    return launch_bucket<16, 2, true>(a, 0, a.B, s);
 }
 
 }  // namespace mpcf

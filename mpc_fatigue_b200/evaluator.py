@@ -328,6 +328,96 @@ class BatchEvaluator:
                 _stream()))
         return (dx, du, lam) if want_lam else (dx, du)
 
+    def riccati_gains(self, jac, B: int, N: int, *, H=None, wx=None, wu=None, gx=None, gu=None, d=None, HN=None, wN=None, gN=None,
+                      dx0=None, want_solution=False, want_lam=False):
+        """The backward pass of `riccati` with the feedback gains as output (include/mpcf.h: mpcf_riccati_gains_batch): returns
+        K [n, 3n+1, N*B] (plane t*(3n+1) + j: row t of [K_k | k_k], unit k*B + b), and with want_solution=True also (dx, du) and,
+        with want_lam=True, lam, bit-identical to `riccati`.  Arguments as for `riccati`; no workspace."""
+        n, B, N = self.n, int(B), int(N)
+        U, nx, P = N * B, 3 * n, 4 * n + 1
+        if not (jac.is_cuda and jac.dtype == torch.float64 and jac.is_contiguous() and tuple(jac.shape) == (nx, P, U)
+                and jac.device == self.device):
+            raise ValueError("jac must be a contiguous CUDA float64 tensor of shape %s" % ((nx, P, U),))
+        if H is not None and not (H.is_cuda and H.dtype == torch.float64 and H.is_contiguous() and tuple(H.shape) == (P, P, U)
+                                  and H.device == self.device):
+            raise ValueError("H must be a contiguous CUDA float64 tensor of shape %s" % ((P, P, U),))
+        K = self._out(None, (n, nx + 1), U, "K")
+        sol = want_solution or want_lam
+        dx = self._out(None, nx, (N + 1) * B, "dx") if sol else None
+        du = self._out(None, n, U, "du") if sol else None
+        lam = self._out(None, nx, (N + 1) * B, "lam") if want_lam else None
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        with torch.cuda.device(self.device):
+            _capi.check(_capi.lib.mpcf_riccati_gains_batch(
+                self.model.handle, B, N, p(jac), p(H), self._in(wx, nx, U, "wx", True), self._in(wu, n, U, "wu", True),
+                self._in(gx, nx, U, "gx", True), self._in(gu, n, U, "gu", True), self._in(d, nx, U, "d", True),
+                self._in(HN, nx * nx, B, "HN", True), self._in(wN, nx, B, "wN", True), self._in(gN, nx, B, "gN", True),
+                self._in(dx0, nx, B, "dx0", True), p(K), p(dx), p(du), p(lam), _stream()))
+        if not sol:
+            return K
+        return (K, dx, du, lam) if want_lam else (K, dx, du)
+
+    def _gains(self, K, U: int) -> None:
+        n = self.n
+        if K is not None and not (K.is_cuda and K.dtype == torch.float64 and K.is_contiguous() and tuple(K.shape) == (n, 3 * n + 1, U)
+                                  and K.device == self.device):
+            raise ValueError("K must be a contiguous CUDA float64 tensor of shape %s" % ((n, 3 * n + 1, U),))
+
+    def _track_cost(self, cost, B: int, N: int):
+        """ctypes mpcf_track_cost of a tracking cost (mpc_fatigue_b200.ilqr.TrackingCost or any object with its fields)."""
+        n = self.n
+        vec = lambda t, rows, nm: None if t is None else self._in(t.view(rows, 1) if t.dim() == 1 else t, rows, 1, nm)
+        tb = cost.bound_table
+        if tb is not None and not (tb.is_cuda and tb.dtype == torch.float64 and tb.is_contiguous() and tuple(tb.shape) == (N, n, 2)
+                                   and tb.device == self.device):
+            raise ValueError("bound_table must be a contiguous CUDA float64 tensor of shape (N, n, 2)")
+        return _capi.TrackCost(self._in(cost.x_ref, 3 * n, (N + 1) * B, "x_ref", True), self._in(cost.tau_ref, n, N * B, "tau_ref", True),
+                               vec(cost.wx, 3 * n, "wx"), vec(cost.wu, n, "wu"), vec(cost.wN, 3 * n, "wN"),
+                               None if tb is None else C.c_void_p(tb.data_ptr()), float(cost.rho_tau), float(cost.f_max), float(cost.rho_f))
+
+    def ilqr_costs(self, cost, x0, xbar, taubar, K, alphas, N: int, dt: float):
+        """Line-search pass (include/mpcf.h: mpcf_ilqr_costs_batch): J [na, B] of the closed-loop rollouts
+        tau_k = taubar_k + alpha k_k + K_k (x_k - xbar_k) from x0 [3n, B] for the step lengths `alphas` (1 to 16 floats); K = None
+        gives the open-loop cost of taubar (xbar may be None).  xbar [3n, (N+1)*B], taubar [n, N*B], K [n, 3n+1, N*B]."""
+        n, N = self.n, int(N)
+        B = x0.shape[1] if x0.dim() == 2 else -1
+        U = N * B
+        al = [float(a) for a in alphas]
+        if not 1 <= len(al) <= 16:
+            raise ValueError("between 1 and 16 step lengths")
+        c = self._track_cost(cost, B, N)
+        self._gains(K, U)
+        J = self._out(None, len(al), B, "J")
+        with torch.cuda.device(self.device):
+            _capi.check(_capi.lib.mpcf_ilqr_costs_batch(
+                self.model.handle, C.byref(c), B, N, self._in(x0, 3 * n, B, "x0"), self._in(xbar, 3 * n, (N + 1) * B, "xbar", K is None),
+                self._in(taubar, n, U, "taubar"), None if K is None else C.c_void_p(K.data_ptr()), (C.c_double * len(al))(*al), len(al),
+                float(dt), C.c_void_p(J.data_ptr()), _stream()))
+        return J
+
+    def feedback_rollout(self, cost, x0, taubar, N: int, dt: float, *, xbar=None, K=None, alpha=None, derivatives=False):
+        """Accept pass (include/mpcf.h: mpcf_feedback_rollout_batch): the closed-loop rollout with per-scenario step lengths
+        alpha [B] (K = None: open loop from x0).  Returns (x [3n, (N+1)*B], tau [n, N*B], J [B]) and, with derivatives=True, the
+        Riccati inputs of the cost at the new trajectory as a dict gx [3n, N*B], gu [n, N*B], wx, wu (curvature planes of the same
+        shapes), gN, wN [3n, B]: the arguments of `riccati_gains`."""
+        n, N = self.n, int(N)
+        B = x0.shape[1] if x0.dim() == 2 else -1
+        U = N * B
+        c = self._track_cost(cost, B, N)
+        self._gains(K, U)
+        x, tau, J = self._out(None, 3 * n, (N + 1) * B, "x"), self._out(None, n, U, "tau"), self._out(None, 1, B, "J").view(B)
+        dv = {}
+        if derivatives:
+            dv = dict(gx=self._out(None, 3 * n, U, "gx"), gu=self._out(None, n, U, "gu"), wx=self._out(None, 3 * n, U, "wx"),
+                      wu=self._out(None, n, U, "wu"), gN=self._out(None, 3 * n, B, "gN"), wN=self._out(None, 3 * n, B, "wN"))
+        p = lambda t: None if t is None else C.c_void_p(t.data_ptr())
+        with torch.cuda.device(self.device):
+            _capi.check(_capi.lib.mpcf_feedback_rollout_batch(
+                self.model.handle, C.byref(c), B, N, self._in(x0, 3 * n, B, "x0"), self._in(xbar, 3 * n, (N + 1) * B, "xbar", K is None),
+                self._in(taubar, n, U, "taubar"), p(K), None if K is None else self._in(alpha.view(1, -1), 1, B, "alpha"), float(dt),
+                p(x), p(tau), p(J), *[p(dv.get(k)) for k in ("gx", "gu", "wx", "wu", "gN", "wN")], _stream()))
+        return (x, tau, J, dv) if derivatives else (x, tau, J)
+
     def step_rk4_jvp_range(self, q, qd, tau, f, dt: float, u0: int, cnt: int, out, jac):
         """Units [u0, u0 + cnt) of a larger batch: states go to columns [u0, u0 + cnt) of the full-size `out` = (qn, qdn, fn),
         the Jacobian to the chunk-local buffer jac[3n, 4n+1, cap] (cap >= cnt) — one Jacobian buffer is reused over the
